@@ -1,6 +1,6 @@
 """bench.py -- headline benchmark of the B200-native tensorflow/compression hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extras] [--dump-outputs DIR]
     (N > 1: launched by `python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...`)
 
 Workload (BASELINE.json configs[1], "cfg2"): bls2017 compress path at batch 256, 256x256x3 images,
@@ -21,6 +21,10 @@ the `decode` / `gdn` / `cfg3_bmshj2018` / `model_path` objects of the JSON line 
             table builder); this arm never imports compression_b200.
 Parity: outside the timed region every rank checks its first batch against the oracle, byte for byte, and
 cross-decodes it (`parity_checked`).
+`--dump-outputs DIR` = after the timed steps, rank 0 writes the strings its last timed step produced (both arms) as
+            DIR/strings_bytes.npy (float32, one element per byte, all strings back to back) and
+            DIR/strings_offsets.npy (float64, the S + 1 offsets delimiting them); the inputs are seeded, so two builds
+            run with the same arguments can be compared output for output.
 
 Weak scaling: every rank codes its own 256-stream batch; rank 0 builds the tables and broadcasts them
 (NCCL); there is no data-path collective.
@@ -156,6 +160,16 @@ def load_fixture():
   z = np.load(FIXTURE)
   return dict(lookup=z["lookup"], cdf_offset=z["cdf_offset"],
               qoff=(z["quantization_offset"] if z["has_qoff"] else None))
+
+
+def dump_strings(out_dir, strings):
+  """Writes a batch of byte strings as the arrays a caller receives: the bytes back to back and their offsets."""
+  offsets = np.concatenate([[0], np.cumsum([len(s) for s in strings])]).astype(np.float64)
+  raw = np.frombuffer(b"".join(strings), np.uint8).astype(np.float32)
+  assert raw.nbytes + offsets.nbytes <= 64 << 20, "the dumped outputs would exceed 64 MB"
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "strings_bytes.npy"), raw)
+  np.save(os.path.join(out_dir, "strings_offsets.npy"), offsets)
 
 
 def stand_in_tables(scales):
@@ -387,8 +401,9 @@ def run_reference(args):
   def one():
     e = O.encoder(lookup, S)
     e.encode(value, None, threads)
-    e.finalize()
+    strings = e.finalize()
     e.close()
+    return strings
 
   for _ in range(max(args.warmup, 1)):
     one()
@@ -397,8 +412,10 @@ def run_reference(args):
   for _ in range(E2E_REPEATS):
     t0 = time.perf_counter()
     for _ in range(args.steps):
-      one()
+      last = one()
     regions.append(time.perf_counter() - t0)
+  if args.dump_outputs:
+    dump_strings(args.dump_outputs, last)
   dt = float(np.median(regions))
   val = S * N * args.steps / dt / 1e6
   spread = {"min": S * N * args.steps / max(regions) / 1e6, "max": S * N * args.steps / min(regions) / 1e6,
@@ -467,7 +484,10 @@ def main():
   ap.add_argument("--warmup", type=int, default=5)
   ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
   ap.add_argument("--no-extras", action="store_true", help="skip the decode / GDN / cfg3 / model-path / CPU side measurements")
+  ap.add_argument("--dump-outputs", metavar="DIR", help="write the strings of the last timed step to DIR as .npy")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
   if args.impl == "reference":
     return run_reference(args)
 
@@ -549,16 +569,16 @@ def main():
   fixture = load_fixture()
   tables_match = None if fixture is None else bool(np.array_equal(fixture["lookup"], model._lookup_host()))
 
-  # ---- the timed region: exactly K steps, CUDA events, max over ranks ----
+  # ---- the timed region: exactly K steps, CUDA events, max over ranks; returns the last step's strings too ----
   def timed_region(k):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     ev0.record()
     for i in range(k):
-      step(i)
+      last = step(i)
     ev1.record()
     barrier()
-    return allmax(ev0.elapsed_time(ev1))
+    return allmax(ev0.elapsed_time(ev1)), last
 
   phase("timed region")
   launches0 = _lib.launch_count()
@@ -566,12 +586,12 @@ def main():
   clocks = ClockSampler(local, str(torch.cuda.get_device_properties(dev).uuid)) if rank == 0 else None
   if clocks:
     clocks.__enter__()
-  elapsed_ms = timed_region(args.steps)
+  elapsed_ms, last_strings = timed_region(args.steps)
   if clocks:
     clocks.__exit__()
   launches = _lib.launch_count() - launches0
   value = world * sym_per_step * args.steps / (elapsed_ms * 1e-3) / 1e6
-  more = [timed_region(args.steps) for _ in range(4)]   # informational spread of the same region
+  more = [timed_region(args.steps)[0] for _ in range(4)]   # informational spread of the same region
   vals = sorted(world * sym_per_step * args.steps / (m * 1e-3) / 1e6 for m in [elapsed_ms] + more)
 
   # ---- e2e: pinned host y -> H2D -> compress -> D2H(bytes, offsets), same K steps ----
@@ -661,6 +681,8 @@ def main():
     except Exception as e:  # pylint:disable=broad-except
       result["extras_error"] = repr(e)
 
+  if rank == 0 and args.dump_outputs:
+    dump_strings(args.dump_outputs, last_strings.tolist())
   if rank == 0:
     print(json.dumps(result))
   if world > 1:

@@ -11,6 +11,7 @@ import pytest
 import torch
 
 import bench
+import golden_util
 import oracle
 
 pytestmark = pytest.mark.gpu
@@ -104,24 +105,30 @@ def test_cfg1_legacy_op_exactly_as_stated(per_channel):
   assert dec.dtype == torch.int16 and np.array_equal(dec.cpu().numpy(), data)
 
 
-def test_pmf_to_cdf_tie_rows_distance_to_the_compiled_reference():
-  """a-7 on tie rows (every symmetric NoisyNormal table of cfg3): the kernel equals the C port (lowest-index tie
-  break); against the compiled-reference flavour (libstdc++ std::sort order) the tables may differ only by moving
-  single counts between bins of EQUAL mass -- recorded here: identical bin-count multiset, |difference| <= 1 per
-  bin, and a coding-cost difference of exactly zero under the table's own PMF."""
-  if not oracle.have_ref():
-    pytest.skip("compiled reference not present")
-  from compression_b200 import gen_ops
+def tie_row_pmfs():
+  """One symmetric discretised-normal PMF row for every 7th of the 64 cfg3 scales."""
+  from scipy.stats import norm
   sig = np.exp(np.log(.11) + np.arange(64) * (np.log(256.) - np.log(.11)) / 63)
-  worst = 0
+  pmfs = []
   for s in sig[::7]:
     half = int(np.ceil(s * 2.8)) + 1
     k = np.arange(-half, half + 1, dtype=np.float64)
-    from scipy.stats import norm
-    pmf = (norm.cdf((k + .5) / s) - norm.cdf((k - .5) / s)).astype(np.float32)[None]
+    pmfs.append((norm.cdf((k + .5) / s) - norm.cdf((k - .5) / s)).astype(np.float32)[None])
+  return pmfs
+
+
+def test_pmf_to_cdf_tie_rows_distance_to_the_compiled_reference():
+  """a-7 on tie rows (every symmetric NoisyNormal table of cfg3): the kernel equals the C port (lowest-index tie
+  break); against the compiled-reference flavour (libstdc++ std::sort order; its tables are stored) the tables may
+  differ only by moving single counts between bins of EQUAL mass -- recorded here: identical bin-count multiset,
+  |difference| <= 1 per bin, and a coding-cost difference of exactly zero under the table's own PMF."""
+  from compression_b200 import gen_ops
+  refs = golden_util.load_reference_outputs()
+  worst = 0
+  for i, pmf in enumerate(tie_row_pmfs()):
     got = gen_ops.pmf_to_quantized_cdf(torch.from_numpy(pmf).cuda(), 12).cpu().numpy()
     assert np.array_equal(got, oracle.port().pmf_to_cdf(pmf, 12))
-    ref = oracle.ref().pmf_to_cdf(pmf, 12)
+    ref = refs[f"tie_row_cdf_{i}"]
     a, b = np.diff(got[0]), np.diff(ref[0])
     assert sorted(a) == sorted(b)
     assert np.abs(a - b).max() <= 1

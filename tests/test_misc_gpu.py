@@ -3,6 +3,7 @@ import numpy as np
 import pytest
 import torch
 
+import golden_util
 import oracle
 import util
 
@@ -60,14 +61,20 @@ def test_legacy_errors(ops):
 
 
 # ---- PmfToQuantizedCdf ----
-@pytest.mark.parametrize("n,precision,scale", [(32, 10, 0.85), (100, 7, 1.0), (257, 12, 1.3), (1500, 12, 1.0),
-                                               (2, 1, 1.0), (7, 16, 0.2)])
-def test_pmf_to_cdf_matches_oracle(ops, n, precision, scale):
+PMF_CASES = [(32, 10, 0.85), (100, 7, 1.0), (257, 12, 1.3), (1500, 12, 1.0), (2, 1, 1.0), (7, 16, 0.2)]
+
+
+def pmf_rows(n, scale):
   rng = np.random.default_rng(n)
   pmf = rng.random((5, n)).astype(np.float32)
   pmf[1] = pmf[1]**8           # peaky
   pmf[2, n // 2:] = 0          # half-zero row (pmf_to_cdf_kernels_test.cc:123-143)
-  pmf = (pmf / pmf.sum(-1, keepdims=True) * scale).astype(np.float32)
+  return (pmf / pmf.sum(-1, keepdims=True) * scale).astype(np.float32)
+
+
+@pytest.mark.parametrize("n,precision,scale", PMF_CASES)
+def test_pmf_to_cdf_matches_oracle(ops, n, precision, scale):
+  pmf = pmf_rows(n, scale)
   got = ops.pmf_to_quantized_cdf(torch.from_numpy(pmf).cuda(), precision).cpu().numpy()
   assert got.shape == (5, n + 1)
   assert (got[:, 0] == 0).all() and (got[:, -1] == 1 << precision).all()
@@ -75,10 +82,9 @@ def test_pmf_to_cdf_matches_oracle(ops, n, precision, scale):
   # The C port breaks ties like the kernel (lowest index, FIFO): always identical.
   assert np.array_equal(got, oracle.port().pmf_to_cdf(pmf, precision))
   # The compiled reference flavour uses std::sort: identical unless exact ties decide.
-  if oracle.have_ref():
-    ref = oracle.ref().pmf_to_cdf(pmf, precision)
-    for r in (0, 1, 3, 4):   # random rows: ties have probability ~0
-      assert np.array_equal(got[r], ref[r])
+  ref = golden_util.load_reference_outputs()[f"pmf_cdf_{n}_{precision}"]
+  for r in (0, 1, 3, 4):   # random rows: ties have probability ~0
+    assert np.array_equal(got[r], ref[r])
 
 
 def test_pmf_to_cdf_errors(ops):
