@@ -1,4 +1,4 @@
-// GDN / IGDN forward on the 5th-generation tensor cores (tcgen05 + TMEM), sm_100a.
+// GDN / IGDN forward and backward on the 5th-generation tensor cores (tcgen05 + TMEM), sm_100a.
 //
 //   n[pix, i] = sum_j p[pix, j] * gamma[j, i]      p = |x|, x^2 or relu(x) variants (py/layers/gdn.py:377-398)
 //
@@ -6,17 +6,19 @@
 // compute bound at ~1/3 of the HBM roofline.  Here the contraction runs as  tcgen05.mma kind::f16  on an
 // error-compensated bf16 split (3 products: hi*hi + lo*hi + hi*lo, fp32 accumulation in TMEM), which keeps the
 // result within ~4e-6 of fp32 (SURVEY.md App. D; the contract is 1e-5) at bf16 tensor throughput.
+// Every kernel is persistent (one CTA per SM, 128-pixel tiles) and specialised at compile time for FAST, the default
+// GDN / IGDN (alpha = 1, epsilon = 1, no rectification); the other instantiation honours TcFlags at run time.
 //
-// One CTA per SM, persistent over 128-pixel tiles.  gamma's hi/lo planes live in shared memory for the whole
-// launch in the UMMA "K-major, no swizzle" core-matrix layout ([K/8][N][8] bf16, LBO = N*16 B, SBO = 128 B).
-// Per tile, K is consumed in chunks of 64 channels:
-//   cp.async x[128, 64] fp32 -> staging  ->  threads split |x| into bf16 hi/lo operand planes
-//   ([8][128][8] bf16 each, LBO = 2048 B, SBO = 128 B)  ->  fence.proxy.async  ->  one thread issues 4 K-steps x
-//   3 MMAs (M=128, N=C, K=16)  ->  tcgen05.commit -> mbarrier.
-// Epilogue, 64 output channels at a time: tcgen05.ld (warp w owns TMEM lanes 32*(w%4)..) -> staging ->
-// coalesced pass  y = x / (beta + n)  with x re-read from L2.
+//   gdn_tc_fwd2_kernel<FAST, IO>     forward, C = 128, fp32 / fp16 / bf16 activations: the x tile resident in shared
+//                                    memory (bulk async copies), y written over it in place
+//   gdn_tc_fwd4_kernel<C, FAST>      forward, C = 192: x in 2-D TMA boxes, gamma's lo plane streamed
+//   gdn_tc_bwd3_kernel<FAST>         backward, C = 128: dx and the per-CTA dgamma / dbeta partials in one kernel
+//   gdn_tc_bwd_dx2_kernel<FAST>      backward, C = 192: dx and q = dL/dn (handed over as bf16 operand planes)
+//   gdn_tc_bwd_dgamma2_kernel<FAST>  backward, C = 192: dgamma / dbeta partials from x and q
+//   gdn_tc_prep_kernel, gdn_tc_prep2_kernel   gamma -> bf16 hi / lo operand planes
 //
-// Everything outside {C in {128, 192}, alpha in {1, 2}, eps in {1, 0.5}} falls back to the fp32 kernels in gdn.cu.
+// Everything outside {C in {128, 192}, alpha in {1, 2}, eps in {1, 0.5}} (and trainable exponents) runs the fp32
+// kernels in gdn.cu.
 #include <cuda.h>  // CUtensorMap (types only; cuTensorMapEncodeTiled is fetched through the runtime)
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -186,32 +188,6 @@ __device__ __forceinline__ void tmem_load<16>(uint32_t taddr, uint32_t (&r)[16])
 //   tcgen05.ld imposes) bank-conflict free, so no staging transposes and no barriers inside the epilogue.
 //   K is consumed in chunks of 16 channels through two small operand-plane buffers.
 // =============================================================================================
-constexpr int kStLd = 36;  // floats per staging row (32 + 4: conflict-free 128-bit access)
-
-__device__ __forceinline__ void stage_store16(float* dst, const uint32_t (&a)[16]) {
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-    *reinterpret_cast<float4*>(dst + 4 * i) = make_float4(__uint_as_float(a[4 * i]), __uint_as_float(a[4 * i + 1]),
-                                                           __uint_as_float(a[4 * i + 2]), __uint_as_float(a[4 * i + 3]));
-}
-
-// dgamma accumulates in TMEM across a CTA's tiles.  The tensor core adds every MMA into the fp32 accumulator with
-// TRUNCATION, so a long-running accumulator shrinks by ~2^-25 per accumulation step: measured 6e-6 of max |dgamma|
-// after one tile per CTA, 6.4e-5 after 110 (2 M pixels), linear in the tile count.  The accumulator is therefore
-// flushed into the CTA's fp32 partial in global memory (round-to-nearest adds, L2 resident) every kDgFlush tiles
-// and restarted; the drift stays below 3e-6 at any pixel count.
-constexpr int kDgFlush = 4;
-
-__device__ __forceinline__ void accum_store16(float* dst, const uint32_t (&a)[16], bool accumulate) {
-  float4 o[4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) o[i] = accumulate ? *reinterpret_cast<const float4*>(dst + 4 * i) : make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-    *reinterpret_cast<float4*>(dst + 4 * i) = make_float4(o[i].x + __uint_as_float(a[4 * i]), o[i].y + __uint_as_float(a[4 * i + 1]),
-                                                           o[i].z + __uint_as_float(a[4 * i + 2]), o[i].w + __uint_as_float(a[4 * i + 3]));
-}
-
 constexpr int kF2Threads = 320;   // 8 compute warps + 1 copy warp + 1 MMA-issue warp
 constexpr int kF2Compute = 256;
 constexpr int kF2XBuf = kTileM * 128 * 4;          // one x / y tile, dense [128][128] fp32 (one bulk copy)
@@ -941,45 +917,32 @@ int launch_tc_fwd4(const float* x, const float* gamma, const float* beta, float*
 }
 
 // =============================================================================================
-// Backward (C = 128): one fused kernel per launch instead of three fp32 passes.
+// Backward.  Per 128-pixel tile:
 //
-//   n  = beta + p . gamma                 MMA1   A = p planes (K-major),        B = gamma planes (K-major)
+//   n  = beta + p . gamma                 MMA1   A = p planes (K-major),        B = gamma (K-major)
 //   q  = dL/dn (elementwise, from g, x, n)
-//   dp = q . gamma^T                      MMA2   A = q planes (K-major),        B = gamma planes (MN-major view)
-//   dx = g / m + dpool/du * dp            (IGDN: g * m + ...)
+//   dp = q . gamma^T                      MMA2   A = q planes (K-major),        B = gamma^T
+//   dx = g / m + dpool/du * dp            (IGDN: g * m + ...; 0 where the rectifier cuts x off)
 //   dgamma[j, i] += sum_pix p[pix, j] q[pix, i]
 //                                         MMA3   A = p planes (MN-major view),  B = q planes (MN-major view)
-//   dbeta[i] += sum_pix q[pix, i]         warp transpose-reduce of the q registers
+//   dbeta[i] += sum_pix q[pix, i]
 //
 // The MN-major views reuse the very same shared-memory planes: a K-major plane [k / 8][row][8] read with the
 // "transposed" descriptor (instruction-descriptor bits 15 / 16) is the operand with the roles of row and k
 // swapped (core matrix = 8 k-rows of 16 bytes, LBO = 128 B between k groups, SBO = plane row-group stride).
-// TMEM: columns [0, C) n, [C, 2C) dp, [2C, 3C) this CTA's dgamma partial (accumulates over all its tiles).
-// HBM traffic per element: x and dy once (their re-reads in the two epilogues are L2 hits), dx once.
 // =============================================================================================
-constexpr int kBwdThreads = 288;  // 8 compute warps + 1 MMA-issue warp
 constexpr int kKg = kTileM * 16 + 16;  // byte stride between 8-channel groups of an operand plane: one 16-byte row
-                                       // of padding makes the coalesced (row, group) stores bank-conflict free;
+                                       // of padding makes the row-per-lane stores bank-conflict free;
                                        // the descriptors take it as LBO (K-major view) or SBO (MN-major view)
 
-template <int C>
-struct BwdSmem {
-  static constexpr int kPlaneB = C * C * 2;            // gamma hi / lo
-  static constexpr int kPlaneP = (C / 8) * kKg;        // p hi / lo (whole K)
-  static constexpr int kPlaneQ = 4 * kKg;              // q hi / lo, one 32-channel chunk
-  static constexpr int kStage = kTileM * kStLd * 4;    // fp32 [128][36]
-  static constexpr int kOffBh = 0;
-  static constexpr int kOffBl = kOffBh + kPlaneB;
-  static constexpr int kOffPh = kOffBl + kPlaneB;
-  static constexpr int kOffPl = kOffPh + kPlaneP;
-  static constexpr int kOffQ = kOffPl + kPlaneP;       // [2 buffers][hi, lo]
-  static constexpr int kOffStage = kOffQ + 4 * kPlaneQ;  // [2]: n, dp
-  static constexpr int kOffBeta = kOffStage + 2 * kStage;
-  static constexpr int kOffDbeta = kOffBeta + C * 4;
-  static constexpr int kOffBar = kOffDbeta + C * 4;
-  static constexpr int kBytes = kOffBar + 64;
-};
+// dgamma accumulates in TMEM across a CTA's tiles.  The tensor core adds every MMA into the fp32 accumulator with
+// TRUNCATION, so a long-running accumulator shrinks by ~2^-25 per accumulation step: measured 6e-6 of max |dgamma|
+// after one tile per CTA, 6.4e-5 after 110 (2 M pixels), linear in the tile count.  The accumulator is therefore
+// flushed into the CTA's fp32 partial in global memory (round-to-nearest adds, L2 resident) every kDgFlush tiles
+// and restarted; the drift stays below 3e-6 at any pixel count.
+constexpr int kDgFlush = 4;
 
+// q = dL/dn = -g u / n^2 (IGDN: g u; epsilon = 1/2: -g u / (2 n^1.5), IGDN g u / (2 sqrt(n))), u = x or relu(x)
 template <bool FAST>
 __device__ __forceinline__ float tc_dl_dn(float g, float x, float n, const TcFlags& f) {
   const float u = (!FAST && f.rectify) ? fmaxf(x, 0.f) : x;
@@ -989,859 +952,23 @@ __device__ __forceinline__ float tc_dl_dn(float g, float x, float n, const TcFla
   return f.inverse ? 0.5f * g * u * rs : -0.5f * g * u * r * rs;
 }
 
+// The direct term of dx: g / m (IGDN: g * m), m = n or sqrt(n)
 template <bool FAST>
-__device__ __forceinline__ float tc_dx(float g, float x, float n, float dp, const TcFlags& f) {
-  const float u = (!FAST && f.rectify) ? fmaxf(x, 0.f) : x;
-  float direct;
-  if (FAST || f.eps_mode == 1) direct = f.inverse ? g * n : g * rcp_approx(n);
-  else direct = f.inverse ? g * sqrtf(n) : g * rsqrtf(n);
+__device__ __forceinline__ float tc_direct(float g, float n, const TcFlags& f) {
+  if (FAST || f.eps_mode == 1) return f.inverse ? g * n : g * rcp_approx(n);
+  return f.inverse ? g * sqrtf(n) : g * rsqrtf(n);
+}
+
+// dx = direct + dpool/du * dp, 0 where the rectifier cuts x off.  The default GDN (FAST) does not call this: its
+// dpool/du is sign(x), which the kernels carry in the low mantissa bits of the direct term instead of x.
+__device__ __forceinline__ float tc_dx(float direct, float x, float dp, const TcFlags& f) {
+  const float u = f.rectify ? fmaxf(x, 0.f) : x;
   float dpool;
-  if (FAST || f.alpha_mode == 1) dpool = (!FAST && f.rectify) ? 1.f : ((u > 0.f) ? 1.f : ((u < 0.f) ? -1.f : 0.f));
+  if (f.alpha_mode == 1) dpool = f.rectify ? 1.f : ((u > 0.f) ? 1.f : ((u < 0.f) ? -1.f : 0.f));
   else dpool = 2.f * u;
-  float d = direct + dpool * dp;
-  if (!FAST && f.rectify && !(x > 0.f)) d = 0.f;
-  return d;
+  return (f.rectify && !(x > 0.f)) ? 0.f : direct + dpool * dp;
 }
 
-// Warp roles: 8 compute warps + 1 MMA-issue warp.  Compute threads never block on a CTA-wide barrier to hand
-// operands over: they ARRIVE on a named barrier once their planes are written and fenced; the issue warp waits
-// on it, issues the MMAs and commits to an mbarrier.  TMEM side, compute thread (r = tid % 128, h = tid / 128)
-// owns pixel row r (= TMEM lane) and half of the columns being moved; memory side, item (row, kg) = 8
-// consecutive channels of one pixel, items enumerated row-major so that a warp reads whole 128-byte lines.
-constexpr int kBwdCompute = 256;
-constexpr int kBwdStLd2 = 68;    // staging row of the 64-column n passes (P2)
-constexpr int kBwdStLd3 = 132;   // staging row of the full n / dp tiles (P3; aliases the dead operand planes)
-
-template <int C, bool FAST>
-__global__ void __launch_bounds__(kBwdThreads, 1)
-gdn_tc_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, const __nv_bfloat16* __restrict__ planes,
-                  const float* __restrict__ beta, float* __restrict__ dx, float* __restrict__ part_g,
-                  float* __restrict__ part_b, long long n_pix, TcFlags f) {
-  using L = BwdSmem<C>;
-  static_assert(C == 128, "TMEM holds n, dp and the dgamma partial only for C = 128");
-  static_assert(2 * L::kStage >= kTileM * kBwdStLd2 * 4, "P2 staging");
-  static_assert(2 * L::kPlaneP + 4 * L::kPlaneQ + 2 * L::kStage >= 2 * kTileM * kBwdStLd3 * 4, "P3 staging");
-  constexpr int NCH = C / 32;
-  extern __shared__ __align__(1024) uint8_t smem[];
-  float* beta_s = reinterpret_cast<float*>(smem + L::kOffBeta);
-  float* dbeta_s = reinterpret_cast<float*>(smem + L::kOffDbeta);
-  float* stage2 = reinterpret_cast<float*>(smem + L::kOffStage);                 // [128][68]
-  float* stage3n = reinterpret_cast<float*>(smem + L::kOffPh);                   // [128][132], planes are dead
-  float* stage3d = stage3n + kTileM * kBwdStLd3;
-  uint64_t* mbars = reinterpret_cast<uint64_t*>(smem + L::kOffBar);  // [0,1] MMA1 halves, [2,3] q buffers
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + L::kOffBar + 40);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int r = tid & 127, h = (tid >> 7) & 1, gwarp = warp & 3;
-  constexpr uint32_t kIdesc1 = umma_idesc(kTileM, 64);                         // MMA1, one 64-column half of n
-  constexpr uint32_t kIdesc2 = umma_idesc(kTileM, C) | (1u << 16);             // B = gamma^T (MN-major view)
-  constexpr uint32_t kIdesc3 = umma_idesc(C, 32) | (1u << 15) | (1u << 16);    // A = p^T, B = q chunk (both views)
-
-  {
-    const uint4* src = reinterpret_cast<const uint4*>(planes);
-    uint4* dst = reinterpret_cast<uint4*>(smem + L::kOffBh);
-    for (int i = tid; i < 2 * L::kPlaneB / 16; i += kBwdThreads) dst[i] = src[i];
-    for (int i = tid; i < C; i += kBwdThreads) {
-      beta_s[i] = beta[i];
-      dbeta_s[i] = 0.f;
-    }
-  }
-  if (tid == 0) {
-    for (int i = 0; i < 4; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mbars + i)));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_n = *tmem_slot, tmem_dp = tmem_n + C, tmem_dg = tmem_n + 2 * C;
-  const uint32_t lane_sel = (uint32_t)(gwarp * 32) << 16;
-  const uint32_t b_hi = smem_u32(smem + L::kOffBh), b_lo = smem_u32(smem + L::kOffBl);
-  const uint32_t p_hi = smem_u32(smem + L::kOffPh), p_lo = smem_u32(smem + L::kOffPl);
-  const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  int t_idx = 0;  // this CTA's tile counter (both roles count alike)
-
-  if (warp == kBwdCompute / 32) {
-    // ------------------------------- MMA-issue warp -------------------------------
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t_idx) {
-      // next tile of this CTA -> L2 (one bulk prefetch per array: the tile is contiguous)
-      if (lane == 1) {
-        const long long pn = (tile + gridDim.x) * kTileM;
-        const long long rows = min((long long)kTileM, n_pix - pn);
-        if (rows > 0) {
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(x + pn * C), "r"((uint32_t)(rows * C * 4)) : "memory");
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(dy + pn * C), "r"((uint32_t)(rows * C * 4)) : "memory");
-        }
-      }
-      // MMA1: n = p . gamma, the two 64-column halves one after the other so that P2 can start on the first
-      asm volatile("bar.sync 2, %0;" ::"n"(kBwdThreads) : "memory");
-      if (lane == 0) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-#pragma unroll
-          for (int s = 0; s < C / 16; ++s) {
-            const uint64_t dah = umma_desc(p_hi + (uint32_t)(2 * s) * kKg, kKg, 128);
-            const uint64_t dal = umma_desc(p_lo + (uint32_t)(2 * s) * kKg, kKg, 128);
-            const uint32_t boff = (uint32_t)(2 * s) * (C * 16) + (uint32_t)(half * 64) * 16u;
-            const uint64_t dbh = umma_desc(b_hi + boff, C * 16, 128);
-            const uint64_t dbl = umma_desc(b_lo + boff, C * 16, 128);
-            umma_bf16(tmem_n + (uint32_t)(half * 64), dah, dbh, kIdesc1, s ? 1u : 0u);
-            umma_bf16(tmem_n + (uint32_t)(half * 64), dal, dbh, kIdesc1, 1u);
-            umma_bf16(tmem_n + (uint32_t)(half * 64), dah, dbl, kIdesc1, 1u);
-          }
-          umma_commit(smem_u32(mbars + half));
-        }
-      }
-      __syncwarp();
-#pragma unroll
-      for (int c = 0; c < NCH; ++c) {
-        const int b = c & 1;
-        asm volatile("bar.sync %0, %1;" ::"r"(3 + b), "n"(kBwdThreads) : "memory");
-        if (lane == 0) {
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          const uint32_t q_hi = smem_u32(smem + L::kOffQ + b * 2 * L::kPlaneQ), q_lo = q_hi + L::kPlaneQ;
-          // MMA2: dp[pix, j] += sum_{i in chunk} q[pix, i] gamma[j, i]   (K = i: 2 steps of 16)
-#pragma unroll
-          for (int s = 0; s < 2; ++s) {
-            const uint64_t dah = umma_desc(q_hi + (uint32_t)(2 * s) * kKg, kKg, 128);
-            const uint64_t dal = umma_desc(q_lo + (uint32_t)(2 * s) * kKg, kKg, 128);
-            // gamma plane viewed with n = j, k = i: k rows are 16 B apart, k groups 128 B, n groups C * 16 B
-            const uint32_t koff = (uint32_t)(c * 32 + s * 16) * 16u;
-            const uint64_t dbh = umma_desc(b_hi + koff, 128, C * 16);
-            const uint64_t dbl = umma_desc(b_lo + koff, 128, C * 16);
-            umma_bf16(tmem_dp, dah, dbh, kIdesc2, (c | s) ? 1u : 0u);
-            umma_bf16(tmem_dp, dal, dbh, kIdesc2, 1u);
-            umma_bf16(tmem_dp, dah, dbl, kIdesc2, 1u);
-          }
-          // MMA3: dgamma[j, i in chunk] += sum_pix p[pix, j] q[pix, i]   (K = pix: 8 steps of 16)
-#pragma unroll
-          for (int s = 0; s < kTileM / 16; ++s) {
-            const uint32_t koff = (uint32_t)(s * 16) * 16u;
-            const uint64_t dah = umma_desc(p_hi + koff, 128, kKg);
-            const uint64_t dal = umma_desc(p_lo + koff, 128, kKg);
-            const uint64_t dbh = umma_desc(q_hi + koff, 128, kKg);
-            const uint64_t dbl = umma_desc(q_lo + koff, 128, kKg);
-            const uint32_t acc_on = ((t_idx % kDgFlush) == 0 && s == 0) ? 0u : 1u;  // restarted after every flush
-            umma_bf16(tmem_dg + (uint32_t)(c * 32), dah, dbh, kIdesc3, acc_on);
-            umma_bf16(tmem_dg + (uint32_t)(c * 32), dal, dbh, kIdesc3, 1u);
-            umma_bf16(tmem_dg + (uint32_t)(c * 32), dah, dbl, kIdesc3, 1u);
-          }
-          umma_commit(smem_u32(mbars + 2 + b));
-        }
-        __syncwarp();
-      }
-    }
-  } else {
-  // --------------------------------- compute warps ---------------------------------
-  uint32_t parn[2] = {0u, 0u}, parq[2] = {0u, 0u};
-  float dbeta_acc[NCH][8];  // channels c * 32 + (tid % 4) * 8 + e, summed over this thread's rows
-#pragma unroll
-  for (int c = 0; c < NCH; ++c)
-#pragma unroll
-    for (int e = 0; e < 8; ++e) dbeta_acc[c][e] = 0.f;
-  const int ckg = tid & 3;         // 8-channel group inside a 32-channel chunk
-  const int crow = tid >> 2;       // rows crow and crow + 64
-  auto compute_sync = [] { asm volatile("bar.sync 1, %0;" ::"n"(kBwdCompute) : "memory"); };
-  bool flushed = false;  // the global partial holds earlier flushes
-  // adds the TMEM dgamma accumulator (lane r = input channel j, this thread's 64 columns) into the CTA's partial
-  auto flush_dgamma = [&]() {
-    float* pg = part_g + (long long)blockIdx.x * C * C + (long long)r * C + h * 64;
-#pragma unroll
-    for (int cb = 0; cb < 4; ++cb) {
-      uint32_t a[16];
-      tmem_load<16>(tmem_dg + lane_sel + (uint32_t)(h * 64 + cb * 16), a);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      accum_store16(pg + cb * 16, a, flushed);
-    }
-    flushed = true;
-  };
-
-  for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t_idx) {
-    const long long p0 = tile * kTileM;
-    // ---- P1: p = pool(x) -> hi / lo planes [j / 8][row][8]; item = (row, kg), 16 groups per row ----
-    {
-      constexpr int ITEMS = kTileM * (C / 8) / kBwdCompute;  // 8
-      float4 xv[ITEMS][2];
-#pragma unroll
-      for (int it = 0; it < ITEMS; ++it) {
-        const int id = it * kBwdCompute + tid;
-        const int row = id / (C / 8), kg = id % (C / 8);
-        const bool live = p0 + row < n_pix;
-        const float4* src = reinterpret_cast<const float4*>(x + (p0 + row) * C + kg * 8);
-        xv[it][0] = live ? __ldg(src) : make_float4(0.f, 0.f, 0.f, 0.f);
-        xv[it][1] = live ? __ldg(src + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-#pragma unroll
-      for (int it = 0; it < ITEMS; ++it) {
-        const int id = it * kBwdCompute + tid;
-        const int row = id / (C / 8), kg = id % (C / 8);
-        const float4 a = xv[it][0], b = xv[it][1];
-        float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
-                      tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
-        uint4 hi, lo;
-        split8(v, &hi, &lo);
-        *reinterpret_cast<uint4*>(smem + L::kOffPh + kg * kKg + row * 16) = hi;
-        *reinterpret_cast<uint4*>(smem + L::kOffPl + kg * kKg + row * 16) = lo;
-      }
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    asm volatile("bar.arrive 2, %0;" ::"n"(kBwdThreads) : "memory");
-    // x and dy of a chunk for this thread's two items (coalesced; L2 hits after the prefetch / P1).  Two register
-    // sets: the loads of the next chunk are issued a whole chunk ahead of their use.
-    float4 xq[2][2][2], gq[2][2][2];  // [set][item][half]
-    auto load_xg = [&](int set, int c) {
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int row = crow + 64 * it;
-        const bool live = p0 + row < n_pix;
-        const long long off = (p0 + row) * C + c * 32 + ckg * 8;
-        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-        xq[set][it][0] = live ? __ldg(reinterpret_cast<const float4*>(x + off)) : z;
-        xq[set][it][1] = live ? __ldg(reinterpret_cast<const float4*>(x + off) + 1) : z;
-        gq[set][it][0] = live ? __ldg(reinterpret_cast<const float4*>(dy + off)) : z;
-        gq[set][it][1] = live ? __ldg(reinterpret_cast<const float4*>(dy + off) + 1) : z;
-      }
-    };
-    // ---- P2: q = dL/dn -> q planes (32-channel chunks); n is staged 64 columns at a time ----
-    load_xg(0, 0);
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int b = c & 1;
-      load_xg(b ^ 1, (c + 1) % NCH);  // next chunk; after the last one: chunk 0 again, for the dx pass
-      if ((c & 1) == 0) {
-        const int half = c >> 1;
-        if (c) compute_sync();  // everyone is done reading the previous 64 staged columns
-        if (!mbar_wait(smem_u32(mbars + half), parn[half])) __trap();
-        parn[half] ^= 1u;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        uint32_t acc[32];
-        tmem_load<32>(tmem_n + lane_sel + (uint32_t)(half * 64 + h * 32), acc);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        float* dst = stage2 + r * kBwdStLd2 + h * 32;
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-          *reinterpret_cast<float4*>(dst + 4 * i) = make_float4(__uint_as_float(acc[4 * i]), __uint_as_float(acc[4 * i + 1]),
-                                                                 __uint_as_float(acc[4 * i + 2]), __uint_as_float(acc[4 * i + 3]));
-        compute_sync();
-      }
-      // the q buffer was read by the MMAs of chunk c - 2 (chunks 2, 3 of the previous tile: waited for before its dx pass)
-      if (c >= 2) {
-        if (!mbar_wait(smem_u32(mbars + 2 + b), parq[b])) __trap();
-        parq[b] ^= 1u;
-      }
-      uint8_t* qh = smem + L::kOffQ + b * 2 * L::kPlaneQ;
-      uint8_t* ql = qh + L::kPlaneQ;
-      const float4 bv0 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8);
-      const float4 bv1 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8 + 4);
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int row = crow + 64 * it;
-        const float* ns = stage2 + row * kBwdStLd2 + (c & 1) * 32 + ckg * 8;
-        const float4 n0 = *reinterpret_cast<const float4*>(ns);
-        const float4 n1 = *reinterpret_cast<const float4*>(ns + 4);
-        const float4 x0 = xq[b][it][0], x1 = xq[b][it][1], g0 = gq[b][it][0], g1 = gq[b][it][1];
-        float q[8];
-        q[0] = tc_dl_dn<FAST>(g0.x, x0.x, bv0.x + n0.x, f);
-        q[1] = tc_dl_dn<FAST>(g0.y, x0.y, bv0.y + n0.y, f);
-        q[2] = tc_dl_dn<FAST>(g0.z, x0.z, bv0.z + n0.z, f);
-        q[3] = tc_dl_dn<FAST>(g0.w, x0.w, bv0.w + n0.w, f);
-        q[4] = tc_dl_dn<FAST>(g1.x, x1.x, bv1.x + n1.x, f);
-        q[5] = tc_dl_dn<FAST>(g1.y, x1.y, bv1.y + n1.y, f);
-        q[6] = tc_dl_dn<FAST>(g1.z, x1.z, bv1.z + n1.z, f);
-        q[7] = tc_dl_dn<FAST>(g1.w, x1.w, bv1.w + n1.w, f);
-        uint4 hi, lo;
-        split8(q, &hi, &lo);
-        *reinterpret_cast<uint4*>(qh + ckg * kKg + row * 16) = hi;
-        *reinterpret_cast<uint4*>(ql + ckg * kKg + row * 16) = lo;
-#pragma unroll
-        for (int e = 0; e < 8; ++e) dbeta_acc[c][e] += q[e];
-      }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      asm volatile("bar.arrive %0, %1;" ::"r"(3 + b), "n"(kBwdThreads) : "memory");
-    }
-    // ---- P3: dx = g / m + dpool/du * dp  (chunk 0 is already in register set 0) ----
-#pragma unroll
-    for (int b = 0; b < 2; ++b) {  // commits of chunks 2 and 3: all MMAs of this tile are done, the planes are dead
-      if (!mbar_wait(smem_u32(mbars + 2 + b), parq[b])) __trap();
-      parq[b] ^= 1u;
-    }
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    // whole n and dp tiles -> staging (over the dead operand planes), thread (r, h) moves 64 columns of each
-#pragma unroll
-    for (int part = 0; part < 4; ++part) {
-      const uint32_t col = (uint32_t)(h * 64 + (part & 1) * 32);
-      uint32_t acc[32];
-      tmem_load<32>(((part >> 1) ? tmem_dp : tmem_n) + lane_sel + col, acc);
-      asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      float* dst = ((part >> 1) ? stage3d : stage3n) + r * kBwdStLd3 + col;
-#pragma unroll
-      for (int i = 0; i < 8; ++i)
-        *reinterpret_cast<float4*>(dst + 4 * i) = make_float4(__uint_as_float(acc[4 * i]), __uint_as_float(acc[4 * i + 1]),
-                                                               __uint_as_float(acc[4 * i + 2]), __uint_as_float(acc[4 * i + 3]));
-    }
-    compute_sync();
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int b = c & 1;
-      if (c + 1 < NCH) load_xg(b ^ 1, c + 1);
-      const float4 bv0 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8);
-      const float4 bv1 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8 + 4);
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int row = crow + 64 * it;
-        const float* ns = stage3n + row * kBwdStLd3 + c * 32 + ckg * 8;
-        const float* ds = stage3d + row * kBwdStLd3 + c * 32 + ckg * 8;
-        const float4 n0 = *reinterpret_cast<const float4*>(ns), n1 = *reinterpret_cast<const float4*>(ns + 4);
-        const float4 d0 = *reinterpret_cast<const float4*>(ds), d1 = *reinterpret_cast<const float4*>(ds + 4);
-        const float4 x0 = xq[b][it][0], x1 = xq[b][it][1], g0 = gq[b][it][0], g1 = gq[b][it][1];
-        float4 o0, o1;
-        o0.x = tc_dx<FAST>(g0.x, x0.x, bv0.x + n0.x, d0.x, f);
-        o0.y = tc_dx<FAST>(g0.y, x0.y, bv0.y + n0.y, d0.y, f);
-        o0.z = tc_dx<FAST>(g0.z, x0.z, bv0.z + n0.z, d0.z, f);
-        o0.w = tc_dx<FAST>(g0.w, x0.w, bv0.w + n0.w, d0.w, f);
-        o1.x = tc_dx<FAST>(g1.x, x1.x, bv1.x + n1.x, d1.x, f);
-        o1.y = tc_dx<FAST>(g1.y, x1.y, bv1.y + n1.y, d1.y, f);
-        o1.z = tc_dx<FAST>(g1.z, x1.z, bv1.z + n1.z, d1.z, f);
-        o1.w = tc_dx<FAST>(g1.w, x1.w, bv1.w + n1.w, d1.w, f);
-        if (p0 + row < n_pix) {
-          float4* dst = reinterpret_cast<float4*>(dx + (p0 + row) * C + c * 32 + ckg * 8);
-          __stcs(dst, o0);  // streaming stores: keep x / dy (re-read from L2) resident instead of the outputs
-          __stcs(dst + 1, o1);
-        }
-      }
-    }
-    // every MMA of this tile has completed (the two waits above): flush the dgamma accumulator when due
-    if ((t_idx % kDgFlush) == kDgFlush - 1) flush_dgamma();
-    // the staging (= operand planes) and the n / dp columns are rewritten by the next tile
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    compute_sync();
-  }
-
-  // ---- this CTA's partial sums ----
-  if (t_idx > 0) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if ((t_idx % kDgFlush) != 0) flush_dgamma();  // tiles since the last flush
-    // dbeta: lanes with the same tid % 4 hold the same channels
-#pragma unroll
-    for (int c = 0; c < NCH; ++c)
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        float v = dbeta_acc[c][e];
-        v += __shfl_xor_sync(0xFFFFFFFFu, v, 4);
-        v += __shfl_xor_sync(0xFFFFFFFFu, v, 8);
-        v += __shfl_xor_sync(0xFFFFFFFFu, v, 16);
-        if (lane < 4) atomicAdd(dbeta_s + c * 32 + lane * 8 + e, v);
-      }
-  }
-  }  // compute warps
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < C) part_b[(long long)blockIdx.x * C + tid] = dbeta_s[tid];
-  if (tid < 32) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*tmem_slot), "n"(512));
-  }
-}
-
-// =============================================================================================
-// Backward for C = 192: two kernels.  n, dp and a dgamma accumulator would need 3 x 192 TMEM columns and the
-// gamma planes plus a full-K p plane 243 KB of shared memory, so the dgamma contraction moves to its own
-// kernel and q = dL/dn travels through global memory (fp32, the caller's workspace):
-//   K1  gdn_tc_bwd_dx_kernel     : n = beta + p.gamma (p converted 16 channels at a time) -> q (stored) ->
-//                                  dp = q.gamma^T -> dx.   TMEM: n | dp (2 x 192 columns).
-//   K2  gdn_tc_bwd_dgamma_kernel : dgamma += p^T q over all tiles of the CTA, dbeta = column sums of q.  No gamma:
-//                                  the full-K p and q planes fill the shared memory.  M = 192 does not exist, so
-//                                  rows j in [0,128) and [64,192) are two overlapping M = 128 blocks.
-// HBM traffic: K1 x, dy in; dx, q out.  K2 x, q in.  (6 passes against the fused kernel's 3.)
-// =============================================================================================
-template <int C>
-struct Bwd2Smem {
-  static constexpr int kPlaneB = C * C * 2;          // gamma hi / lo
-  static constexpr int kPlaneP = 2 * kKg;            // p hi or lo, one 16-channel chunk
-  static constexpr int kPlaneQ = 4 * kKg;            // q hi or lo, one 32-channel chunk
-  static constexpr int kStage = kTileM * kStLd * 4;  // fp32 [128][36]
-  static constexpr int kOffBh = 0;
-  static constexpr int kOffBl = kOffBh + kPlaneB;
-  static constexpr int kOffP = kOffBl + kPlaneB;     // [2 buffers][hi, lo]
-  static constexpr int kOffQ = kOffP + 4 * kPlaneP;  // [2 buffers][hi, lo]; the dx pass stages dp here
-  static constexpr int kOffStage = kOffQ + 4 * kPlaneQ;
-  static constexpr int kOffBeta = kOffStage + kStage;
-  static constexpr int kOffBar = kOffBeta + C * 4;
-  static constexpr int kBytes = kOffBar + 64;
-  static_assert(4 * kPlaneQ >= kStage, "dp staging aliases the q planes");
-  static_assert(kBytes <= 232448, "shared memory budget");
-};
-
-template <int C, bool FAST>
-__global__ void __launch_bounds__(kBwdThreads, 1)
-gdn_tc_bwd_dx_kernel(const float* __restrict__ x, const float* __restrict__ dy, const __nv_bfloat16* __restrict__ planes,
-                     const float* __restrict__ beta, float* __restrict__ dx, float* __restrict__ q_out, long long n_pix,
-                     TcFlags f) {
-  using L = Bwd2Smem<C>;
-  constexpr int NCH = C / 32;   // q / dx chunks
-  constexpr int NK = C / 16;    // p chunks (one MMA K step each)
-  static_assert(2 * C <= 512 && NK % 2 == 0 && NCH % 2 == 0, "layout");
-  extern __shared__ __align__(1024) uint8_t smem[];
-  float* beta_s = reinterpret_cast<float*>(smem + L::kOffBeta);
-  float* stage_n = reinterpret_cast<float*>(smem + L::kOffStage);
-  float* stage_d = reinterpret_cast<float*>(smem + L::kOffQ);
-  uint64_t* mbars = reinterpret_cast<uint64_t*>(smem + L::kOffBar);  // [0,1] p buffers, [2,3] q buffers
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + L::kOffBar + 40);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int r = tid & 127, h = (tid >> 7) & 1, gwarp = warp & 3;
-  constexpr uint32_t kIdesc1 = umma_idesc(kTileM, C);
-  constexpr uint32_t kIdesc2 = umma_idesc(kTileM, C) | (1u << 16);  // B = gamma^T (MN-major view)
-  {
-    const uint4* src = reinterpret_cast<const uint4*>(planes);
-    uint4* dst = reinterpret_cast<uint4*>(smem + L::kOffBh);
-    for (int i = tid; i < 2 * L::kPlaneB / 16; i += kBwdThreads) dst[i] = src[i];
-    for (int i = tid; i < C; i += kBwdThreads) beta_s[i] = beta[i];
-  }
-  if (tid == 0) {
-    for (int i = 0; i < 4; ++i) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mbars + i)));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_n = *tmem_slot, tmem_dp = tmem_n + C;
-  const uint32_t lane_sel = (uint32_t)(gwarp * 32) << 16;
-  const uint32_t b_hi = smem_u32(smem + L::kOffBh), b_lo = smem_u32(smem + L::kOffBl);
-  const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-
-  if (warp == kBwdCompute / 32) {
-    // ------------------------------- MMA-issue warp -------------------------------
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      if (lane == 1) {
-        const long long pn = (tile + gridDim.x) * kTileM;
-        const long long rows = min((long long)kTileM, n_pix - pn);
-        if (rows > 0) {
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(x + pn * C), "r"((uint32_t)(rows * C * 4)) : "memory");
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(dy + pn * C), "r"((uint32_t)(rows * C * 4)) : "memory");
-        }
-      }
-#pragma unroll 1
-      for (int c = 0; c < NK; ++c) {  // MMA1: one K step per 16-channel p chunk
-        const int pb = c & 1;
-        asm volatile("bar.sync %0, %1;" ::"r"(2 + pb), "n"(kBwdThreads) : "memory");
-        if (lane == 0) {
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          const uint32_t ph = smem_u32(smem + L::kOffP + pb * 2 * L::kPlaneP), pl = ph + L::kPlaneP;
-          const uint64_t dah = umma_desc(ph, kKg, 128), dal = umma_desc(pl, kKg, 128);
-          const uint64_t dbh = umma_desc(b_hi + (uint32_t)(2 * c) * (C * 16), C * 16, 128);
-          const uint64_t dbl = umma_desc(b_lo + (uint32_t)(2 * c) * (C * 16), C * 16, 128);
-          umma_bf16(tmem_n, dah, dbh, kIdesc1, c ? 1u : 0u);
-          umma_bf16(tmem_n, dal, dbh, kIdesc1, 1u);
-          umma_bf16(tmem_n, dah, dbl, kIdesc1, 1u);
-          umma_commit(smem_u32(mbars + pb));
-        }
-        __syncwarp();
-      }
-#pragma unroll 1
-      for (int c = 0; c < NCH; ++c) {  // MMA2: dp += q chunk . gamma^T
-        const int b = c & 1;
-        asm volatile("bar.sync %0, %1;" ::"r"(4 + b), "n"(kBwdThreads) : "memory");
-        if (lane == 0) {
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          const uint32_t q_hi = smem_u32(smem + L::kOffQ + b * 2 * L::kPlaneQ), q_lo = q_hi + L::kPlaneQ;
-#pragma unroll
-          for (int s2 = 0; s2 < 2; ++s2) {
-            const uint64_t dah = umma_desc(q_hi + (uint32_t)(2 * s2) * kKg, kKg, 128);
-            const uint64_t dal = umma_desc(q_lo + (uint32_t)(2 * s2) * kKg, kKg, 128);
-            const uint32_t koff = (uint32_t)(c * 32 + s2 * 16) * 16u;
-            const uint64_t dbh = umma_desc(b_hi + koff, 128, C * 16);
-            const uint64_t dbl = umma_desc(b_lo + koff, 128, C * 16);
-            umma_bf16(tmem_dp, dah, dbh, kIdesc2, (c | s2) ? 1u : 0u);
-            umma_bf16(tmem_dp, dal, dbh, kIdesc2, 1u);
-            umma_bf16(tmem_dp, dah, dbl, kIdesc2, 1u);
-          }
-          umma_commit(smem_u32(mbars + 2 + b));
-        }
-        __syncwarp();
-      }
-    }
-  } else {
-  // --------------------------------- compute warps ---------------------------------
-  uint32_t parp[2] = {0u, 0u}, parq[2] = {0u, 0u};
-  const int ckg = tid & 3, crow = tid >> 2;   // items of a 32-channel chunk: rows crow, crow + 64
-  const int pkg = tid & 1, prow = tid >> 1;   // item of a 16-channel p chunk
-  auto compute_sync = [] { asm volatile("bar.sync 1, %0;" ::"n"(kBwdCompute) : "memory"); };
-
-  for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const long long p0 = tile * kTileM;
-    // ---- P1: p chunks -> planes -> MMA1, the loads of six chunks in flight at a time ----
-    {
-      const bool live = p0 + prow < n_pix;
-      const float* xr = x + (p0 + prow) * C + pkg * 8;
-#pragma unroll
-      for (int half = 0; half < 2; ++half) {
-        float4 xv[NK / 2][2];
-#pragma unroll
-        for (int k = 0; k < NK / 2; ++k) {
-          const float4* src = reinterpret_cast<const float4*>(xr + (half * (NK / 2) + k) * 16);
-          xv[k][0] = live ? __ldg(src) : make_float4(0.f, 0.f, 0.f, 0.f);
-          xv[k][1] = live ? __ldg(src + 1) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-#pragma unroll
-        for (int k = 0; k < NK / 2; ++k) {
-          const int c = half * (NK / 2) + k, pb = c & 1;
-          if (c >= 2) {
-            if (!mbar_wait(smem_u32(mbars + pb), parp[pb])) __trap();
-            parp[pb] ^= 1u;
-          }
-          const float4 a = xv[k][0], b = xv[k][1];
-          float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
-                        tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
-          uint4 hi, lo;
-          split8(v, &hi, &lo);
-          uint8_t* ph = smem + L::kOffP + pb * 2 * L::kPlaneP;
-          *reinterpret_cast<uint4*>(ph + pkg * kKg + prow * 16) = hi;
-          *reinterpret_cast<uint4*>(ph + L::kPlaneP + pkg * kKg + prow * 16) = lo;
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-          asm volatile("bar.arrive %0, %1;" ::"r"(2 + pb), "n"(kBwdThreads) : "memory");
-        }
-      }
-    }
-    float4 xq[2][2][2], gq[2][2][2];  // [set][item][half]
-    auto load_xg = [&](int set, int c) {
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int row = crow + 64 * it;
-        const bool live = p0 + row < n_pix;
-        const long long off = (p0 + row) * C + c * 32 + ckg * 8;
-        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-        xq[set][it][0] = live ? __ldg(reinterpret_cast<const float4*>(x + off)) : z;
-        xq[set][it][1] = live ? __ldg(reinterpret_cast<const float4*>(x + off) + 1) : z;
-        gq[set][it][0] = live ? __ldg(reinterpret_cast<const float4*>(dy + off)) : z;
-        gq[set][it][1] = live ? __ldg(reinterpret_cast<const float4*>(dy + off) + 1) : z;
-      }
-    };
-    load_xg(0, 0);
-    // the last two p commits cover every MMA1 step: n is complete
-#pragma unroll
-    for (int pb = 0; pb < 2; ++pb) {
-      if (!mbar_wait(smem_u32(mbars + pb), parp[pb])) __trap();
-      parp[pb] ^= 1u;
-    }
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    // ---- P2: q = dL/dn per 32-channel chunk -> q planes + global q; MMA2 ----
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int b = c & 1;
-      load_xg(b ^ 1, (c + 1) % NCH);
-      {
-        uint32_t acc[16];
-        tmem_load<16>(tmem_n + lane_sel + (uint32_t)(c * 32 + h * 16), acc);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        stage_store16(stage_n + r * kStLd + h * 16, acc);
-      }
-      if (c >= 2) {
-        if (!mbar_wait(smem_u32(mbars + 2 + b), parq[b])) __trap();
-        parq[b] ^= 1u;
-      }
-      compute_sync();
-      uint8_t* qh = smem + L::kOffQ + b * 2 * L::kPlaneQ;
-      uint8_t* ql = qh + L::kPlaneQ;
-      const float4 bv0 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8);
-      const float4 bv1 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8 + 4);
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int row = crow + 64 * it;
-        const float4 n0 = *reinterpret_cast<const float4*>(stage_n + row * kStLd + ckg * 8);
-        const float4 n1 = *reinterpret_cast<const float4*>(stage_n + row * kStLd + ckg * 8 + 4);
-        const float4 x0 = xq[b][it][0], x1 = xq[b][it][1], g0 = gq[b][it][0], g1 = gq[b][it][1];
-        float q[8];
-        q[0] = tc_dl_dn<FAST>(g0.x, x0.x, bv0.x + n0.x, f);
-        q[1] = tc_dl_dn<FAST>(g0.y, x0.y, bv0.y + n0.y, f);
-        q[2] = tc_dl_dn<FAST>(g0.z, x0.z, bv0.z + n0.z, f);
-        q[3] = tc_dl_dn<FAST>(g0.w, x0.w, bv0.w + n0.w, f);
-        q[4] = tc_dl_dn<FAST>(g1.x, x1.x, bv1.x + n1.x, f);
-        q[5] = tc_dl_dn<FAST>(g1.y, x1.y, bv1.y + n1.y, f);
-        q[6] = tc_dl_dn<FAST>(g1.z, x1.z, bv1.z + n1.z, f);
-        q[7] = tc_dl_dn<FAST>(g1.w, x1.w, bv1.w + n1.w, f);
-        uint4 hi, lo;
-        split8(q, &hi, &lo);
-        *reinterpret_cast<uint4*>(qh + ckg * kKg + row * 16) = hi;
-        *reinterpret_cast<uint4*>(ql + ckg * kKg + row * 16) = lo;
-        if (p0 + row < n_pix) {
-          float4* dst = reinterpret_cast<float4*>(q_out + (p0 + row) * C + c * 32 + ckg * 8);
-          __stcs(dst, make_float4(q[0], q[1], q[2], q[3]));
-          __stcs(dst + 1, make_float4(q[4], q[5], q[6], q[7]));
-        }
-      }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      asm volatile("bar.arrive %0, %1;" ::"r"(4 + b), "n"(kBwdThreads) : "memory");
-      compute_sync();  // staging free again
-    }
-    // ---- P3: dx = g / m + dpool/du * dp ----
-#pragma unroll
-    for (int b = 0; b < 2; ++b) {
-      if (!mbar_wait(smem_u32(mbars + 2 + b), parq[b])) __trap();
-      parq[b] ^= 1u;
-    }
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-    for (int c = 0; c < NCH; ++c) {
-      const int b = c & 1;
-      if (c + 1 < NCH) load_xg(b ^ 1, c + 1);
-      {
-        uint32_t an[16], ad[16];
-        tmem_load<16>(tmem_n + lane_sel + (uint32_t)(c * 32 + h * 16), an);
-        tmem_load<16>(tmem_dp + lane_sel + (uint32_t)(c * 32 + h * 16), ad);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        stage_store16(stage_n + r * kStLd + h * 16, an);
-        stage_store16(stage_d + r * kStLd + h * 16, ad);
-      }
-      compute_sync();
-      const float4 bv0 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8);
-      const float4 bv1 = *reinterpret_cast<const float4*>(beta_s + c * 32 + ckg * 8 + 4);
-#pragma unroll
-      for (int it = 0; it < 2; ++it) {
-        const int row = crow + 64 * it;
-        const float4 n0 = *reinterpret_cast<const float4*>(stage_n + row * kStLd + ckg * 8);
-        const float4 n1 = *reinterpret_cast<const float4*>(stage_n + row * kStLd + ckg * 8 + 4);
-        const float4 d0 = *reinterpret_cast<const float4*>(stage_d + row * kStLd + ckg * 8);
-        const float4 d1 = *reinterpret_cast<const float4*>(stage_d + row * kStLd + ckg * 8 + 4);
-        const float4 x0 = xq[b][it][0], x1 = xq[b][it][1], g0 = gq[b][it][0], g1 = gq[b][it][1];
-        float4 o0, o1;
-        o0.x = tc_dx<FAST>(g0.x, x0.x, bv0.x + n0.x, d0.x, f);
-        o0.y = tc_dx<FAST>(g0.y, x0.y, bv0.y + n0.y, d0.y, f);
-        o0.z = tc_dx<FAST>(g0.z, x0.z, bv0.z + n0.z, d0.z, f);
-        o0.w = tc_dx<FAST>(g0.w, x0.w, bv0.w + n0.w, d0.w, f);
-        o1.x = tc_dx<FAST>(g1.x, x1.x, bv1.x + n1.x, d1.x, f);
-        o1.y = tc_dx<FAST>(g1.y, x1.y, bv1.y + n1.y, d1.y, f);
-        o1.z = tc_dx<FAST>(g1.z, x1.z, bv1.z + n1.z, d1.z, f);
-        o1.w = tc_dx<FAST>(g1.w, x1.w, bv1.w + n1.w, d1.w, f);
-        if (p0 + row < n_pix) {
-          float4* dst = reinterpret_cast<float4*>(dx + (p0 + row) * C + c * 32 + ckg * 8);
-          __stcs(dst, o0);  // streaming stores: keep x / dy (re-read from L2) resident instead of the outputs
-          __stcs(dst + 1, o1);
-        }
-      }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      compute_sync();
-    }
-  }
-  }  // compute warps
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (tid < 32) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*tmem_slot), "n"(512));
-  }
-}
-
-template <int C>
-struct Bwd3Smem {
-  static constexpr int kPlane = (C / 8) * kKg;       // one full-K plane
-  static constexpr int kOffPh = 0;
-  static constexpr int kOffPl = kOffPh + kPlane;
-  static constexpr int kOffQh = kOffPl + kPlane;
-  static constexpr int kOffQl = kOffQh + kPlane;
-  static constexpr int kOffDbeta = kOffQl + kPlane;
-  static constexpr int kOffBar = kOffDbeta + C * 4;
-  static constexpr int kBytes = kOffBar + 64;
-  static_assert(kBytes <= 232448, "shared memory budget");
-};
-
-template <int C, bool FAST>
-__global__ void __launch_bounds__(kBwdThreads, 1)
-gdn_tc_bwd_dgamma_kernel(const float* __restrict__ x, const float* __restrict__ q, float* __restrict__ part_g,
-                         float* __restrict__ part_b, long long n_pix, TcFlags f) {
-  using L = Bwd3Smem<C>;
-  constexpr int KG = C / 8;                                     // 8-channel groups per row
-  constexpr int ITEMS = kTileM * KG / kBwdCompute;              // (row, kg) items per thread and array: 12
-  constexpr int PERIOD = 3;                                     // kg of a thread's items repeats with this period
-  static_assert(C == 192 && (kTileM * KG) % kBwdCompute == 0 && ITEMS % 4 == 0, "item mapping");
-  extern __shared__ __align__(1024) uint8_t smem[];
-  float* dbeta_s = reinterpret_cast<float*>(smem + L::kOffDbeta);
-  uint64_t* mbar = reinterpret_cast<uint64_t*>(smem + L::kOffBar);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + L::kOffBar + 16);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int r = tid & 127, h = (tid >> 7) & 1, gwarp = warp & 3;
-  constexpr uint32_t kIdesc = umma_idesc(kTileM, C) | (1u << 15) | (1u << 16);  // A = p^T, B = q, both MN-major views
-  for (int i = tid; i < C; i += kBwdThreads) dbeta_s[i] = 0.f;
-  if (tid == 0) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(mbar)));
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(512));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::);
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_a = *tmem_slot, tmem_b = tmem_a + C;  // rows j in [0,128) | rows j in [64,192)
-  const uint32_t lane_sel = (uint32_t)(gwarp * 32) << 16;
-  const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  int t_idx = 0;  // this CTA's tile counter (both roles count alike)
-
-  if (warp == kBwdCompute / 32) {
-    const uint32_t p_hi = smem_u32(smem + L::kOffPh), p_lo = smem_u32(smem + L::kOffPl);
-    const uint32_t q_hi = smem_u32(smem + L::kOffQh), q_lo = smem_u32(smem + L::kOffQl);
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t_idx) {
-      if (lane == 1) {
-        const long long pn = (tile + gridDim.x) * kTileM;
-        const long long rows = min((long long)kTileM, n_pix - pn);
-        if (rows > 0) {
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(x + pn * C), "r"((uint32_t)(rows * C * 4)) : "memory");
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(q + pn * C), "r"((uint32_t)(rows * C * 4)) : "memory");
-        }
-      }
-      asm volatile("bar.sync 2, %0;" ::"n"(kBwdThreads) : "memory");
-      if (lane == 0) {
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll 1
-        for (int blk = 0; blk < 2; ++blk) {
-          const uint32_t moff = (uint32_t)(blk * 8) * kKg;  // second block starts at channel 64 = m group 8
-          const uint32_t td = blk ? tmem_b : tmem_a;
-#pragma unroll
-          for (int s = 0; s < kTileM / 16; ++s) {
-            const uint32_t koff = (uint32_t)(s * 16) * 16u;
-            const uint64_t dah = umma_desc(p_hi + moff + koff, 128, kKg);
-            const uint64_t dal = umma_desc(p_lo + moff + koff, 128, kKg);
-            const uint64_t dbh = umma_desc(q_hi + koff, 128, kKg);
-            const uint64_t dbl = umma_desc(q_lo + koff, 128, kKg);
-            umma_bf16(td, dah, dbh, kIdesc, ((t_idx % kDgFlush) == 0 && s == 0) ? 0u : 1u);  // restarted after a flush
-            umma_bf16(td, dal, dbh, kIdesc, 1u);
-            umma_bf16(td, dah, dbl, kIdesc, 1u);
-          }
-        }
-        umma_commit(smem_u32(mbar));
-      }
-      __syncwarp();
-    }
-  } else {
-  uint32_t par = 0u;
-  bool flushed = false;  // the global partial holds earlier flushes
-  // block a: lane r = channel j = r; block b: lane r = channel 64 + r (only its rows >= 128 are new)
-  auto flush_dgamma = [&]() {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll 1
-    for (int blk = 0; blk < 2; ++blk) {
-      const int j = blk ? 64 + r : r;
-      float* pg = part_g + (long long)blockIdx.x * C * C + (long long)j * C + h * (C / 2);
-#pragma unroll
-      for (int cb = 0; cb < C / 32; ++cb) {
-        uint32_t a[16];
-        tmem_load<16>((blk ? tmem_b : tmem_a) + lane_sel + (uint32_t)(h * (C / 2) + cb * 16), a);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-        if (!blk || r >= 64) accum_store16(pg + cb * 16, a, flushed);
-      }
-    }
-    flushed = true;
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  };
-  float dbeta_acc[PERIOD][8];
-#pragma unroll
-  for (int a = 0; a < PERIOD; ++a)
-#pragma unroll
-    for (int e = 0; e < 8; ++e) dbeta_acc[a][e] = 0.f;
-  for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++t_idx) {
-    const long long p0 = tile * kTileM;
-    bool waited = t_idx == 0;
-#pragma unroll
-    for (int pass = 0; pass < ITEMS / 4; ++pass) {
-      float4 xv[4][2], qv[4][2];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int id = (pass * 4 + i) * kBwdCompute + tid;
-        const int row = id / KG, kg = id % KG;
-        const bool live = p0 + row < n_pix;
-        const long long off = (p0 + row) * C + kg * 8;
-        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-        xv[i][0] = live ? __ldg(reinterpret_cast<const float4*>(x + off)) : z;
-        xv[i][1] = live ? __ldg(reinterpret_cast<const float4*>(x + off) + 1) : z;
-        qv[i][0] = live ? __ldg(reinterpret_cast<const float4*>(q + off)) : z;
-        qv[i][1] = live ? __ldg(reinterpret_cast<const float4*>(q + off) + 1) : z;
-      }
-      if (!waited) {  // the planes are being read by the previous tile's MMAs
-        if (!mbar_wait(smem_u32(mbar), par)) __trap();
-        par ^= 1u;
-        waited = true;
-        if ((t_idx % kDgFlush) == 0) flush_dgamma();  // t_idx tiles are in the accumulator and complete
-      }
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const int j = pass * 4 + i;
-        const int id = j * kBwdCompute + tid;
-        const int row = id / KG, kg = id % KG;
-        const float4 a = xv[i][0], b = xv[i][1];
-        float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
-                      tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
-        uint4 hi, lo;
-        split8(v, &hi, &lo);
-        *reinterpret_cast<uint4*>(smem + L::kOffPh + kg * kKg + row * 16) = hi;
-        *reinterpret_cast<uint4*>(smem + L::kOffPl + kg * kKg + row * 16) = lo;
-        float w[8] = {qv[i][0].x, qv[i][0].y, qv[i][0].z, qv[i][0].w, qv[i][1].x, qv[i][1].y, qv[i][1].z, qv[i][1].w};
-        split8(w, &hi, &lo);
-        *reinterpret_cast<uint4*>(smem + L::kOffQh + kg * kKg + row * 16) = hi;
-        *reinterpret_cast<uint4*>(smem + L::kOffQl + kg * kKg + row * 16) = lo;
-#pragma unroll
-        for (int e = 0; e < 8; ++e) dbeta_acc[j % PERIOD][e] += w[e];
-      }
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    asm volatile("bar.arrive 2, %0;" ::"n"(kBwdThreads) : "memory");
-  }
-  if (t_idx > 0) {
-    if (!mbar_wait(smem_u32(mbar), par)) __trap();
-    // the tiles since the last flush (a flush is due at the top of a NEXT tile, so a full period may be pending)
-    flush_dgamma();
-#pragma unroll
-    for (int a = 0; a < PERIOD; ++a) {
-      const int kg = (a * kBwdCompute + tid) % KG;
-#pragma unroll
-      for (int e = 0; e < 8; ++e) atomicAdd(dbeta_s + kg * 8 + e, dbeta_acc[a][e]);
-    }
-  }
-  }  // compute warps
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  for (int i = tid; i < C; i += kBwdThreads) part_b[(long long)blockIdx.x * C + i] = dbeta_s[i];
-  if (tid < 32) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(*tmem_slot), "n"(512));
-  }
-}
-
-// =============================================================================================
-// Backward, C = 128, second kernel shape (the default GDN / IGDN: alpha = 1, epsilon = 1, no rectification).
-//
-// Same mathematics and the same operand planes / MN-major views as gdn_tc_bwd_kernel above, rebuilt along the
-// lines of the C = 192 forward: everything that touches HBM is an asynchronous 2-D TMA box, every compute thread
-// (r, h) owns pixel row r (= its TMEM lane) and 8 of the 32 channels of a box, so there are no staging
-// transposes and no CTA-wide barriers, and x and dy are read exactly once:
-//
-//   conv(t)   x boxes -> p = |x| hi / lo planes (whole K)                -> MMA1  n = p . gamma
-//             the raw x values are parked in 128 spare TMEM columns (tcgen05.st) for pass 2
-//   pass2(t)  g boxes + n, x from TMEM -> q hi / lo planes (whole tile, written 32 channels at a time)
-//                                                                         -> MMA2  dp += q_chunk . gamma^T  per chunk
-//             the direct term g / n (IGDN: g * n) goes back into n's TMEM columns with sign(x) in the two low
-//             mantissa bits (2 ulp, the contract is 1e-5): the dx pass needs neither x nor g again
-//   pass3(t)  dx = direct + sign(x) * dp  from TMEM only -> box -> TMA store;  meanwhile
-//                                                                         -> MMA3  dgamma += p^T q, 24 full-width MMAs
-//
-// (With 32-channel q buffers MMA3 was 96 MMAs of N = 32 per tile, each re-reading its 4 KB A operand from shared
-// memory for 16 cycles of math: switching them off saved 20 % of the kernel.)  The whole-tile q planes take the
-// place of the resident gamma planes: gamma (and gamma^T for MMA2) is streamed from L2 in 32-channel K chunks
-// (16 KB hi + lo, double buffered) by a "gamma" warp, 128 KB per tile.
-// One ring of four 16 KB boxes serves every box request in program order: g x 4 (pass 2), output x 4 (pass 3),
-// x x 4 (conversion of the CTA's next tile).  TMEM: n | dp | dgamma partial | parked x (4 x 128 columns).
-// HBM traffic: x, dy in, dx out, nothing else.
-// =============================================================================================
 __device__ __forceinline__ void tmem_store8(uint32_t taddr, const uint32_t (&r)[8]) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]),
                "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
@@ -1884,6 +1011,33 @@ __global__ void gdn_tc_prep2_kernel(const float* __restrict__ gamma, int C, __nv
   }
 }
 
+// =============================================================================================
+// Backward, C = 128: one fused kernel.
+//
+// Everything that touches HBM is an asynchronous 2-D TMA box, every compute thread (r, h) owns pixel row r (= its
+// TMEM lane) and 8 of the 32 channels of a box, so there are no staging transposes and no CTA-wide barriers, and x
+// and dy are read exactly once:
+//
+//   conv(t)   x boxes -> p = pool(x) hi / lo planes (whole K)            -> MMA1  n = p . gamma
+//             the raw x values are parked in 128 spare TMEM columns (tcgen05.st) for pass 2
+//   pass2(t)  g boxes + n, x from TMEM -> q hi / lo planes (whole tile, written 32 channels at a time)
+//                                                                         -> MMA2  dp += q_chunk . gamma^T  per chunk
+//             the direct term g / m (IGDN: g * m) goes back into n's TMEM columns; for the default GDN (FAST) with
+//             sign(x) in the two low mantissa bits (2 ulp, the contract is 1e-5), so that its dx pass needs neither
+//             x nor g again
+//   pass3(t)  dx = direct + dpool/du * dp  from TMEM -> box -> TMA store;  meanwhile
+//                                                                         -> MMA3  dgamma += p^T q, 24 full-width MMAs
+//             (the variants read dpool/du off the parked x: the next tile's conversion overwrites it only after
+//             this pass)
+//
+// (With 32-channel q buffers MMA3 was 96 MMAs of N = 32 per tile, each re-reading its 4 KB A operand from shared
+// memory for 16 cycles of math: switching them off saved 20 % of the kernel.)  The whole-tile q planes take the
+// place of resident gamma planes: gamma (and gamma^T for MMA2) is streamed from L2 in 32-channel K chunks
+// (16 KB hi + lo, double buffered) by a "gamma" warp, 128 KB per tile.
+// One ring of four 16 KB boxes serves every box request in program order: g x 4 (pass 2), output x 4 (pass 3),
+// x x 4 (conversion of the CTA's next tile).  TMEM: n | dp | dgamma partial | parked x (4 x 128 columns).
+// HBM traffic: x, dy in, dx out, nothing else.
+// =============================================================================================
 constexpr int kB3Compute = 512;                // 16 compute warps
 constexpr int kB3Threads = kB3Compute + 160;   // + two MMA-issue warps, box-copy, gamma and store warps
 constexpr int kB3SyncA = kB3Compute + 32;      // compute + first issue warp
@@ -1911,11 +1065,12 @@ struct BwdFusedSmem {
   static_assert(kBytes <= 232448, "shared memory budget");
 };
 
+template <bool FAST>
 __global__ void __launch_bounds__(kB3Threads, 1)
 gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constant__ CUtensorMap g_map,
                    const __grid_constant__ CUtensorMap dx_map, const float* __restrict__ x, const float* __restrict__ dy,
                    const __nv_bfloat16* __restrict__ planes, const float* __restrict__ beta, float* __restrict__ part_g,
-                   float* __restrict__ part_b, long long n_pix, int inverse, int dbg) {
+                   float* __restrict__ part_b, long long n_pix, TcFlags f) {
   using L = BwdFusedSmem;
   constexpr int C = L::C, NCH = C / 32;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -2144,24 +1299,20 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       if (lane == 0) {
         // let the tile's last MMA2s through first: the dx pass waits for them, nothing waits for MMA3 until the next
         // conversion (both issue warps leave the same barrier; 24 MMAs ahead of 6 cost the dx pass ~0.8 us per tile)
-        if (!(dbg & 8)) {
-          if (!mbar_wait(bar(L::kBarDp), (uint32_t)t & 1u)) __trap();
-        }
+        if (!mbar_wait(bar(L::kBarDp), (uint32_t)t & 1u)) __trap();
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         // dgamma[j, i] += sum_pix p[pix, j] q[pix, i]   (K = pix: 8 steps of 16)
-        if (!(dbg & 1)) {
-          const bool restart = (t == 0) || (((t + fphase) % kDgFlush) == 0);  // first MMA after a flush
+        const bool restart = (t == 0) || (((t + fphase) % kDgFlush) == 0);  // first MMA after a flush
 #pragma unroll
-          for (int s = 0; s < kTileM / 16; ++s) {
-            const uint32_t koff = (uint32_t)(s * 16) * 16u;
-            const uint64_t dah = umma_desc(p_hi + koff, 128, kKg);
-            const uint64_t dal = umma_desc(p_lo + koff, 128, kKg);
-            const uint64_t dbh = umma_desc(q_hi + koff, 128, kKg);
-            const uint64_t dbl = umma_desc(q_lo + koff, 128, kKg);
-            umma_bf16(tmem_dg, dah, dbh, kIdesc3, (restart && s == 0) ? 0u : 1u);
-            umma_bf16(tmem_dg, dal, dbh, kIdesc3, 1u);
-            umma_bf16(tmem_dg, dah, dbl, kIdesc3, 1u);
-          }
+        for (int s = 0; s < kTileM / 16; ++s) {
+          const uint32_t koff = (uint32_t)(s * 16) * 16u;
+          const uint64_t dah = umma_desc(p_hi + koff, 128, kKg);
+          const uint64_t dal = umma_desc(p_lo + koff, 128, kKg);
+          const uint64_t dbh = umma_desc(q_hi + koff, 128, kKg);
+          const uint64_t dbl = umma_desc(q_lo + koff, 128, kKg);
+          umma_bf16(tmem_dg, dah, dbh, kIdesc3, (restart && s == 0) ? 0u : 1u);
+          umma_bf16(tmem_dg, dal, dbh, kIdesc3, 1u);
+          umma_bf16(tmem_dg, dah, dbl, kIdesc3, 1u);
         }
         umma_commit(bar(L::kBarM3));
       }
@@ -2209,7 +1360,7 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
     flushed = true;
   };
 
-  // One tile: p = |x| -> hi / lo planes chunk by chunk (each chunk arrives on its own named barrier), raw x -> TMEM
+  // One tile: p = pool(x) -> hi / lo planes chunk by chunk (each chunk arrives on its own named barrier), raw x -> TMEM
   auto conv_tile = [&]() {
 #pragma unroll 1
     for (int c = 0; c < NCH; ++c, ++n) {
@@ -2220,7 +1371,8 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       const uint32_t raw[8] = {__float_as_uint(a.x), __float_as_uint(a.y), __float_as_uint(a.z), __float_as_uint(a.w),
                                __float_as_uint(b.x), __float_as_uint(b.y), __float_as_uint(b.z), __float_as_uint(b.w)};
       tmem_store8(tmem_x + lane_sel + (uint32_t)(c * 32 + h * 8), raw);
-      float v[8] = {fabsf(a.x), fabsf(a.y), fabsf(a.z), fabsf(a.w), fabsf(b.x), fabsf(b.y), fabsf(b.z), fabsf(b.w)};
+      float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
+                    tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
       uint4 hi, lo;
       split8(v, &hi, &lo);
       *reinterpret_cast<uint4*>(smem + L::kOffPh + (4 * c + h) * kKg + r * 16) = hi;
@@ -2238,7 +1390,7 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");  // this thread's parked x values are in TMEM
     if (!mbar_wait(bar(L::kBarN), (uint32_t)t & 1u)) __trap();  // MMA1 of this tile has completed
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    // ---- pass 2: q = dL/dn -> q planes; the direct term and sign(x) go back into n's columns ----
+    // ---- pass 2: q = dL/dn -> q planes; the direct term (FAST: and sign(x)) goes back into n's columns ----
 #pragma unroll
     for (int c = 0; c < NCH; ++c, ++n) {
       const uint32_t slot = n & 3u;
@@ -2260,17 +1412,9 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       for (int e = 0; e < 8; ++e) {
         const float xe = __uint_as_float(xraw[e]);
         const float nn = bs[e] + __uint_as_float(nacc[e]);
-        float direct;
-        if (inverse) {
-          direct = gs[e] * nn;
-          q[e] = gs[e] * xe;
-        } else {
-          const float rn = rcp_approx(nn);
-          direct = gs[e] * rn;
-          q[e] = -gs[e] * xe * rn * rn;
-        }
-        const uint32_t code = (xe > 0.f) ? 1u : ((xe < 0.f) ? 2u : 0u);
-        dbits[e] = (__float_as_uint(direct) & ~3u) | code;
+        q[e] = tc_dl_dn<FAST>(gs[e], xe, nn, f);
+        dbits[e] = __float_as_uint(tc_direct<FAST>(gs[e], nn, f));
+        if (FAST) dbits[e] = (dbits[e] & ~3u) | ((xe > 0.f) ? 1u : ((xe < 0.f) ? 2u : 0u));
         dbeta_acc[c][e] += q[e];
       }
       uint4 hi, lo;
@@ -2283,25 +1427,30 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       if (c == NCH - 1) asm volatile("bar.arrive %0, %1;" ::"r"(6 + c), "n"(kB3SyncB) : "memory");
       else asm volatile("bar.arrive %0, %1;" ::"r"(6 + c), "n"(kB3SyncA) : "memory");  // (also releases the g box)
     }
-    // ---- pass 3: dx = direct + sign(x) * dp, from TMEM only ----
+    // ---- pass 3: dx = direct + dpool/du * dp, from TMEM only ----
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");  // this thread's direct terms are in TMEM
     if (!mbar_wait(bar(L::kBarDp), (uint32_t)t & 1u)) __trap();  // every MMA2 of this tile has completed
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 #pragma unroll 1
     for (int c = 0; c < NCH; ++c, ++n) {
       const uint32_t slot = n & 3u, round = n >> 2;
-      uint32_t d[8], p[8];
+      uint32_t d[8], p[8], xraw[8];
       tmem_load<8>(tmem_n + lane_sel + (uint32_t)(c * 32 + h * 8), d);
       tmem_load<8>(tmem_dp + lane_sel + (uint32_t)(c * 32 + h * 8), p);
+      if (!FAST) tmem_load<8>(tmem_x + lane_sel + (uint32_t)(c * 32 + h * 8), xraw);
       uint8_t* box = smem + L::kOffRing + slot * kF4Box;
       if (!mbar_wait(bar(L::kBarFull + slot), round & 1u)) __trap();  // the slot's previous user has left
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
       float o[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
-        const uint32_t code = d[e] & 3u;
-        const float s = (code == 1u) ? 1.f : ((code == 2u) ? -1.f : 0.f);
-        o[e] = fmaf(s, __uint_as_float(p[e]), __uint_as_float(d[e]));
+        if (FAST) {
+          const uint32_t code = d[e] & 3u;
+          const float s = (code == 1u) ? 1.f : ((code == 2u) ? -1.f : 0.f);
+          o[e] = fmaf(s, __uint_as_float(p[e]), __uint_as_float(d[e]));
+        } else {
+          o[e] = tc_dx(__uint_as_float(d[e]), __uint_as_float(xraw[e]), __uint_as_float(p[e]), f);
+        }
       }
       *chunk_at(box, r, 2 * h) = make_float4(o[0], o[1], o[2], o[3]);
       *chunk_at(box, r, 2 * h + 1) = make_float4(o[4], o[5], o[6], o[7]);
@@ -2312,7 +1461,7 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
     // MMA3 of this tile has completed: the p and q planes are dead, the dgamma accumulator is up to date
     if (!mbar_wait(bar(L::kBarM3), (uint32_t)t & 1u)) __trap();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (((t + fphase) % kDgFlush) == kDgFlush - 1 && !(dbg & 4)) flush_dgamma();
+    if (((t + fphase) % kDgFlush) == kDgFlush - 1) flush_dgamma();
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");  // TMEM reads precede the next tile's MMAs
     if (has_next) conv_tile();
   }
@@ -2340,8 +1489,9 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
   }
 }
 
+template <bool FAST>
 int launch_tc_bwd3(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* part_g,
-                   float* part_b, int* n_parts, long long n_pix, int inverse, cudaStream_t s) {
+                   float* part_b, int* n_parts, long long n_pix, TcFlags f, cudaStream_t s) {
   constexpr int C = 128;
   using L = BwdFusedSmem;
   CUtensorMap x_map, g_map, dx_map;
@@ -2352,7 +1502,7 @@ int launch_tc_bwd3(const float* x, const float* gamma, const float* beta, const 
   TFCB_TRY(dev_alloc((void**)&planes, (size_t)4 * C * C * sizeof(__nv_bfloat16), s));
   gdn_tc_prep2_kernel<true><<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
   TFCB_LAUNCHED();
-  cudaError_t e = cudaFuncSetAttribute(gdn_tc_bwd3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kBytes);
+  cudaError_t e = cudaFuncSetAttribute(gdn_tc_bwd3_kernel<FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kBytes);
   if (e != cudaSuccess) {
     (void)cudaGetLastError();
     dev_free(planes, s);
@@ -2363,10 +1513,8 @@ int launch_tc_bwd3(const float* x, const float* gamma, const float* beta, const 
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
   const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
-  int dbg = 0;  // timing experiments only (results are wrong with any bit set): 1 no MMA3, 4 no dgamma flushes
-  if (const char* env = getenv("TFCB_GDN_DBG")) dbg = atoi(env);
-  gdn_tc_bwd3_kernel<<<grid, kB3Threads, L::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta, part_g, part_b, n_pix,
-                                                        inverse, dbg);
+  gdn_tc_bwd3_kernel<FAST><<<grid, kB3Threads, L::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta, part_g, part_b,
+                                                              n_pix, f);
   TFCB_LAUNCHED();
   e = cudaGetLastError();
   dev_free(planes, s);
@@ -2384,11 +1532,13 @@ int launch_tc_bwd3(const float* x, const float* gamma, const float* beta, const 
 // needs ([tile][hi, lo][24 groups][128 rows][8], 4 B/element like fp32): this kernel's q chunk buffers are bulk-stored
 // as they are, the second kernel bulk-loads a tile's planes with one copy and converts nothing.  Per 128-pixel tile:
 //
-//   conv(t)   x boxes -> p = |x| hi / lo planes, one 32-channel K chunk at a time (two chunk buffers)  -> MMA1  n += p_c . gamma_c
+//   conv(t)   x boxes -> p = pool(x) hi / lo planes, one 32-channel K chunk at a time (two chunk buffers) -> MMA1  n += p_c . gamma_c
 //   pass2(t)  x (L2 hit), g boxes + n from TMEM -> q hi / lo planes of the chunk (also bulk-stored to the workspace)
 //                                                                                                      -> MMA2  dp += q_c . gammaT_c
-//             the direct term g / n (IGDN: g * n) goes back into n's columns with sign(x) in the two low mantissa bits
-//   pass3(t)  dx = direct + sign(x) * dp, from TMEM only -> output box -> TMA store
+//             the direct term g / m (IGDN: g * m) goes back into n's columns; FAST: with sign(x) in the two low
+//             mantissa bits
+//   pass3(t)  dx = direct + dpool/du * dp, from TMEM (the variants read x again, plain loads that hit L2)
+//             -> output box -> TMA store
 //
 // gamma's hi plane is resident (72 KB; MMA2 reads it through the MN-major view); the lo planes of gamma (MMA1) and
 // gamma^T (MMA2) arrive as 12 KB K chunks, double buffered, from a "gamma" warp, and each chunk's two hi products are
@@ -2421,11 +1571,12 @@ struct BwdDx2Smem {
   static_assert(kBytes <= 232448, "shared memory budget");
 };
 
+template <bool FAST>
 __global__ void __launch_bounds__(kD2Threads, 1)
 gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constant__ CUtensorMap g_map,
                       const __grid_constant__ CUtensorMap dx_map, const float* __restrict__ x,
                       const float* __restrict__ dy, const __nv_bfloat16* __restrict__ planes,
-                      const float* __restrict__ beta, uint8_t* __restrict__ q_planes, long long n_pix, int inverse) {
+                      const float* __restrict__ beta, uint8_t* __restrict__ q_planes, long long n_pix, TcFlags f) {
   using L = BwdDx2Smem;
   constexpr int C = L::C, NCH = C / 32;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -2717,7 +1868,8 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
     for (int c = 0; c < NCH; ++c, ++n) {
       uint8_t* box = wait_full(n);
       const float4 a = *chunk_at(box, r, 2 * h), b = *chunk_at(box, r, 2 * h + 1);
-      float v[8] = {fabsf(a.x), fabsf(a.y), fabsf(a.z), fabsf(a.w), fabsf(b.x), fabsf(b.y), fabsf(b.z), fabsf(b.w)};
+      float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
+                    tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
       uint4 hi, lo, *ph, *pl;
       split8(v, &hi, &lo);
       operand_rows(&ph, &pl, after_pass2 && c < 2);  // chunks 0, 1 reuse the buffers of the tile's last two q chunks
@@ -2736,7 +1888,7 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
     const bool has_next = tile + gridDim.x < n_tiles;
     if (!mbar_wait(bar(L::kBarN), (uint32_t)t & 1u)) __trap();  // MMA1 of this tile has completed
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    // ---- pass 2: q = dL/dn -> output box + q planes; the direct term and sign(x) go back into n's columns ----
+    // ---- pass 2: q = dL/dn -> q planes; the direct term (FAST: and sign(x)) goes back into n's columns ----
 #pragma unroll 1
     for (int c = 0; c < NCH; ++c, n += 2) {
       const uint32_t col = tmem_n + lane_sel + (uint32_t)(c * 32 + h * 8);
@@ -2757,17 +1909,9 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const float nn = bs[e] + __uint_as_float(nacc[e]);
-        float direct;
-        if (inverse) {
-          direct = gs[e] * nn;
-          q[e] = gs[e] * xs[e];
-        } else {
-          const float rn = rcp_approx(nn);
-          direct = gs[e] * rn;
-          q[e] = -gs[e] * xs[e] * rn * rn;
-        }
-        const uint32_t code = (xs[e] > 0.f) ? 1u : ((xs[e] < 0.f) ? 2u : 0u);
-        dbits[e] = (__float_as_uint(direct) & ~3u) | code;
+        q[e] = tc_dl_dn<FAST>(gs[e], xs[e], nn, f);
+        dbits[e] = __float_as_uint(tc_direct<FAST>(gs[e], nn, f));
+        if (FAST) dbits[e] = (dbits[e] & ~3u) | ((xs[e] > 0.f) ? 1u : ((xs[e] < 0.f) ? 2u : 0u));
       }
       uint4 hi, lo, *qh, *ql;
       split8(q, &hi, &lo);
@@ -2782,7 +1926,7 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
       if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(L::kBarQready + (m & 1u))) : "memory");
       ++m;
     }
-    // ---- pass 3: dx = direct + sign(x) * dp, from TMEM only ----
+    // ---- pass 3: dx = direct + dpool/du * dp (FAST: from TMEM only) ----
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");  // this thread's direct terms are in TMEM
     if (!mbar_wait(bar(L::kBarDp), (uint32_t)t & 1u)) __trap();  // every MMA2 of this tile has completed
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -2791,14 +1935,27 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
       uint32_t d[8], p[8];
       tmem_load<8>(tmem_n + lane_sel + (uint32_t)(c * 32 + h * 8), d);
       tmem_load<8>(tmem_dp + lane_sel + (uint32_t)(c * 32 + h * 8), p);
+      float4 x0, x1;  // the variants: this thread's 8 values of x, read again (TMEM has no room to park them)
+      if (!FAST) {
+        const long long row = tile * kTileM + r;
+        const float4* src = reinterpret_cast<const float4*>(x + row * C + c * 32 + h * 8);
+        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+        x0 = row < n_pix ? __ldg(src) : z;
+        x1 = row < n_pix ? __ldg(src + 1) : z;
+      }
       uint8_t* box = wait_full(n);  // the slot's previous user has left
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+      const float xs[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
       float o[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
-        const uint32_t code = d[e] & 3u;
-        const float s = (code == 1u) ? 1.f : ((code == 2u) ? -1.f : 0.f);
-        o[e] = fmaf(s, __uint_as_float(p[e]), __uint_as_float(d[e]));
+        if (FAST) {
+          const uint32_t code = d[e] & 3u;
+          const float s = (code == 1u) ? 1.f : ((code == 2u) ? -1.f : 0.f);
+          o[e] = fmaf(s, __uint_as_float(p[e]), __uint_as_float(d[e]));
+        } else {
+          o[e] = tc_dx(__uint_as_float(d[e]), xs[e], __uint_as_float(p[e]), f);
+        }
       }
       *chunk_at(box, r, 2 * h) = make_float4(o[0], o[1], o[2], o[3]);
       *chunk_at(box, r, 2 * h + 1) = make_float4(o[4], o[5], o[6], o[7]);
@@ -2822,7 +1979,7 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
 //
 // Per 128-pixel tile: the tile's q hi / lo planes arrive from the workspace with ONE bulk copy (96 KB, written in
 // exactly this layout by gdn_tc_bwd_dx2_kernel); the x tile (six TMA boxes, 96 KB) lands IN THE MEMORY OF THE p PLANES
-// (same size), every compute thread (r, h) takes its 48 values into registers, and after a barrier the p = |x| hi / lo
+// (same size), every compute thread (r, h) takes its 48 values into registers, and after a barrier the p = pool(x) hi / lo
 // planes are written over the boxes; 48 MMAs (two overlapping M = 128 row blocks [0,128) and [64,192) of p^T, N = 192,
 // K = 128 pixels) accumulate into TMEM.  Nothing is double buffered (4 x 48 KB of planes): a tile costs one load
 // latency + the conversion + the MMAs.  dbeta comes from the planes (q = hi + lo to 2^-17): warp w sums 8-channel
@@ -2849,10 +2006,11 @@ struct BwdDg2Smem {
   static_assert(2 * kPlane == 6 * kF4Box && 2 * kPlane >= kTileM * C * 4, "x tile / flush staging fit in the p planes");
 };
 
+template <bool FAST>
 __global__ void __launch_bounds__(kG2Threads, 1)
 gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float* __restrict__ x,
                           const uint8_t* __restrict__ q_planes, float* __restrict__ part_g, float* __restrict__ part_b,
-                          long long n_pix) {
+                          long long n_pix, TcFlags f) {
   using L = BwdDg2Smem;
   constexpr int C = L::C, NCH = C / 32;
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -3023,8 +2181,8 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
     asm volatile("bar.sync 1, %0;" ::"n"(kG2Compute) : "memory");  // every thread holds its values
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
-      float v[8] = {fabsf(xa[c].x), fabsf(xa[c].y), fabsf(xa[c].z), fabsf(xa[c].w),
-                    fabsf(xb[c].x), fabsf(xb[c].y), fabsf(xb[c].z), fabsf(xb[c].w)};
+      float v[8] = {tc_pool<FAST>(xa[c].x, f), tc_pool<FAST>(xa[c].y, f), tc_pool<FAST>(xa[c].z, f), tc_pool<FAST>(xa[c].w, f),
+                    tc_pool<FAST>(xb[c].x, f), tc_pool<FAST>(xb[c].y, f), tc_pool<FAST>(xb[c].z, f), tc_pool<FAST>(xb[c].w, f)};
       uint4 hi, lo;
       split8(v, &hi, &lo);
       *reinterpret_cast<uint4*>(smem + L::kOffPh + (4 * c + h) * kDKg + r * 16) = hi;
@@ -3080,118 +2238,42 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
   }
 }
 
+// q travels from the dx kernel to the dgamma kernel as bf16 hi / lo planes ([tile][2][24][128][8], 4 B/element; the
+// workspace is sized in whole tiles, tfcb_gdn_backward_workspace_bytes)
 template <bool FAST>
 int launch_tc_bwd192(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* q_ws,
                      float* part_g, float* part_b, int* n_parts, long long n_pix, TcFlags f, cudaStream_t s) {
   constexpr int C = 192;
-  __nv_bfloat16* planes = nullptr;
-  TFCB_TRY(dev_alloc((void**)&planes, (size_t)2 * C * C * sizeof(__nv_bfloat16), s));
-  gdn_tc_prep_kernel<<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
-  TFCB_LAUNCHED();
-  bool attr_set = false;  // the attribute is per device: set it on every launch (microseconds)
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(gdn_tc_bwd_dx_kernel<C, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         Bwd2Smem<C>::kBytes);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(gdn_tc_bwd_dgamma_kernel<C, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               Bwd3Smem<C>::kBytes);
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      dev_free(planes, s);
-      return fail(TFCB_CUDA_ERROR, "cannot reserve shared memory for the C=192 backward: %s", cudaGetErrorString(e));
-    }
-    attr_set = true;
+  using L2 = BwdDx2Smem;
+  using L3 = BwdDg2Smem;
+  CUtensorMap x_map, g_map, dx_map, x_map3;  // x_map3: the whole [128 x 192] x tile as one 3-D box
+  TFCB_TRY(make_tensor_map_2d(&x_map, x, n_pix, C, kTileM, 32, true));
+  TFCB_TRY(make_tensor_map_2d(&g_map, dy, n_pix, C, kTileM, 32, true));
+  TFCB_TRY(make_tensor_map_2d(&dx_map, dx, n_pix, C, kTileM, 32, true));
+  TFCB_TRY(make_tensor_map_3d(&x_map3, x, n_pix, C, kTileM, C / 32));
+  if (cudaFuncSetAttribute(gdn_tc_bwd_dx2_kernel<FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L2::kBytes) != cudaSuccess ||
+      cudaFuncSetAttribute(gdn_tc_bwd_dgamma2_kernel<FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L3::kBytes) != cudaSuccess) {
+    (void)cudaGetLastError();
+    return fail(TFCB_CUDA_ERROR, "cannot reserve shared memory for the C=192 backward");
   }
+  __nv_bfloat16* planes = nullptr;
+  TFCB_TRY(dev_alloc((void**)&planes, (size_t)4 * C * C * sizeof(__nv_bfloat16), s));
+  gdn_tc_prep2_kernel<false><<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
+  TFCB_LAUNCHED();
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
   const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
-  const char* v1 = getenv("TFCB_GDN_BWD_V1");  // A/B timing: the register-fed kernels
-  if (FAST && n_pix < (1ll << 31) && !(v1 && v1[0] == '1')) {
-    // box-fed pair: q travels as bf16 hi / lo planes ([tile][2][24][128][8], 4 B/element; the workspace is sized in
-    // whole tiles, tfcb_gdn_backward_workspace_bytes)
-    using L2 = BwdDx2Smem;
-    using L3 = BwdDg2Smem;
-    CUtensorMap x_map, g_map, dx_map;
-    __nv_bfloat16* planes4 = nullptr;
-    int rc = make_tensor_map_2d(&x_map, x, n_pix, C, kTileM, 32, true);
-    if (rc == TFCB_OK) rc = make_tensor_map_2d(&g_map, dy, n_pix, C, kTileM, 32, true);
-    if (rc == TFCB_OK) rc = make_tensor_map_2d(&dx_map, dx, n_pix, C, kTileM, 32, true);
-    if (rc == TFCB_OK) rc = dev_alloc((void**)&planes4, (size_t)4 * C * C * sizeof(__nv_bfloat16), s);
-    if (rc == TFCB_OK && (cudaFuncSetAttribute(gdn_tc_bwd_dx2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L2::kBytes) != cudaSuccess ||
-                          cudaFuncSetAttribute(gdn_tc_bwd_dgamma2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, L3::kBytes) != cudaSuccess)) {
-      (void)cudaGetLastError();
-      rc = fail(TFCB_CUDA_ERROR, "cannot reserve shared memory for the C=192 backward");
-    }
-    if (rc != TFCB_OK) {
-      dev_free(planes4, s);
-      dev_free(planes, s);
-      return rc;
-    }
-    gdn_tc_prep2_kernel<false><<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes4);
-    TFCB_LAUNCHED();
-    gdn_tc_bwd_dx2_kernel<<<grid, kD2Threads, L2::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes4, beta,
-                                                              reinterpret_cast<uint8_t*>(q_ws), n_pix, f.inverse);
-    TFCB_LAUNCHED();
-    CUtensorMap x_map3;  // the whole [128 x 192] x tile as one 3-D box
-    rc = make_tensor_map_3d(&x_map3, x, n_pix, C, kTileM, C / 32);
-    if (rc != TFCB_OK) {
-      dev_free(planes4, s);
-      dev_free(planes, s);
-      return rc;
-    }
-    gdn_tc_bwd_dgamma2_kernel<<<grid, kG2Threads, L3::kBytes, s>>>(x_map3, x, reinterpret_cast<const uint8_t*>(q_ws), part_g,
-                                                                   part_b, n_pix);
-    TFCB_LAUNCHED();
-    cudaError_t e2 = cudaGetLastError();
-    dev_free(planes4, s);
-    dev_free(planes, s);
-    if (e2 != cudaSuccess) return fail(TFCB_CUDA_ERROR, "GDN tensor-core backward (C=192) launch failed: %s", cudaGetErrorString(e2));
-    *n_parts = grid;
-    return TFCB_OK;
-  }
-  gdn_tc_bwd_dx_kernel<C, FAST><<<grid, kBwdThreads, Bwd2Smem<C>::kBytes, s>>>(x, dy, planes, beta, dx, q_ws, n_pix, f);
+  gdn_tc_bwd_dx2_kernel<FAST><<<grid, kD2Threads, L2::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta,
+                                                                  reinterpret_cast<uint8_t*>(q_ws), n_pix, f);
   TFCB_LAUNCHED();
-  gdn_tc_bwd_dgamma_kernel<C, FAST><<<grid, kBwdThreads, Bwd3Smem<C>::kBytes, s>>>(x, q_ws, part_g, part_b, n_pix, f);
+  gdn_tc_bwd_dgamma2_kernel<FAST><<<grid, kG2Threads, L3::kBytes, s>>>(x_map3, x, reinterpret_cast<const uint8_t*>(q_ws),
+                                                                       part_g, part_b, n_pix, f);
   TFCB_LAUNCHED();
-  cudaError_t e = cudaGetLastError();
+  const cudaError_t e = cudaGetLastError();
   dev_free(planes, s);
   if (e != cudaSuccess) return fail(TFCB_CUDA_ERROR, "GDN tensor-core backward (C=192) launch failed: %s", cudaGetErrorString(e));
-  *n_parts = grid;
-  return TFCB_OK;
-}
-
-template <bool FAST>
-int launch_tc_bwd(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* part_g,
-                  float* part_b, int* n_parts, long long n_pix, TcFlags f, cudaStream_t s) {
-  constexpr int C = 128;
-  using L = BwdSmem<C>;
-  __nv_bfloat16* planes = nullptr;
-  TFCB_TRY(dev_alloc((void**)&planes, (size_t)2 * C * C * sizeof(__nv_bfloat16), s));
-  gdn_tc_prep_kernel<<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
-  TFCB_LAUNCHED();
-  bool attr_set = false;  // the attribute is per device: set it on every launch (microseconds)
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(gdn_tc_bwd_kernel<C, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         L::kBytes);
-    if (e != cudaSuccess) {
-      (void)cudaGetLastError();
-      dev_free(planes, s);
-      return fail(TFCB_CUDA_ERROR, "cannot reserve %d bytes of shared memory: %s", L::kBytes, cudaGetErrorString(e));
-    }
-    attr_set = true;
-  }
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
-  gdn_tc_bwd_kernel<C, FAST><<<grid, kBwdThreads, L::kBytes, s>>>(x, dy, planes, beta, dx, part_g, part_b, n_pix, f);
-  TFCB_LAUNCHED();
-  cudaError_t e = cudaGetLastError();
-  dev_free(planes, s);
-  if (e != cudaSuccess) return fail(TFCB_CUDA_ERROR, "GDN tensor-core backward launch failed: %s", cudaGetErrorString(e));
   *n_parts = grid;
   return TFCB_OK;
 }
@@ -3205,9 +2287,6 @@ int gdn_tc_forward(const float* x, const float* gamma, const float* beta, float*
   if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return TFCB_OK;
   if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return TFCB_OK;  // trainable exponents: literal pow
   if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(beta)) & 15) return TFCB_OK;  // 16-byte rows
-  if (const char* env = getenv("TFCB_GDN_FP32")) {
-    if (env[0] == '1') return TFCB_OK;  // debugging aid: force the CUDA-core kernels
-  }
   TcFlags f;
   f.inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
   f.rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
@@ -3258,9 +2337,7 @@ int gdn_tc_backward(const float* x, const float* gamma, const float* beta, const
   if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return TFCB_OK;
   if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return TFCB_OK;  // trainable exponents: literal pow
   if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dx)) & 15) return TFCB_OK;
-  if (const char* env = getenv("TFCB_GDN_FP32")) {
-    if (env[0] == '1') return TFCB_OK;
-  }
+  if (n_pix >= (1ll << 31)) return TFCB_OK;  // the box kernels take 32-bit TMA row coordinates
   TcFlags f;
   f.inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
   f.rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
@@ -3268,16 +2345,11 @@ int gdn_tc_backward(const float* x, const float* gamma, const float* beta, const
   f.eps_mode = (eps == 0.5f) ? 2 : 1;
   *handled = true;
   const bool fast = (alpha == 1.f) && (eps == 1.f) && !f.rectify;
-  if (C == 192)
-    return fast ? launch_tc_bwd192<true>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s)
-                : launch_tc_bwd192<false>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
-  // C == 128.  The default GDN / IGDN goes through the box-fed kernel; TFCB_GDN_BWD_V1=1 keeps the register-fed one
-  // (A/B timing), which also serves the alpha = 2 / epsilon = 1/2 / rectified variants.
-  const char* v1 = getenv("TFCB_GDN_BWD_V1");
-  if (fast && n_pix < (1ll << 31) && !(v1 && v1[0] == '1'))
-    return launch_tc_bwd3(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f.inverse, s);
-  return fast ? launch_tc_bwd<true>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s)
-              : launch_tc_bwd<false>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+  if (C == 128)
+    return fast ? launch_tc_bwd3<true>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s)
+                : launch_tc_bwd3<false>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+  return fast ? launch_tc_bwd192<true>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s)
+              : launch_tc_bwd192<false>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
 }
 
 }  // namespace tfcb

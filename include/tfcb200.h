@@ -204,7 +204,7 @@ int tfcb_stochastic_round(const void* inputs_dev, int dtype, int64_t n, float st
  * alpha in {1, 2} and eps in {1, 0.5} take the reference's fast paths; other values use powf.
  * C in {128, 192} with those alpha / eps and 16-byte aligned pointers run on the tensor cores (bf16 split with
  * fp32 accumulation: <= 1e-5 relative forward, <= 2e-5 of the largest gradient backward); every other shape
- * runs the fp32 kernels.  TFCB_GDN_FP32=1 in the environment forces the fp32 kernels.
+ * runs the fp32 kernels.
  * The reference has no native GDN code (TF graph of abs / conv1x1 / bias_add / div); the backward
  * pass replaces TF autodiff of that graph.
  * ---------------------------------------------------------------------------------------------- */

@@ -103,10 +103,12 @@ def test_backward_vs_fp64_oracle(F, C, n_pix, inverse):
 @pytest.mark.parametrize("C", [64, 128, 192])
 @pytest.mark.parametrize("alpha,epsilon,rectify", [(1, 1, True), (2, 0.5, False), (2, 1, False), (1, 0.5, False),
                                                    (1.5, 0.7, True)])
-def test_backward_variants(F, C, alpha, epsilon, rectify):
+# 700 pixels are 6 tiles, one per CTA; 297 tiles give every CTA of a 148-SM grid a second tile (dgamma flushes)
+@pytest.mark.parametrize("n_pix", [700, 128 * 148 * 2 + 77])
+def test_backward_variants(F, C, alpha, epsilon, rectify, n_pix):
   gamma, beta = _params(C, 21)
-  x = _x(700, C, 22)
-  dy = torch.randn(700, C, generator=torch.Generator().manual_seed(23))
+  x = _x(n_pix, C, 22)
+  dy = torch.randn(n_pix, C, generator=torch.Generator().manual_seed(23))
   for inverse in (False, True):
     wx, wg, wb = gdn_oracle.gdn_reference_grads(x, gamma, beta, dy, inverse, rectify, alpha, epsilon)
     dx, dg, db = F.gdn_backward(x.cuda(), gamma.cuda(), beta.cuda(), dy.cuda(), inverse, rectify, alpha, epsilon)
