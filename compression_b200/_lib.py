@@ -70,6 +70,7 @@ SIGNATURES = {
     "tfcb_gdn_exponent_grads_workspace_bytes": (_i64, []),
     "tfcb_gdn_exponent_grads": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _f32, _f32, _vp]),
     "tfcb_gdn_backward": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _f32, _f32, _vp]),
+    "tfcb_gdn_backward_16bit": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _f32, _f32, _vp]),
 }
 
 _lib = None

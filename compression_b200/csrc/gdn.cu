@@ -485,6 +485,9 @@ int gdn_tc_forward16(const void* x, const float* gamma, const float* beta, void*
 int gdn_tc_backward(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* q_ws,
                     float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
                     float eps, cudaStream_t s, bool* handled);
+int gdn_tc_backward16(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
+                      float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
+                      float eps, int dtype, cudaStream_t s, bool* handled);
 
 }  // namespace tfcb
 
@@ -540,8 +543,9 @@ int tfcb_gdn_forward_16bit(const void* x_dev, const float* gamma_dev, const floa
   bool handled = false;
   TFCB_TRY(gdn_tc_forward16(x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, flags, alpha, epsilon, dtype, as_stream(stream), &handled));
   if (!handled)
-    return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: only C = 128 with alpha in {1, 2}, epsilon in {1, 1/2} has a native 16-bit kernel; "
-                "convert to float32 for this configuration");
+    return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: only C in {128, 192} with fixed alpha in {1, 2}, epsilon in {1, 1/2}, 16-byte "
+                "aligned x / y / beta (and fewer than 2^31 pixels at C = 192) has a native 16-bit kernel; convert to float32 "
+                "for this configuration");
   TFCB_CUDA_TRY(cudaGetLastError());
   return TFCB_OK;
 }
@@ -550,6 +554,40 @@ int64_t tfcb_gdn_backward_workspace_bytes(int64_t n_pix, int C) {
   const int64_t q = ((n_pix + 127) / 128 * 128) * C * (int64_t)sizeof(float);  // whole 128-pixel tiles (the C = 192 tensor-core pair hands q over tile by tile)
   const int64_t parts = (int64_t)kDgammaGrid * ((int64_t)C * C + C) * (int64_t)sizeof(float);
   return q + parts + 256;
+}
+
+int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, const void* dy_dev,
+                            void* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix, int C,
+                            int dtype, int flags, float alpha, float epsilon, void* stream) {
+  if (n_pix < 0 || C <= 0) return fail(TFCB_INVALID_ARGUMENT, "bad GDN shape: n_pix=%lld C=%d", (long long)n_pix, C);
+  if (dtype != 1 && dtype != 2) return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: dtype must be 1 (float16) or 2 (bfloat16)");
+  if (!x_dev || !gamma_dev || !beta_dev || !dy_dev || !dx_dev || !dgamma_dev || !dbeta_dev || !workspace_dev)
+    return fail(TFCB_INVALID_ARGUMENT, "null pointer");
+  cudaStream_t s = as_stream(stream);
+  if (n_pix == 0) {
+    TFCB_CUDA_TRY(cudaMemsetAsync(dgamma_dev, 0, (size_t)C * C * sizeof(float), s));
+    TFCB_CUDA_TRY(cudaMemsetAsync(dbeta_dev, 0, (size_t)C * sizeof(float), s));
+    return TFCB_OK;
+  }
+  // the same workspace layout as the float32 entry: q (C = 192: bf16 operand planes), then the per-CTA partials
+  float* q = reinterpret_cast<float*>(workspace_dev);
+  float* part_g = q + (size_t)((n_pix + 127) / 128 * 128) * C;
+  float* part_b = part_g + (size_t)kDgammaGrid * C * C;
+  bool handled = false;
+  int n_parts = 0;
+  TFCB_TRY(gdn_tc_backward16(x_dev, gamma_dev, beta_dev, dy_dev, dx_dev, q, part_g, part_b, &n_parts, n_pix, C, flags,
+                             alpha, epsilon, dtype, s, &handled));
+  if (!handled)
+    return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit backward: only C in {128, 192} with fixed alpha in {1, 2}, epsilon in "
+                "{1, 1/2}, 16-byte aligned x / dy / dx / workspace and fewer than 2^31 pixels has a native 16-bit kernel; "
+                "convert to float32 for this configuration");
+  const long long ng = (long long)C * C;
+  reduce_partials_kernel<<<(unsigned)((ng + 255) / 256), 256, 0, s>>>(part_g, n_parts, ng, dgamma_dev);
+  reduce_partials_kernel<<<(unsigned)((C + 255) / 256), 256, 0, s>>>(part_b, n_parts, C, dbeta_dev);
+  TFCB_LAUNCHED();
+  TFCB_LAUNCHED();
+  TFCB_CUDA_TRY(cudaGetLastError());
+  return TFCB_OK;
 }
 
 int tfcb_gdn_backward(const float* x_dev, const float* gamma_dev, const float* beta_dev, const float* dy_dev,

@@ -7,14 +7,16 @@
 // error-compensated bf16 split (3 products: hi*hi + lo*hi + hi*lo, fp32 accumulation in TMEM), which keeps the
 // result within ~4e-6 of fp32 (SURVEY.md App. D; the contract is 1e-5) at bf16 tensor throughput.
 // Every kernel is persistent (one CTA per SM, 128-pixel tiles) and specialised at compile time for FAST, the default
-// GDN / IGDN (alpha = 1, epsilon = 1, no rectification); the other instantiation honours TcFlags at run time.
+// GDN / IGDN (alpha = 1, epsilon = 1, no rectification); the other instantiation honours TcFlags at run time.  IO is
+// the element type of the activations x, dy, y, dx in memory (0 float32, 1 float16, 2 bfloat16; see IoBytes): 16-bit
+// elements are widened exactly on load and rounded once at the store, everything else is the same for every IO.
 //
-//   gdn_tc_fwd2_kernel<FAST, IO>     forward, C = 128, fp32 / fp16 / bf16 activations: the x tile resident in shared
-//                                    memory (bulk async copies), y written over it in place
-//   gdn_tc_fwd4_kernel<C, FAST>      forward, C = 192: x in 2-D TMA boxes, gamma's lo plane streamed
-//   gdn_tc_bwd3_kernel<FAST>         backward, C = 128: dx and the per-CTA dgamma / dbeta partials in one kernel
-//   gdn_tc_bwd_dx2_kernel<FAST>      backward, C = 192: dx and q = dL/dn (handed over as bf16 operand planes)
-//   gdn_tc_bwd_dgamma2_kernel<FAST>  backward, C = 192: dgamma / dbeta partials from x and q
+//   gdn_tc_fwd2_kernel<FAST, IO>         forward, C = 128: the x tile resident in shared memory (bulk async
+//                                        copies), y written over it in place
+//   gdn_tc_fwd4_kernel<C, FAST, IO>      forward, C = 192: x in 2-D TMA boxes, gamma's lo plane streamed
+//   gdn_tc_bwd3_kernel<FAST, IO>         backward, C = 128: dx and the per-CTA dgamma / dbeta partials in one kernel
+//   gdn_tc_bwd_dx2_kernel<FAST, IO>      backward, C = 192: dx and q = dL/dn (handed over as bf16 operand planes)
+//   gdn_tc_bwd_dgamma2_kernel<FAST, IO>  backward, C = 192: dgamma / dbeta partials from x and q
 //   gdn_tc_prep_kernel, gdn_tc_prep2_kernel   gamma -> bf16 hi / lo operand planes
 //
 // Everything outside {C in {128, 192}, alpha in {1, 2}, eps in {1, 0.5}} (and trainable exponents) runs the fp32
@@ -22,6 +24,8 @@
 #include <cuda.h>  // CUtensorMap (types only; cuTensorMapEncodeTiled is fetched through the runtime)
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -214,8 +218,7 @@ template <int IO>
 struct IoBytes { static constexpr int value = IO == 0 ? 4 : 2; };
 
 template <int IO>
-__device__ __forceinline__ void io_load8(const uint8_t* src, float (&v)[8]) {  // 8 consecutive 16-bit elements
-  const uint4 raw = *reinterpret_cast<const uint4*>(src);
+__device__ __forceinline__ void io_widen8(const uint4 raw, float (&v)[8]) {  // 8 consecutive 16-bit elements, exactly
   const uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
@@ -232,6 +235,11 @@ __device__ __forceinline__ void io_load8(const uint8_t* src, float (&v)[8]) {  /
 }
 
 template <int IO>
+__device__ __forceinline__ void io_load8(const uint8_t* src, float (&v)[8]) {
+  io_widen8<IO>(*reinterpret_cast<const uint4*>(src), v);
+}
+
+template <int IO>
 __device__ __forceinline__ void io_store8(uint8_t* dst, const float (&v)[8]) {
   uint32_t w[4];
 #pragma unroll
@@ -244,6 +252,46 @@ __device__ __forceinline__ void io_store8(uint8_t* dst, const float (&v)[8]) {
     }
   }
   *reinterpret_cast<uint4*>(dst) = make_uint4(w[0], w[1], w[2], w[3]);
+}
+
+// One [128 rows x 32 channels] TMA box of x / dy / dx in shared memory (the C = 192 forward and every backward kernel):
+//   float32: 128-byte rows, 128-byte swizzle: 16-byte chunk j (4 channels) of row r sits at chunk j ^ (r & 7);
+//   16-bit:   64-byte rows,  64-byte swizzle: 16-byte chunk j (8 channels) of row r sits at chunk j ^ ((r >> 1) & 3).
+// The thread that owns row r and channel octet `oct` of a box moves its 8 values with two 16-byte accesses (float32)
+// or one (16-bit).  Both are conflict free: the 8 lanes of each 16-byte access phase are 8 consecutive rows, which
+// land on 8 different 16-byte bank groups.  A ring slot keeps the float32 size (kF4Box below); a 16-bit box fills half.
+template <int IO>
+struct Box {
+  static constexpr int kRowB = 32 * IoBytes<IO>::value;  // bytes per box row
+  static constexpr int kBytes = kTileM * kRowB;          // bytes per box: the expect_tx count of one copy
+};
+
+template <int IO>
+__device__ __forceinline__ uint8_t* box_chunk(uint8_t* box, int row, int j) {  // 16-byte chunk j of box row `row`
+  if constexpr (IO == 0) return box + row * 128 + ((j ^ (row & 7)) << 4);
+  else return box + row * 64 + ((j ^ ((row >> 1) & 3)) << 4);
+}
+
+template <int IO>
+__device__ __forceinline__ void box_load8(uint8_t* box, int row, int oct, float (&v)[8]) {
+  if constexpr (IO == 0) {
+    const float4 a = *reinterpret_cast<const float4*>(box_chunk<0>(box, row, 2 * oct));
+    const float4 b = *reinterpret_cast<const float4*>(box_chunk<0>(box, row, 2 * oct + 1));
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w;
+    v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+  } else {
+    io_load8<IO>(box_chunk<IO>(box, row, oct), v);  // widened exactly
+  }
+}
+
+template <int IO>
+__device__ __forceinline__ void box_store8(uint8_t* box, int row, int oct, const float (&v)[8]) {
+  if constexpr (IO == 0) {
+    *reinterpret_cast<float4*>(box_chunk<0>(box, row, 2 * oct)) = make_float4(v[0], v[1], v[2], v[3]);
+    *reinterpret_cast<float4*>(box_chunk<0>(box, row, 2 * oct + 1)) = make_float4(v[4], v[5], v[6], v[7]);
+  } else {
+    io_store8<IO>(box_chunk<IO>(box, row, oct), v);  // rounded once, to nearest even
+  }
 }
 
 template <bool FAST, int IO>
@@ -525,7 +573,7 @@ int launch_tc_fwd2(const void* x, const float* gamma, const float* beta, void* y
 // back-pressure, 3 k waiting for boxes of a three-slot ring, 1.7 k waiting for the tensor pipe).  So:
 //   * only gamma's HI plane is resident (72 KB); the LO plane is needed by one of the three products only and is
 //     streamed from L2 per 32-channel K chunk (12 KB bulk copies, double buffered) by a "gamma" warp;
-//   * x arrives as [128 rows x 32 channels] 2-D TMA boxes (128-byte swizzle) in two three-slot rings, twice per
+//   * x arrives as [128 rows x 32 channels] 2-D TMA boxes (Box<IO>) in two three-slot rings, twice per
 //     tile: boxes C0..C5 feed the pool + bf16 split, boxes E0..E5 (L2 hits) feed the epilogue; the whole next tile is
 //     prefetched into L2 with one bulk prefetch;
 //   * the epilogue needs no transpose: thread (r, h) takes 16 accumulator columns of ITS pixel row from TMEM,
@@ -543,7 +591,7 @@ constexpr unsigned long long kEvictFirst = 0x12F0000000000000ull, kEvictLast = 0
 constexpr int kF4Compute = 512;                  // 16 compute warps: four per scheduler, the work is latency bound
 constexpr int kF4Threads = kF4Compute + 160;     // + MMA-issue, C-copy, E-copy, gamma and store warps
 constexpr int kF4Sync = kF4Compute + 32;         // compute + issue warps (the named barriers of the plane hand-off)
-constexpr int kF4Box = kTileM * 32 * 4;          // one x box: [128][32] fp32, 128-byte rows, 128B-swizzled
+constexpr int kF4Box = kTileM * 32 * 4;          // one ring slot: a [128][32] fp32 box (a 16-bit box fills half, Box<IO>)
 constexpr int kF4Kg = kTileM * 16 + 32;          // plane group stride: padding = 2 (mod 8) 16-byte units (see kF2Kg)
 constexpr int kF4Plane = 4 * kF4Kg;              // hi or lo plane of a 32-channel chunk
 
@@ -565,13 +613,15 @@ struct Fwd4Smem {
   static_assert(kBytes <= 232448, "shared memory budget");
 };
 
-template <int C, bool FAST>
+template <int C, bool FAST, int IO>
 __global__ void __launch_bounds__(kF4Threads, 1)
 gdn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constant__ CUtensorMap y_map,
-                   const float* __restrict__ x, const __nv_bfloat16* __restrict__ planes,
+                   const void* __restrict__ x_, const __nv_bfloat16* __restrict__ planes,
                    const float* __restrict__ beta, long long n_pix, TcFlags f) {
   using L = Fwd4Smem<C>;
   constexpr int NCH = C / 32;  // 6 boxes per pass over a tile
+  constexpr int kRowB = C * IoBytes<IO>::value;  // bytes per pixel row of x / y
+  const uint8_t* x = static_cast<const uint8_t*>(x_);
   extern __shared__ __align__(1024) uint8_t smem[];
   float* beta_s = reinterpret_cast<float*>(smem + L::kOffBeta);
   uint64_t* mbars = reinterpret_cast<uint64_t*>(smem + L::kOffBar);
@@ -616,8 +666,8 @@ gdn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
         const long long pn = (tile + gridDim.x) * kTileM;
         const long long rows = min((long long)kTileM, n_pix - pn);
         if (rows > 0)
-          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(x + pn * C),
-                       "r"((uint32_t)(rows * C * 4)), "l"(kEvictLast)
+          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(x + pn * kRowB),
+                       "r"((uint32_t)(rows * kRowB)), "l"(kEvictLast)
                        : "memory");
       }
 #pragma unroll 1
@@ -628,7 +678,7 @@ gdn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
         }
         const uint32_t full = bar(full0 + slot);
         const uint32_t dst = smem_u32(smem + L::kOffRing + (ring * 3 + slot) * kF4Box);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "n"(kF4Box) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "n"(Box<IO>::kBytes) : "memory");
         // x is read twice (C box, then E box about a tile later): the first read asks L2 to keep the lines, the
         // second releases them (ncu before the hints: 1.54x the algorithmic DRAM reads at 16.7 M pixels)
         asm volatile(
@@ -726,23 +776,22 @@ gdn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
   uint32_t parp[2] = {0u, 0u};
   uint32_t nc = 0, ne = 0;                     // C boxes converted / E boxes finished so far
   const int ckg = tid & 3, crow = tid >> 2;    // conversion item of a box: row crow, 8 channels
-  // 128-byte swizzle: the 16-byte chunk j of box row `row` sits at chunk j ^ (row & 7)
-  auto chunk_at = [](uint8_t* box, int row, int j) { return reinterpret_cast<float4*>(box + row * 128 + ((j ^ (row & 7)) << 4)); };
 
   auto convert = [&](int c, bool wait_planes) {
     const int pb = c & 1;
     const uint32_t slot = nc % 3u, round = nc / 3u;
     uint8_t* box = smem + L::kOffRing + slot * kF4Box;
     if (!mbar_wait(bar(L::kBarCfull + slot), round & 1u)) __trap();
-    const float4 a = *chunk_at(box, crow, 2 * ckg), b = *chunk_at(box, crow, 2 * ckg + 1);
+    float v[8];
+    box_load8<IO>(box, crow, ckg, v);
     if (wait_planes) {  // the plane buffer is still being read by the MMAs of the chunk two before this one
       if (!mbar_wait(bar(L::kBarPlane + pb), parp[pb])) __trap();
       parp[pb] ^= 1u;
     }
     uint8_t* ph = smem + L::kOffP + pb * 2 * kF4Plane;
     {
-      float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
-                    tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
+#pragma unroll
+      for (int e = 0; e < 8; ++e) v[e] = tc_pool<FAST>(v[e], f);
       uint4 hi, lo;
       split8(v, &hi, &lo);
       *reinterpret_cast<uint4*>(ph + ckg * kF4Kg + crow * 16) = hi;
@@ -764,17 +813,25 @@ gdn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
     if (!mbar_wait(bar(L::kBarEfull + slot), round & 1u)) __trap();
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
     const float* bs = beta_s + k * 32 + h * 8;
+    if constexpr (IO == 0) {
 #pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      float4* px = chunk_at(box, r, 2 * h + j);
-      const float4 xv = *px;
-      const float4 bv = *reinterpret_cast<const float4*>(bs + 4 * j);  // same address in every lane: broadcast
-      float4 o;
-      o.x = tc_out<FAST>(xv.x, bv.x + __uint_as_float(nacc[4 * j]), f);
-      o.y = tc_out<FAST>(xv.y, bv.y + __uint_as_float(nacc[4 * j + 1]), f);
-      o.z = tc_out<FAST>(xv.z, bv.z + __uint_as_float(nacc[4 * j + 2]), f);
-      o.w = tc_out<FAST>(xv.w, bv.w + __uint_as_float(nacc[4 * j + 3]), f);
-      *px = o;
+      for (int j = 0; j < 2; ++j) {
+        float4* px = reinterpret_cast<float4*>(box_chunk<0>(box, r, 2 * h + j));
+        const float4 xv = *px;
+        const float4 bv = *reinterpret_cast<const float4*>(bs + 4 * j);  // same address in every lane: broadcast
+        float4 o;
+        o.x = tc_out<FAST>(xv.x, bv.x + __uint_as_float(nacc[4 * j]), f);
+        o.y = tc_out<FAST>(xv.y, bv.y + __uint_as_float(nacc[4 * j + 1]), f);
+        o.z = tc_out<FAST>(xv.z, bv.z + __uint_as_float(nacc[4 * j + 2]), f);
+        o.w = tc_out<FAST>(xv.w, bv.w + __uint_as_float(nacc[4 * j + 3]), f);
+        *px = o;
+      }
+    } else {  // 16-bit: the row's 8 channels are one 16-byte chunk, y written over x in place
+      float xv[8], o[8];
+      box_load8<IO>(box, r, h, xv);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) o[e] = tc_out<FAST>(xv[e], bs[e] + __uint_as_float(nacc[e]), f);
+      box_store8<IO>(box, r, h, o);
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // y box -> TMA store
     __syncwarp();
@@ -824,80 +881,89 @@ gdn_tc_fwd4_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
   }
 }
 
-// 2-D tensor map of a row-major fp32 [rows, cols] array with [box_rows x box_cols] boxes (zero fill; optionally the
-// 128-byte swizzle: 16-byte chunk j of box row i lands at chunk j ^ (i & 7); needs 128-byte box rows).
 // cuTensorMapEncodeTiled is a driver entry point; it is looked up through the runtime so that the library keeps
 // linking against libcudart only.
-int make_tensor_map_2d(CUtensorMap* map, const float* base, long long rows, int cols, int box_rows, int box_cols,
-                       bool swizzle128 = false) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn encode = [] {
+typedef CUresult (*TensorMapEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
+                                      const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
+                                      CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+TensorMapEncodeFn tensor_map_encoder() {
+  static TensorMapEncodeFn encode = [] {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult st;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &st) != cudaSuccess ||
         st != cudaDriverEntryPointSuccess)
       fn = nullptr;
     (void)cudaGetLastError();
-    return reinterpret_cast<EncodeFn>(fn);
+    return reinterpret_cast<TensorMapEncodeFn>(fn);
   }();
+  return encode;
+}
+
+// Element type and swizzle of the [128 rows x 32 channels] activation boxes (see Box<IO>): 128-byte rows of float32
+// with the 128-byte swizzle, or 64-byte rows of float16 / bfloat16 with the 64-byte swizzle.
+template <int IO>
+struct IoMap {
+  static constexpr CUtensorMapDataType kType =
+      IO == 0 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : (IO == 1 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16);
+  static constexpr CUtensorMapSwizzle kSwizzle = IO == 0 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
+};
+
+inline int tensor_map_elem_bytes(CUtensorMapDataType t) { return t == CU_TENSOR_MAP_DATA_TYPE_FLOAT32 ? 4 : 2; }
+
+// 2-D tensor map of a row-major [rows, cols] array of `type` elements with [box_rows x box_cols] boxes (zero fill).
+int make_tensor_map_2d(CUtensorMap* map, const void* base, long long rows, int cols, int box_rows, int box_cols,
+                       CUtensorMapDataType type, CUtensorMapSwizzle swizzle) {
+  const TensorMapEncodeFn encode = tensor_map_encoder();
   if (!encode) return fail(TFCB_CUDA_ERROR, "cuTensorMapEncodeTiled is not available from this driver");
   const cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  const cuuint64_t strides[1] = {(cuuint64_t)cols * sizeof(float)};
+  const cuuint64_t strides[1] = {(cuuint64_t)cols * tensor_map_elem_bytes(type)};
   const cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
   const cuuint32_t estr[2] = {1u, 1u};
-  const CUresult rc = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
-                             CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  const CUresult rc = encode(map, type, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                             swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (rc != CUDA_SUCCESS) return fail(TFCB_CUDA_ERROR, "cuTensorMapEncodeTiled failed (%d)", (int)rc);
   return TFCB_OK;
 }
 
-// 3-D view of a row-major fp32 [rows, cols] array as (32 channels, rows, cols / 32 chunks) with boxes of
-// [chunks_per_box][box_rows][32 channels], 128-byte swizzle: ONE copy instruction moves several of the kernels'
-// [128 rows x 32 channels] boxes, which land back to back in shared memory exactly as separate 2-D boxes would.
+// 3-D view of a row-major [rows, cols] array as (32 channels, rows, cols / 32 chunks) with boxes of
+// [chunks_per_box][box_rows][32 channels]: ONE copy instruction moves several of the kernels' [128 rows x 32 channels]
+// boxes, which land back to back in shared memory exactly as separate 2-D boxes would.
 // (The SM's async-copy engine retires ~2.5 copy instructions per microsecond whatever their size -- 0.39 us per 16 KB
 // box, tools/tma_probe.py -- so the number of instructions per tile, not the bytes, bounded the box-fed kernels.)
-int make_tensor_map_3d(CUtensorMap* map, const float* base, long long rows, int cols, int box_rows, int chunks_per_box) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  static EncodeFn encode = [] {
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult st;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &st) != cudaSuccess ||
-        st != cudaDriverEntryPointSuccess)
-      fn = nullptr;
-    (void)cudaGetLastError();
-    return reinterpret_cast<EncodeFn>(fn);
-  }();
+int make_tensor_map_3d(CUtensorMap* map, const void* base, long long rows, int cols, int box_rows, int chunks_per_box,
+                       CUtensorMapDataType type, CUtensorMapSwizzle swizzle) {
+  const TensorMapEncodeFn encode = tensor_map_encoder();
   if (!encode) return fail(TFCB_CUDA_ERROR, "cuTensorMapEncodeTiled is not available from this driver");
+  const int eb = tensor_map_elem_bytes(type);
   const cuuint64_t dims[3] = {32u, (cuuint64_t)rows, (cuuint64_t)(cols / 32)};
-  const cuuint64_t strides[2] = {(cuuint64_t)cols * sizeof(float), 32u * sizeof(float)};  // row stride, chunk stride
+  const cuuint64_t strides[2] = {(cuuint64_t)cols * eb, 32u * (cuuint64_t)eb};  // row stride, chunk stride
   const cuuint32_t box[3] = {32u, (cuuint32_t)box_rows, (cuuint32_t)chunks_per_box};
   const cuuint32_t estr[3] = {1u, 1u, 1u};
-  const CUresult rc = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(base), dims, strides, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  const CUresult rc = encode(map, type, 3, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                             swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (rc != CUDA_SUCCESS) return fail(TFCB_CUDA_ERROR, "cuTensorMapEncodeTiled (3-D) failed (%d)", (int)rc);
   return TFCB_OK;
 }
 
-template <bool FAST>
-int launch_tc_fwd4(const float* x, const float* gamma, const float* beta, float* y, long long n_pix, TcFlags f,
+// [128 x 32] activation boxes of a row-major [n_pix, C] array of IO elements
+template <int IO>
+int make_box_map(CUtensorMap* map, const void* base, long long n_pix, int C) {
+  return make_tensor_map_2d(map, base, n_pix, C, kTileM, 32, IoMap<IO>::kType, IoMap<IO>::kSwizzle);
+}
+
+template <bool FAST, int IO>
+int launch_tc_fwd4(const void* x, const float* gamma, const float* beta, void* y, long long n_pix, TcFlags f,
                    cudaStream_t s) {
   constexpr int C = 192;
   using L = Fwd4Smem<C>;
   CUtensorMap x_map, y_map;
-  TFCB_TRY(make_tensor_map_2d(&x_map, x, n_pix, C, kTileM, 32, true));
-  TFCB_TRY(make_tensor_map_2d(&y_map, y, n_pix, C, kTileM, 32, true));
+  TFCB_TRY(make_box_map<IO>(&x_map, x, n_pix, C));
+  TFCB_TRY(make_box_map<IO>(&y_map, y, n_pix, C));
   __nv_bfloat16* planes = nullptr;
   TFCB_TRY(dev_alloc((void**)&planes, (size_t)2 * C * C * sizeof(__nv_bfloat16), s));
   gdn_tc_prep_kernel<<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
   TFCB_LAUNCHED();
-  cudaError_t e = cudaFuncSetAttribute(gdn_tc_fwd4_kernel<C, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kBytes);
+  cudaError_t e = cudaFuncSetAttribute(gdn_tc_fwd4_kernel<C, FAST, IO>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kBytes);
   if (e != cudaSuccess) {
     (void)cudaGetLastError();
     dev_free(planes, s);
@@ -908,7 +974,7 @@ int launch_tc_fwd4(const float* x, const float* gamma, const float* beta, float*
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
   const int grid = (int)std::min<long long>(n_tiles, sms);
-  gdn_tc_fwd4_kernel<C, FAST><<<grid, kF4Threads, L::kBytes, s>>>(x_map, y_map, x, planes, beta, n_pix, f);
+  gdn_tc_fwd4_kernel<C, FAST, IO><<<grid, kF4Threads, L::kBytes, s>>>(x_map, y_map, x, planes, beta, n_pix, f);
   TFCB_LAUNCHED();
   e = cudaGetLastError();
   dev_free(planes, s);
@@ -1065,14 +1131,17 @@ struct BwdFusedSmem {
   static_assert(kBytes <= 232448, "shared memory budget");
 };
 
-template <bool FAST>
+template <bool FAST, int IO>
 __global__ void __launch_bounds__(kB3Threads, 1)
 gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constant__ CUtensorMap g_map,
-                   const __grid_constant__ CUtensorMap dx_map, const float* __restrict__ x, const float* __restrict__ dy,
+                   const __grid_constant__ CUtensorMap dx_map, const void* __restrict__ x_, const void* __restrict__ dy_,
                    const __nv_bfloat16* __restrict__ planes, const float* __restrict__ beta, float* __restrict__ part_g,
                    float* __restrict__ part_b, long long n_pix, TcFlags f) {
   using L = BwdFusedSmem;
   constexpr int C = L::C, NCH = C / 32;
+  constexpr int kRowB = C * IoBytes<IO>::value;  // bytes per pixel row of x / dy / dx
+  const uint8_t* x = static_cast<const uint8_t*>(x_);
+  const uint8_t* dy = static_cast<const uint8_t*>(dy_);
   extern __shared__ __align__(1024) uint8_t smem[];
   float* beta_s = reinterpret_cast<float*>(smem + L::kOffBeta);
   float* dbeta_s = reinterpret_cast<float*>(smem + L::kOffDbeta);
@@ -1129,7 +1198,7 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       auto load = [&](const CUtensorMap* map, int c, int row0) {
         const uint32_t slot = acquire();
         const uint32_t full = bar(L::kBarFull + slot);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "n"(kF4Box) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "n"(Box<IO>::kBytes) : "memory");
         asm volatile(
             "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], [%4], %5;" ::"r"(
                 smem_u32(smem + L::kOffRing + slot * kF4Box)),
@@ -1137,12 +1206,12 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
             : "memory");
         ++n;
       };
-      auto prefetch_tile = [&](const float* base, long long tile) {  // one contiguous block -> L2
+      auto prefetch_tile = [&](const uint8_t* base, long long tile) {  // one contiguous block -> L2
         const long long p0 = tile * kTileM;
         const long long rows = min((long long)kTileM, n_pix - p0);
         if (rows > 0)
-          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(base + p0 * C),
-                       "r"((uint32_t)(rows * C * 4)), "l"(kEvictLast)
+          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(base + p0 * kRowB),
+                       "r"((uint32_t)(rows * kRowB)), "l"(kEvictLast)
                        : "memory");
       };
       if (first < n_tiles) {
@@ -1326,8 +1395,6 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
   for (int c = 0; c < NCH; ++c)
 #pragma unroll
     for (int e = 0; e < 8; ++e) dbeta_acc[c][e] = 0.f;
-  // 128-byte swizzle: the 16-byte chunk j of box row `row` sits at chunk j ^ (row & 7)
-  auto chunk_at = [](uint8_t* box, int row, int j) { return reinterpret_cast<float4*>(box + row * 128 + ((j ^ (row & 7)) << 4)); };
   bool flushed = false;  // the global partial holds earlier flushes
   // The accumulator (TMEM lane = input channel j, 32 columns per thread) is transposed through the dead q planes
   // ([128][128] fp32, 16-byte units XOR-swizzled by the row) so that every warp adds 512 contiguous bytes to the CTA's
@@ -1367,12 +1434,14 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       const uint32_t slot = n & 3u, round = n >> 2;
       uint8_t* box = smem + L::kOffRing + slot * kF4Box;
       if (!mbar_wait(bar(L::kBarFull + slot), round & 1u)) __trap();
-      const float4 a = *chunk_at(box, r, 2 * h), b = *chunk_at(box, r, 2 * h + 1);
-      const uint32_t raw[8] = {__float_as_uint(a.x), __float_as_uint(a.y), __float_as_uint(a.z), __float_as_uint(a.w),
-                               __float_as_uint(b.x), __float_as_uint(b.y), __float_as_uint(b.z), __float_as_uint(b.w)};
+      float v[8];
+      box_load8<IO>(box, r, h, v);
+      uint32_t raw[8];  // x widened to float32 is what pass 2 and the variants' pass 3 read back
+#pragma unroll
+      for (int e = 0; e < 8; ++e) raw[e] = __float_as_uint(v[e]);
       tmem_store8(tmem_x + lane_sel + (uint32_t)(c * 32 + h * 8), raw);
-      float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
-                    tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
+#pragma unroll
+      for (int e = 0; e < 8; ++e) v[e] = tc_pool<FAST>(v[e], f);
       uint4 hi, lo;
       split8(v, &hi, &lo);
       *reinterpret_cast<uint4*>(smem + L::kOffPh + (4 * c + h) * kKg + r * 16) = hi;
@@ -1400,11 +1469,11 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
       tmem_load<8>(tmem_x + col, xraw);
       if (!mbar_wait(bar(L::kBarFull + slot), (n >> 2) & 1u)) __trap();
       uint8_t* bg = smem + L::kOffRing + slot * kF4Box;
-      const float4 g0 = *chunk_at(bg, r, 2 * h), g1 = *chunk_at(bg, r, 2 * h + 1);
+      float gs[8];
+      box_load8<IO>(bg, r, h, gs);
       const float4 bv0 = *reinterpret_cast<const float4*>(beta_s + c * 32 + h * 8);      // same address in every lane
       const float4 bv1 = *reinterpret_cast<const float4*>(beta_s + c * 32 + h * 8 + 4);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      const float gs[8] = {g0.x, g0.y, g0.z, g0.w, g1.x, g1.y, g1.z, g1.w};
       const float bs[8] = {bv0.x, bv0.y, bv0.z, bv0.w, bv1.x, bv1.y, bv1.z, bv1.w};
       float q[8];
       uint32_t dbits[8];
@@ -1452,8 +1521,7 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
           o[e] = tc_dx(__uint_as_float(d[e]), __uint_as_float(xraw[e]), __uint_as_float(p[e]), f);
         }
       }
-      *chunk_at(box, r, 2 * h) = make_float4(o[0], o[1], o[2], o[3]);
-      *chunk_at(box, r, 2 * h + 1) = make_float4(o[4], o[5], o[6], o[7]);
+      box_store8<IO>(box, r, h, o);
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // dx box -> TMA store
       __syncwarp();
       if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(L::kBarY + slot)) : "memory");
@@ -1489,20 +1557,20 @@ gdn_tc_bwd3_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_const
   }
 }
 
-template <bool FAST>
-int launch_tc_bwd3(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* part_g,
+template <bool FAST, int IO>
+int launch_tc_bwd3(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* part_g,
                    float* part_b, int* n_parts, long long n_pix, TcFlags f, cudaStream_t s) {
   constexpr int C = 128;
   using L = BwdFusedSmem;
   CUtensorMap x_map, g_map, dx_map;
-  TFCB_TRY(make_tensor_map_2d(&x_map, x, n_pix, C, kTileM, 32, true));
-  TFCB_TRY(make_tensor_map_2d(&g_map, dy, n_pix, C, kTileM, 32, true));
-  TFCB_TRY(make_tensor_map_2d(&dx_map, dx, n_pix, C, kTileM, 32, true));
+  TFCB_TRY(make_box_map<IO>(&x_map, x, n_pix, C));
+  TFCB_TRY(make_box_map<IO>(&g_map, dy, n_pix, C));
+  TFCB_TRY(make_box_map<IO>(&dx_map, dx, n_pix, C));
   __nv_bfloat16* planes = nullptr;
   TFCB_TRY(dev_alloc((void**)&planes, (size_t)4 * C * C * sizeof(__nv_bfloat16), s));
   gdn_tc_prep2_kernel<true><<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
   TFCB_LAUNCHED();
-  cudaError_t e = cudaFuncSetAttribute(gdn_tc_bwd3_kernel<FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kBytes);
+  cudaError_t e = cudaFuncSetAttribute(gdn_tc_bwd3_kernel<FAST, IO>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::kBytes);
   if (e != cudaSuccess) {
     (void)cudaGetLastError();
     dev_free(planes, s);
@@ -1513,8 +1581,8 @@ int launch_tc_bwd3(const float* x, const float* gamma, const float* beta, const 
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
   const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
-  gdn_tc_bwd3_kernel<FAST><<<grid, kB3Threads, L::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta, part_g, part_b,
-                                                              n_pix, f);
+  gdn_tc_bwd3_kernel<FAST, IO><<<grid, kB3Threads, L::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta, part_g,
+                                                                  part_b, n_pix, f);
   TFCB_LAUNCHED();
   e = cudaGetLastError();
   dev_free(planes, s);
@@ -1571,14 +1639,17 @@ struct BwdDx2Smem {
   static_assert(kBytes <= 232448, "shared memory budget");
 };
 
-template <bool FAST>
+template <bool FAST, int IO>
 __global__ void __launch_bounds__(kD2Threads, 1)
 gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_constant__ CUtensorMap g_map,
-                      const __grid_constant__ CUtensorMap dx_map, const float* __restrict__ x,
-                      const float* __restrict__ dy, const __nv_bfloat16* __restrict__ planes,
+                      const __grid_constant__ CUtensorMap dx_map, const void* __restrict__ x_,
+                      const void* __restrict__ dy_, const __nv_bfloat16* __restrict__ planes,
                       const float* __restrict__ beta, uint8_t* __restrict__ q_planes, long long n_pix, TcFlags f) {
   using L = BwdDx2Smem;
   constexpr int C = L::C, NCH = C / 32;
+  constexpr int EB = IoBytes<IO>::value, kRowB = C * EB;  // bytes per element / per pixel row of x / dy / dx
+  const uint8_t* x = static_cast<const uint8_t*>(x_);
+  const uint8_t* dy = static_cast<const uint8_t*>(dy_);
   extern __shared__ __align__(1024) uint8_t smem[];
   float* beta_s = reinterpret_cast<float*>(smem + L::kOffBeta);
   uint64_t* mbars = reinterpret_cast<uint64_t*>(smem + L::kOffBar);
@@ -1635,7 +1706,7 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
       auto load = [&](const CUtensorMap* map, int c, int row0) {
         const uint32_t slot = acquire();
         const uint32_t full = bar(L::kBarFull + slot);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "n"(kF4Box) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(full), "n"(Box<IO>::kBytes) : "memory");
         asm volatile(
             "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], [%4], %5;" ::"r"(
                 smem_u32(smem + L::kOffRing + slot * kF4Box)),
@@ -1648,12 +1719,12 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
         asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(L::kBarFull + slot)) : "memory");
         ++n;
       };
-      auto prefetch_tile = [&](const float* base, long long tile) {  // one contiguous block -> L2
+      auto prefetch_tile = [&](const uint8_t* base, long long tile) {  // one contiguous block -> L2
         const long long p0 = tile * kTileM;
         const long long rows = min((long long)kTileM, n_pix - p0);
         if (rows > 0)
-          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(base + p0 * C),
-                       "r"((uint32_t)(rows * C * 4)), "l"(kEvictLast)
+          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(base + p0 * kRowB),
+                       "r"((uint32_t)(rows * kRowB)), "l"(kEvictLast)
                        : "memory");
       };
       if (first < n_tiles) {
@@ -1840,8 +1911,6 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
   } else if (warp < W0) {
   // --------------------------------- compute warps ---------------------------------
   uint32_t n = 0, m = 0;
-  // 128-byte swizzle: the 16-byte chunk j of box row `row` sits at chunk j ^ (row & 7)
-  auto chunk_at = [](uint8_t* box, int row, int j) { return reinterpret_cast<float4*>(box + row * 128 + ((j ^ (row & 7)) << 4)); };
   auto wait_full = [&](uint32_t req) {
     if (!mbar_wait(bar(L::kBarFull + slot_of(req)), round_of(req) & 1u)) __trap();
     return smem + L::kOffRing + slot_of(req) * kF4Box;
@@ -1867,9 +1936,10 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
 #pragma unroll 1
     for (int c = 0; c < NCH; ++c, ++n) {
       uint8_t* box = wait_full(n);
-      const float4 a = *chunk_at(box, r, 2 * h), b = *chunk_at(box, r, 2 * h + 1);
-      float v[8] = {tc_pool<FAST>(a.x, f), tc_pool<FAST>(a.y, f), tc_pool<FAST>(a.z, f), tc_pool<FAST>(a.w, f),
-                    tc_pool<FAST>(b.x, f), tc_pool<FAST>(b.y, f), tc_pool<FAST>(b.z, f), tc_pool<FAST>(b.w, f)};
+      float v[8];
+      box_load8<IO>(box, r, h, v);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) v[e] = tc_pool<FAST>(v[e], f);
       uint4 hi, lo, *ph, *pl;
       split8(v, &hi, &lo);
       operand_rows(&ph, &pl, after_pass2 && c < 2);  // chunks 0, 1 reuse the buffers of the tile's last two q chunks
@@ -1896,13 +1966,12 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
       tmem_load<8>(col, nacc);
       uint8_t* bx = wait_full(n);
       uint8_t* bg = wait_full(n + 1);
-      const float4 x0 = *chunk_at(bx, r, 2 * h), x1 = *chunk_at(bx, r, 2 * h + 1);
-      const float4 g0 = *chunk_at(bg, r, 2 * h), g1 = *chunk_at(bg, r, 2 * h + 1);
+      float xs[8], gs[8];
+      box_load8<IO>(bx, r, h, xs);
+      box_load8<IO>(bg, r, h, gs);
       const float4 bv0 = *reinterpret_cast<const float4*>(beta_s + c * 32 + h * 8);      // same address in every lane
       const float4 bv1 = *reinterpret_cast<const float4*>(beta_s + c * 32 + h * 8 + 4);
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      const float xs[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
-      const float gs[8] = {g0.x, g0.y, g0.z, g0.w, g1.x, g1.y, g1.z, g1.w};
       const float bs[8] = {bv0.x, bv0.y, bv0.z, bv0.w, bv1.x, bv1.y, bv1.z, bv1.w};
       float q[8];
       uint32_t dbits[8];
@@ -1935,17 +2004,25 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
       uint32_t d[8], p[8];
       tmem_load<8>(tmem_n + lane_sel + (uint32_t)(c * 32 + h * 8), d);
       tmem_load<8>(tmem_dp + lane_sel + (uint32_t)(c * 32 + h * 8), p);
-      float4 x0, x1;  // the variants: this thread's 8 values of x, read again (TMEM has no room to park them)
+      float xs[8];  // the variants: this thread's 8 values of x, read again (TMEM has no room to park them)
       if (!FAST) {
         const long long row = tile * kTileM + r;
-        const float4* src = reinterpret_cast<const float4*>(x + row * C + c * 32 + h * 8);
-        const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
-        x0 = row < n_pix ? __ldg(src) : z;
-        x1 = row < n_pix ? __ldg(src + 1) : z;
+        const uint8_t* src = x + row * kRowB + (c * 32 + h * 8) * EB;
+        if (IO == 0) {
+          const float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+          const float4 x0 = row < n_pix ? __ldg(reinterpret_cast<const float4*>(src)) : z;
+          const float4 x1 = row < n_pix ? __ldg(reinterpret_cast<const float4*>(src) + 1) : z;
+          xs[0] = x0.x; xs[1] = x0.y; xs[2] = x0.z; xs[3] = x0.w;
+          xs[4] = x1.x; xs[5] = x1.y; xs[6] = x1.z; xs[7] = x1.w;
+        } else if (row < n_pix) {
+          io_load8<IO>(src, xs);  // one 16-byte load, widened exactly
+        } else {
+#pragma unroll
+          for (int e = 0; e < 8; ++e) xs[e] = 0.f;
+        }
       }
       uint8_t* box = wait_full(n);  // the slot's previous user has left
       asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-      const float xs[8] = {x0.x, x0.y, x0.z, x0.w, x1.x, x1.y, x1.z, x1.w};
       float o[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
@@ -1957,8 +2034,7 @@ gdn_tc_bwd_dx2_kernel(const __grid_constant__ CUtensorMap x_map, const __grid_co
           o[e] = tc_dx(__uint_as_float(d[e]), xs[e], __uint_as_float(p[e]), f);
         }
       }
-      *chunk_at(box, r, 2 * h) = make_float4(o[0], o[1], o[2], o[3]);
-      *chunk_at(box, r, 2 * h + 1) = make_float4(o[4], o[5], o[6], o[7]);
+      box_store8<IO>(box, r, h, o);
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // dx box -> TMA store
       __syncwarp();
       if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(L::kBarY + slot_of(n))) : "memory");
@@ -2006,13 +2082,15 @@ struct BwdDg2Smem {
   static_assert(2 * kPlane == 6 * kF4Box && 2 * kPlane >= kTileM * C * 4, "x tile / flush staging fit in the p planes");
 };
 
-template <bool FAST>
+template <bool FAST, int IO>
 __global__ void __launch_bounds__(kG2Threads, 1)
-gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float* __restrict__ x,
+gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const void* __restrict__ x_,
                           const uint8_t* __restrict__ q_planes, float* __restrict__ part_g, float* __restrict__ part_b,
                           long long n_pix, TcFlags f) {
   using L = BwdDg2Smem;
   constexpr int C = L::C, NCH = C / 32;
+  constexpr int kRowB = C * IoBytes<IO>::value;  // bytes per pixel row of x
+  const uint8_t* x = static_cast<const uint8_t*>(x_);
   extern __shared__ __align__(1024) uint8_t smem[];
   float* dbeta_s = reinterpret_cast<float*>(smem + L::kOffDbeta);
   uint64_t* mbars = reinterpret_cast<uint64_t*>(smem + L::kOffBar);
@@ -2052,8 +2130,8 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
         if (next < n_tiles) {  // the next tile of this CTA -> L2
           const long long p0 = next * kTileM;
           const long long rows = min((long long)kTileM, n_pix - p0);
-          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(x + p0 * C),
-                       "r"((uint32_t)(rows * C * 4)), "l"(kEvictLast)
+          asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(x + p0 * kRowB),
+                       "r"((uint32_t)(rows * kRowB)), "l"(kEvictLast)
                        : "memory");
           asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(q_planes + (size_t)next * (2 * L::kPlane)),
                        "n"(2 * L::kPlane), "l"(kEvictLast)
@@ -2072,7 +2150,7 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
         // the p planes are free once the compute warps say so (previous MMAs done, flush staging consumed)
         if (!mbar_wait(bar(L::kBarPfree), (uint32_t)t & 1u)) __trap();
         const uint32_t xfull = bar(L::kBarXfull);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(xfull), "n"(6 * kF4Box) : "memory");
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(xfull), "n"(NCH * Box<IO>::kBytes) : "memory");
         // ONE 3-D box: all six [128 x 32] boxes of the tile, back to back (a copy instruction costs the SM's copy
         // engine ~0.35 us whatever its size, tools/tma_probe.py)
         asm volatile(
@@ -2122,6 +2200,7 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
   for (int k = 0; k < 2; ++k)
 #pragma unroll
     for (int e = 0; e < 8; ++e) dbeta_acc[k][e] = 0.f;
+  // float32 boxes (= box_chunk<0>; as a lambda the float32 instantiation compiles to the same code as before IO existed)
   auto chunk_at = [](uint8_t* box, int row, int j) { return reinterpret_cast<float4*>(box + row * 128 + ((j ^ (row & 7)) << 4)); };
   bool flushed = false;
   // one row block of the accumulator (lane r = row, 48 columns per thread) -> swizzled [128][192] fp32 staging in
@@ -2171,18 +2250,32 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
     if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar(L::kBarPfree)) : "memory");
     // the x tile has landed in the p planes: take this thread's 48 values, then overwrite the boxes with the planes
     if (!mbar_wait(bar(L::kBarXfull), (uint32_t)t & 1u)) __trap();
-    float4 xa[NCH], xb[NCH];
+    // (the six boxes sit back to back: 96 KB of float32, or 48 KB of 16-bit elements in the hi plane's memory;
+    // 16-bit values stay packed in registers until after the barrier)
+    using XReg = typename std::conditional<IO == 0, float4, uint4>::type;
+    XReg xa[NCH], xb[NCH];
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
-      uint8_t* box = smem + L::kOffPh + c * kF4Box;
-      xa[c] = *chunk_at(box, r, 2 * h);
-      xb[c] = *chunk_at(box, r, 2 * h + 1);
+      uint8_t* box = smem + L::kOffPh + c * Box<IO>::kBytes;
+      if constexpr (IO == 0) {
+        xa[c] = *chunk_at(box, r, 2 * h);
+        xb[c] = *chunk_at(box, r, 2 * h + 1);
+      } else {
+        xa[c] = *reinterpret_cast<const uint4*>(box_chunk<IO>(box, r, h));
+      }
     }
     asm volatile("bar.sync 1, %0;" ::"n"(kG2Compute) : "memory");  // every thread holds its values
 #pragma unroll
     for (int c = 0; c < NCH; ++c) {
-      float v[8] = {tc_pool<FAST>(xa[c].x, f), tc_pool<FAST>(xa[c].y, f), tc_pool<FAST>(xa[c].z, f), tc_pool<FAST>(xa[c].w, f),
-                    tc_pool<FAST>(xb[c].x, f), tc_pool<FAST>(xb[c].y, f), tc_pool<FAST>(xb[c].z, f), tc_pool<FAST>(xb[c].w, f)};
+      float v[8];
+      if constexpr (IO == 0) {
+        v[0] = xa[c].x; v[1] = xa[c].y; v[2] = xa[c].z; v[3] = xa[c].w;
+        v[4] = xb[c].x; v[5] = xb[c].y; v[6] = xb[c].z; v[7] = xb[c].w;
+      } else {
+        io_widen8<IO>(xa[c], v);
+      }
+#pragma unroll
+      for (int e = 0; e < 8; ++e) v[e] = tc_pool<FAST>(v[e], f);
       uint4 hi, lo;
       split8(v, &hi, &lo);
       *reinterpret_cast<uint4*>(smem + L::kOffPh + (4 * c + h) * kDKg + r * 16) = hi;
@@ -2240,19 +2333,19 @@ gdn_tc_bwd_dgamma2_kernel(const __grid_constant__ CUtensorMap x_map, const float
 
 // q travels from the dx kernel to the dgamma kernel as bf16 hi / lo planes ([tile][2][24][128][8], 4 B/element; the
 // workspace is sized in whole tiles, tfcb_gdn_backward_workspace_bytes)
-template <bool FAST>
-int launch_tc_bwd192(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* q_ws,
+template <bool FAST, int IO>
+int launch_tc_bwd192(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
                      float* part_g, float* part_b, int* n_parts, long long n_pix, TcFlags f, cudaStream_t s) {
   constexpr int C = 192;
   using L2 = BwdDx2Smem;
   using L3 = BwdDg2Smem;
   CUtensorMap x_map, g_map, dx_map, x_map3;  // x_map3: the whole [128 x 192] x tile as one 3-D box
-  TFCB_TRY(make_tensor_map_2d(&x_map, x, n_pix, C, kTileM, 32, true));
-  TFCB_TRY(make_tensor_map_2d(&g_map, dy, n_pix, C, kTileM, 32, true));
-  TFCB_TRY(make_tensor_map_2d(&dx_map, dx, n_pix, C, kTileM, 32, true));
-  TFCB_TRY(make_tensor_map_3d(&x_map3, x, n_pix, C, kTileM, C / 32));
-  if (cudaFuncSetAttribute(gdn_tc_bwd_dx2_kernel<FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L2::kBytes) != cudaSuccess ||
-      cudaFuncSetAttribute(gdn_tc_bwd_dgamma2_kernel<FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L3::kBytes) != cudaSuccess) {
+  TFCB_TRY(make_box_map<IO>(&x_map, x, n_pix, C));
+  TFCB_TRY(make_box_map<IO>(&g_map, dy, n_pix, C));
+  TFCB_TRY(make_box_map<IO>(&dx_map, dx, n_pix, C));
+  TFCB_TRY(make_tensor_map_3d(&x_map3, x, n_pix, C, kTileM, C / 32, IoMap<IO>::kType, IoMap<IO>::kSwizzle));
+  if (cudaFuncSetAttribute(gdn_tc_bwd_dx2_kernel<FAST, IO>, cudaFuncAttributeMaxDynamicSharedMemorySize, L2::kBytes) != cudaSuccess ||
+      cudaFuncSetAttribute(gdn_tc_bwd_dgamma2_kernel<FAST, IO>, cudaFuncAttributeMaxDynamicSharedMemorySize, L3::kBytes) != cudaSuccess) {
     (void)cudaGetLastError();
     return fail(TFCB_CUDA_ERROR, "cannot reserve shared memory for the C=192 backward");
   }
@@ -2265,11 +2358,11 @@ int launch_tc_bwd192(const float* x, const float* gamma, const float* beta, cons
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
   const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
-  gdn_tc_bwd_dx2_kernel<FAST><<<grid, kD2Threads, L2::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta,
-                                                                  reinterpret_cast<uint8_t*>(q_ws), n_pix, f);
+  gdn_tc_bwd_dx2_kernel<FAST, IO><<<grid, kD2Threads, L2::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta,
+                                                                      reinterpret_cast<uint8_t*>(q_ws), n_pix, f);
   TFCB_LAUNCHED();
-  gdn_tc_bwd_dgamma2_kernel<FAST><<<grid, kG2Threads, L3::kBytes, s>>>(x_map3, x, reinterpret_cast<const uint8_t*>(q_ws),
-                                                                       part_g, part_b, n_pix, f);
+  gdn_tc_bwd_dgamma2_kernel<FAST, IO><<<grid, kG2Threads, L3::kBytes, s>>>(x_map3, x, reinterpret_cast<const uint8_t*>(q_ws),
+                                                                           part_g, part_b, n_pix, f);
   TFCB_LAUNCHED();
   const cudaError_t e = cudaGetLastError();
   dev_free(planes, s);
@@ -2278,78 +2371,107 @@ int launch_tc_bwd192(const float* x, const float* gamma, const float* beta, cons
   return TFCB_OK;
 }
 
+// The tensor-core kernels take alpha in {1, 2}, epsilon in {1, 1/2} as fixed exponents; false otherwise.
+bool tc_flags(int flags, float alpha, float eps, TcFlags* f, bool* fast) {
+  if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return false;
+  if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return false;  // trainable exponents: literal pow
+  f->inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
+  f->rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
+  f->alpha_mode = (alpha == 2.f) ? 2 : 1;
+  f->eps_mode = (eps == 0.5f) ? 2 : 1;
+  *fast = (alpha == 1.f) && (eps == 1.f) && !f->rectify;
+  return true;
+}
+
+bool misaligned16(const void* a, const void* b, const void* c) {
+  return ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c)) & 15) != 0;
+}
+
+// 16-bit activations (float16 / bfloat16 in, same type out; parameters and arithmetic float32): the same kernels as the
+// float32 path, instantiated for 16-bit elements.  *handled = false -> no native kernel for this call.
+template <int IO>
+int gdn_tc_forward16_io(const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C, TcFlags f,
+                        bool fast, cudaStream_t s) {
+  if (C == 128)
+    return fast ? launch_tc_fwd2<true, IO>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd2<false, IO>(x, gamma, beta, y, n_pix, f, s);
+  return fast ? launch_tc_fwd4<true, IO>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd4<false, IO>(x, gamma, beta, y, n_pix, f, s);
+}
+
+// Tensor-core backward; fills the per-CTA partial sums (part_g [n_parts][C][C], part_b [n_parts][C]) that the caller
+// reduces.  *handled = false -> no tensor-core kernel for this call (float32: the caller runs the fp32 kernels).
+template <int IO>
+int gdn_tc_backward_io(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
+                       float* part_g, float* part_b, int* n_parts, long long n_pix, int C, TcFlags f, bool fast,
+                       cudaStream_t s) {
+  if (C == 128)
+    return fast ? launch_tc_bwd3<true, IO>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s)
+                : launch_tc_bwd3<false, IO>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+  return fast ? launch_tc_bwd192<true, IO>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s)
+              : launch_tc_bwd192<false, IO>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+}
+
+// The conditions under which the box-fed backward kernels apply, whatever the activation type
+bool tc_backward_applies(const void* x, const void* dy, const void* dx, const float* q_ws, long long n_pix, int C,
+                         int flags, float alpha, float eps, TcFlags* f, bool* fast) {
+  if (C != 128 && C != 192) return false;
+  if (C == 192 && (reinterpret_cast<uintptr_t>(q_ws) & 15)) return false;
+  if (!tc_flags(flags, alpha, eps, f, fast)) return false;
+  if (misaligned16(x, dy, dx)) return false;
+  return n_pix < (1ll << 31);  // the box kernels take 32-bit TMA row coordinates
+}
+
 }  // namespace
 
 int gdn_tc_forward(const float* x, const float* gamma, const float* beta, float* y, long long n_pix, int C,
                    int flags, float alpha, float eps, cudaStream_t s, bool* handled) {
   *handled = false;
   if (!(C == 128 || C == 192)) return TFCB_OK;
-  if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return TFCB_OK;
-  if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return TFCB_OK;  // trainable exponents: literal pow
-  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(beta)) & 15) return TFCB_OK;  // 16-byte rows
   TcFlags f;
-  f.inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
-  f.rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
-  f.alpha_mode = (alpha == 2.f) ? 2 : 1;
-  f.eps_mode = (eps == 0.5f) ? 2 : 1;
+  bool fast;
+  if (!tc_flags(flags, alpha, eps, &f, &fast)) return TFCB_OK;
+  if (misaligned16(x, y, beta)) return TFCB_OK;  // 16-byte rows
   *handled = true;
-  const bool fast = (alpha == 1.f) && (eps == 1.f) && !f.rectify;
   if (C == 128)  // x tile resident in shared memory, bulk async copies
     return fast ? launch_tc_fwd2<true, 0>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd2<false, 0>(x, gamma, beta, y, n_pix, f, s);
   // C == 192: x through rings of 2-D TMA boxes, gamma's lo plane streamed, y through TMA stores
   if (n_pix >= (1ll << 31)) return fail(TFCB_INVALID_ARGUMENT, "GDN: more than 2^31 pixels in one call");
-  return fast ? launch_tc_fwd4<true>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd4<false>(x, gamma, beta, y, n_pix, f, s);
+  return fast ? launch_tc_fwd4<true, 0>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd4<false, 0>(x, gamma, beta, y, n_pix, f, s);
 }
 
-// 16-bit activations (float16 / bfloat16 in, same type out; parameters and arithmetic float32): the C = 128 resident
-// tile kernel with 256-byte rows.  *handled = false -> the caller converts and runs the float32 path.
 int gdn_tc_forward16(const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C, int flags,
                      float alpha, float eps, int dtype, cudaStream_t s, bool* handled) {
   *handled = false;
-  if (C != 128 || (dtype != 1 && dtype != 2)) return TFCB_OK;
-  if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return TFCB_OK;
-  if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return TFCB_OK;
-  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y) | reinterpret_cast<uintptr_t>(beta)) & 15) return TFCB_OK;
+  if (!(C == 128 || C == 192) || (dtype != 1 && dtype != 2)) return TFCB_OK;
   TcFlags f;
-  f.inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
-  f.rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
-  f.alpha_mode = (alpha == 2.f) ? 2 : 1;
-  f.eps_mode = (eps == 0.5f) ? 2 : 1;
+  bool fast;
+  if (!tc_flags(flags, alpha, eps, &f, &fast)) return TFCB_OK;
+  if (misaligned16(x, y, beta)) return TFCB_OK;
+  if (C == 192 && n_pix >= (1ll << 31)) return TFCB_OK;  // 32-bit TMA row coordinates
   *handled = true;
-  const bool fast = (alpha == 1.f) && (eps == 1.f) && !f.rectify;
-  if (dtype == 1)
-    return fast ? launch_tc_fwd2<true, 1>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd2<false, 1>(x, gamma, beta, y, n_pix, f, s);
-  return fast ? launch_tc_fwd2<true, 2>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd2<false, 2>(x, gamma, beta, y, n_pix, f, s);
+  return dtype == 1 ? gdn_tc_forward16_io<1>(x, gamma, beta, y, n_pix, C, f, fast, s)
+                    : gdn_tc_forward16_io<2>(x, gamma, beta, y, n_pix, C, f, fast, s);
 }
 
-}  // namespace tfcb
-
-namespace tfcb {
-
-// Fused tensor-core backward; fills the per-CTA partial sums (part_g [n_parts][C][C], part_b [n_parts][C]) that
-// the caller reduces.  *handled = false -> the caller runs the fp32 kernels.
 int gdn_tc_backward(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* q_ws,
                     float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
                     float eps, cudaStream_t s, bool* handled) {
-  *handled = false;
-  if (C != 128 && C != 192) return TFCB_OK;
-  if (C == 192 && (reinterpret_cast<uintptr_t>(q_ws) & 15)) return TFCB_OK;
-  if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return TFCB_OK;
-  if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return TFCB_OK;  // trainable exponents: literal pow
-  if ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(dx)) & 15) return TFCB_OK;
-  if (n_pix >= (1ll << 31)) return TFCB_OK;  // the box kernels take 32-bit TMA row coordinates
   TcFlags f;
-  f.inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
-  f.rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
-  f.alpha_mode = (alpha == 2.f) ? 2 : 1;
-  f.eps_mode = (eps == 0.5f) ? 2 : 1;
-  *handled = true;
-  const bool fast = (alpha == 1.f) && (eps == 1.f) && !f.rectify;
-  if (C == 128)
-    return fast ? launch_tc_bwd3<true>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s)
-                : launch_tc_bwd3<false>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
-  return fast ? launch_tc_bwd192<true>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s)
-              : launch_tc_bwd192<false>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+  bool fast;
+  *handled = tc_backward_applies(x, dy, dx, q_ws, n_pix, C, flags, alpha, eps, &f, &fast);
+  if (!*handled) return TFCB_OK;
+  return gdn_tc_backward_io<0>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, C, f, fast, s);
+}
+
+// 16-bit x, dy and dx (dtype 1 float16, 2 bfloat16); float32 parameters, partial sums and arithmetic
+int gdn_tc_backward16(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
+                      float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
+                      float eps, int dtype, cudaStream_t s, bool* handled) {
+  TcFlags f;
+  bool fast;
+  *handled = (dtype == 1 || dtype == 2) && tc_backward_applies(x, dy, dx, q_ws, n_pix, C, flags, alpha, eps, &f, &fast);
+  if (!*handled) return TFCB_OK;
+  return dtype == 1 ? gdn_tc_backward_io<1>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, C, f, fast, s)
+                    : gdn_tc_backward_io<2>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, C, f, fast, s);
 }
 
 }  // namespace tfcb

@@ -42,16 +42,25 @@ def _gdn_args(x, gamma, beta):
   return x, gamma, beta, C_, x.numel() // C_
 
 
+def _native16(x, beta, C_, n_pix, alpha, epsilon, pow_alpha, pow_epsilon, dy=None, boxes=True):
+  """True where a kernel reads and writes the 16-bit activations itself (mixed precision, gdn_test.py:200-210):
+  C in {128, 192}, fixed alpha in {1, 2} and epsilon in {1, 1/2}, at least one pixel (fewer than 2^31 where the
+  kernel moves x in TMA boxes, which take 32-bit row coordinates), 16-byte aligned x / beta / dy, and dy of x's
+  type.  Everything else converts to float32 and back."""
+  return (x.dtype in _IO16 and C_ in (128, 192) and not pow_alpha and not pow_epsilon and
+          float(alpha) in (1.0, 2.0) and float(epsilon) in (1.0, 0.5) and n_pix > 0 and
+          (n_pix < 2**31 or not boxes) and (dy is None or dy.dtype == x.dtype) and
+          all(t.data_ptr() % 16 == 0 for t in (x, beta) + (() if dy is None else (dy,))))
+
+
 def gdn_forward(x, gamma, beta, inverse=False, rectify=False, alpha=1.0, epsilon=1.0, pow_alpha=False,
                 pow_epsilon=False):
-  """x: float32 CUDA [..., C] (channels-last, contiguous) -> y of the same shape."""
+  """x: float32 / float16 / bfloat16 CUDA [..., C] (channels-last, contiguous) -> y of the same shape and type."""
   x, gamma, beta, C_, n_pix = _gdn_args(x, gamma, beta)
   if x.dtype in _IO16:
-    # mixed precision (gdn_test.py:200-210): 16-bit activations, float32 parameters and arithmetic.  C = 128 with the
-    # fixed exponents has a kernel that reads and writes 16-bit elements; everything else converts to float32.
-    native = (C_ == 128 and not pow_alpha and not pow_epsilon and float(alpha) in (1.0, 2.0) and
-              float(epsilon) in (1.0, 0.5) and n_pix > 0)
-    if native:
+    # 16-bit activations, float32 parameters and arithmetic: the kernel reads and writes the 16-bit elements where
+    # _native16 allows it (C = 128 keeps the whole tile in shared memory and needs no boxes); otherwise convert.
+    if _native16(x, beta, C_, n_pix, alpha, epsilon, pow_alpha, pow_epsilon, boxes=C_ != 128):
       y = torch.empty_like(x)
       check(_lib.lib().tfcb_gdn_forward_16bit(_p(x), _p(gamma), _p(beta), _p(y), n_pix, C_, _IO16[x.dtype],
                                               _flags(inverse, rectify), float(alpha), float(epsilon), _stream()))
@@ -66,9 +75,20 @@ def gdn_forward(x, gamma, beta, inverse=False, rectify=False, alpha=1.0, epsilon
 
 def gdn_backward(x, gamma, beta, dy, inverse=False, rectify=False, alpha=1.0, epsilon=1.0, pow_alpha=False,
                  pow_epsilon=False):
-  """Returns (dx, dgamma, dbeta) for upstream gradient dy."""
+  """Returns (dx, dgamma, dbeta) for upstream gradient dy; dx has x's type, dgamma / dbeta are float32."""
   x, gamma, beta, C_, n_pix = _gdn_args(x, gamma, beta)
-  if x.dtype in _IO16:  # the backward kernels are float32: convert, run, hand dx back in the activations' type
+  if x.dtype in _IO16:
+    dy16 = dy.contiguous()
+    if _native16(x, beta, C_, n_pix, alpha, epsilon, pow_alpha, pow_epsilon, dy=dy16):
+      dx = torch.empty_like(x)
+      dgamma = torch.empty_like(gamma)
+      dbeta = torch.empty_like(beta)
+      ws = torch.empty(int(_lib.lib().tfcb_gdn_backward_workspace_bytes(n_pix, C_)), dtype=torch.uint8, device=x.device)
+      check(_lib.lib().tfcb_gdn_backward_16bit(_p(x), _p(gamma), _p(beta), _p(dy16), _p(dx), _p(dgamma), _p(dbeta),
+                                               _p(ws), n_pix, C_, _IO16[x.dtype], _flags(inverse, rectify), float(alpha),
+                                               float(epsilon), _stream()))
+      return dx, dgamma, dbeta
+    # no native kernel (or a float32 dy, which keeps its precision): convert, run, hand dx back in x's type
     dx, dgamma, dbeta = gdn_backward(x.float(), gamma, beta, dy, inverse, rectify, alpha, epsilon, pow_alpha, pow_epsilon)
     return dx.to(x.dtype), dgamma, dbeta
   dy = dy.to(dtype=torch.float32).contiguous()

@@ -218,21 +218,30 @@ int tfcb_stochastic_round(const void* inputs_dev, int dtype, int64_t n, float st
 int tfcb_gdn_forward(const float* x_dev, const float* gamma_dev, const float* beta_dev, float* y_dev,
                      int64_t n_pix, int C, int flags, float alpha, float epsilon, void* stream);
 
-/* Gradients for upstream dy: dx [n_pix, C], dgamma [C, C], dbeta [C] (dgamma / dbeta are
- * OVERWRITTEN, reduced over all pixels).  `workspace_dev` must hold
- * tfcb_gdn_backward_workspace_bytes(n_pix, C) bytes. */
 /* Mixed-precision variant (gdn_test.py:200-210: float32 variables, float16 / bfloat16 activations): x and y in
- * 16 bits (dtype 1 float16, 2 bfloat16), arithmetic in float32 -- 4 bytes of HBM traffic per element instead of 8.
- * Native kernel for C = 128 with alpha in {1, 2}, epsilon in {1, 1/2}; TFCB_INVALID_ARGUMENT otherwise (the caller
- * converts to float32). */
+ * 16 bits (dtype 1 float16, 2 bfloat16), arithmetic in float32, y rounded once to nearest even -- 4 bytes of HBM
+ * traffic per element instead of 8.  Native kernels for C in {128, 192} with fixed alpha in {1, 2}, epsilon in
+ * {1, 1/2} and 16-byte aligned x, y and beta (C = 192: fewer than 2^31 pixels); TFCB_INVALID_ARGUMENT otherwise (the
+ * caller converts to float32). */
 int tfcb_gdn_forward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, void* y_dev,
                            int64_t n_pix, int C, int dtype, int flags, float alpha, float epsilon, void* stream);
 
+/* Gradients for upstream dy: dx [n_pix, C], dgamma [C, C], dbeta [C] (dgamma / dbeta are
+ * OVERWRITTEN, reduced over all pixels).  `workspace_dev` must hold
+ * tfcb_gdn_backward_workspace_bytes(n_pix, C) bytes. */
 int64_t tfcb_gdn_backward_workspace_bytes(int64_t n_pix, int C);
 int tfcb_gdn_backward(const float* x_dev, const float* gamma_dev, const float* beta_dev,
                       const float* dy_dev, float* dx_dev, float* dgamma_dev, float* dbeta_dev,
                       void* workspace_dev, int64_t n_pix, int C, int flags, float alpha,
                       float epsilon, void* stream);
+/* Mixed-precision backward: x, dy and dx in 16 bits of the same dtype (1 float16, 2 bfloat16); gamma, beta, dgamma,
+ * dbeta float32; arithmetic float32, dx rounded once to nearest even -- 6 bytes of HBM traffic per element for x, dy
+ * and dx.  Same workspace as tfcb_gdn_backward.  Native kernels for C in {128, 192} with fixed alpha in {1, 2},
+ * epsilon in {1, 1/2}, 16-byte aligned x, dy, dx and workspace and fewer than 2^31 pixels; TFCB_INVALID_ARGUMENT
+ * otherwise (the caller converts to float32).  n_pix == 0 zeroes dgamma and dbeta. */
+int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, const void* dy_dev,
+                            void* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix,
+                            int C, int dtype, int flags, float alpha, float epsilon, void* stream);
 
 /* Number of kernel launches issued by this library since load (bench.py's `gpu_launches`). */
 /* Gradients of the loss with respect to the scalar exponents alpha and epsilon (gdn.py:345-367 makes them
