@@ -71,6 +71,7 @@ SIGNATURES = {
     "tfcb_gdn_exponent_grads": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _f32, _f32, _vp]),
     "tfcb_gdn_backward": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _f32, _f32, _vp]),
     "tfcb_gdn_backward_16bit": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _f32, _f32, _vp]),
+    "tfcb_gdn_native_16bit": (_int, [_int, _vp, _vp, _vp, _i64, _int, _int, _int, _f32, _f32]),
 }
 
 _lib = None

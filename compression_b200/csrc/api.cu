@@ -57,6 +57,13 @@ void dev_free(void* p, cudaStream_t s) {
   }
 }
 
+int device_sm_count() {
+  int dev = 0, n = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+  return n > 0 ? n : 148;
+}
+
 }  // namespace tfcb
 
 extern "C" {

@@ -42,6 +42,13 @@ inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s
 int dev_alloc(void** p, size_t bytes, cudaStream_t s);
 void dev_free(void* p, cudaStream_t s);
 
+// Multiprocessors of the current device, asked on every call (the process may switch devices); 148 if the query fails.
+int device_sm_count();
+
+// Per-CTA dgamma / dbeta partial sums the GDN backward workspace holds (tfcb_gdn_backward_workspace_bytes): every
+// backward kernel that writes partials runs at most this many CTAs.
+constexpr int kGdnPartSlots = 148;
+
 // ---- range-coder arithmetic shared by the encoder and the decoder -----------------------------
 // floor(((span + 1) * c) / 2^p) truncated to 32 bits, for span < 2^32, c <= 2^16, 1 <= p <= 16.
 // One IMAD.WIDE.U32 (with the `+ c` folded into the 64-bit addend) and one funnel shift.

@@ -453,17 +453,6 @@ int parse_flags(int flags, float alpha, float eps, GdnFlags* f) {
   return TFCB_OK;
 }
 
-int sm_count() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    if (n <= 0) n = 148;
-  }
-  return n;
-}
-
 bool fast_c(int C) { return C % 32 == 0 && C >= 32 && C <= 192; }
 
 size_t fast_smem(int C) { return ((size_t)C * C + (size_t)kTM * (C + 4)) * sizeof(float); }
@@ -474,20 +463,14 @@ int set_smem(K kernel, size_t bytes) {
   return TFCB_OK;
 }
 
-constexpr int kDgammaGrid = 148;
-
 }  // namespace
 
-int gdn_tc_forward(const float* x, const float* gamma, const float* beta, float* y, long long n_pix, int C,
+// gdn_tc.cu: the tensor-core kernels; *handled = false where none takes the call
+int gdn_tc_forward(int io, const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C,
                    int flags, float alpha, float eps, cudaStream_t s, bool* handled);
-int gdn_tc_forward16(const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C, int flags,
-                     float alpha, float eps, int dtype, cudaStream_t s, bool* handled);
-int gdn_tc_backward(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* q_ws,
-                    float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
-                    float eps, cudaStream_t s, bool* handled);
-int gdn_tc_backward16(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
-                      float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
-                      float eps, int dtype, cudaStream_t s, bool* handled);
+int gdn_tc_backward(int io, const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
+                    float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha, float eps,
+                    cudaStream_t s, bool* handled);
 
 }  // namespace tfcb
 
@@ -504,63 +487,49 @@ using namespace tfcb;
     default: return fail(TFCB_INVALID_ARGUMENT, "unsupported channel count %d", (C)); \
   }
 
-extern "C" {
+namespace {
 
-int tfcb_gdn_forward(const float* x_dev, const float* gamma_dev, const float* beta_dev, float* y_dev,
-                     int64_t n_pix, int C, int flags, float alpha, float epsilon, void* stream) {
+// One forward for every activation type io (0 float32, 1 float16, 2 bfloat16).  The tensor cores take what tc_rule
+// (gdn_tc.cu) admits; the rest of the float32 calls run the fp32 kernels, and 16-bit calls have no other kernel.
+int gdn_forward(int io, const void* x_dev, const float* gamma_dev, const float* beta_dev, void* y_dev, int64_t n_pix,
+                int C, int flags, float alpha, float epsilon, void* stream) {
   if (n_pix < 0 || C <= 0) return fail(TFCB_INVALID_ARGUMENT, "bad GDN shape: n_pix=%lld C=%d", (long long)n_pix, C);
   if (n_pix == 0) return TFCB_OK;
   if (!x_dev || !gamma_dev || !beta_dev || !y_dev) return fail(TFCB_INVALID_ARGUMENT, "null pointer");
   cudaStream_t s = as_stream(stream);
+  bool handled = false;
+  TFCB_TRY(gdn_tc_forward(io, x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, flags, alpha, epsilon, s, &handled));
+  if (handled) return TFCB_OK;
+  if (io != 0)
+    return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: only C in {128, 192} with fixed alpha in {1, 2}, epsilon in {1, 1/2}, 16-byte "
+                "aligned x / y / beta (and fewer than 2^31 pixels at C = 192) has a native 16-bit kernel; convert to float32 "
+                "for this configuration");
+  const float* x = static_cast<const float*>(x_dev);
+  float* y = static_cast<float*>(y_dev);
   GdnFlags f;
   parse_flags(flags, alpha, epsilon, &f);
-  bool handled = false;
-  TFCB_TRY(gdn_tc_forward(x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, flags, alpha, epsilon, s, &handled));
-  if (handled) return TFCB_OK;
   if (fast_c(C)) {
     const size_t smem = fast_smem(C);
     const long long n_tiles = (n_pix + kTM - 1) / kTM;
-    const int grid = (int)std::min<long long>(n_tiles, sm_count());
+    const int grid = (int)std::min<long long>(n_tiles, device_sm_count());
     DISPATCH_CPL(C, {
       TFCB_TRY(set_smem(gdn_fwd_kernel<CPL>, smem));
-      gdn_fwd_kernel<CPL><<<grid, kThreads, smem, s>>>(x_dev, gamma_dev, beta_dev, y_dev, n_pix, f);
+      gdn_fwd_kernel<CPL><<<grid, kThreads, smem, s>>>(x, gamma_dev, beta_dev, y, n_pix, f);
     });
   } else {
     const long long blocks = (n_pix + 3) / 4;
-    gdn_fwd_generic_kernel<<<(unsigned)blocks, 128, 0, s>>>(x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, f);
+    gdn_fwd_generic_kernel<<<(unsigned)blocks, 128, 0, s>>>(x, gamma_dev, beta_dev, y, n_pix, C, f);
   }
   TFCB_LAUNCHED();
   TFCB_CUDA_TRY(cudaGetLastError());
   return TFCB_OK;
 }
 
-int tfcb_gdn_forward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, void* y_dev, int64_t n_pix,
-                           int C, int dtype, int flags, float alpha, float epsilon, void* stream) {
+// One backward for every activation type io, on the same terms as gdn_forward.
+int gdn_backward(int io, const void* x_dev, const float* gamma_dev, const float* beta_dev, const void* dy_dev,
+                 void* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix, int C, int flags,
+                 float alpha, float epsilon, void* stream) {
   if (n_pix < 0 || C <= 0) return fail(TFCB_INVALID_ARGUMENT, "bad GDN shape: n_pix=%lld C=%d", (long long)n_pix, C);
-  if (dtype != 1 && dtype != 2) return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: dtype must be 1 (float16) or 2 (bfloat16)");
-  if (!x_dev || !gamma_dev || !beta_dev || !y_dev) return fail(TFCB_INVALID_ARGUMENT, "null pointer");
-  if (n_pix == 0) return TFCB_OK;
-  bool handled = false;
-  TFCB_TRY(gdn_tc_forward16(x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, flags, alpha, epsilon, dtype, as_stream(stream), &handled));
-  if (!handled)
-    return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: only C in {128, 192} with fixed alpha in {1, 2}, epsilon in {1, 1/2}, 16-byte "
-                "aligned x / y / beta (and fewer than 2^31 pixels at C = 192) has a native 16-bit kernel; convert to float32 "
-                "for this configuration");
-  TFCB_CUDA_TRY(cudaGetLastError());
-  return TFCB_OK;
-}
-
-int64_t tfcb_gdn_backward_workspace_bytes(int64_t n_pix, int C) {
-  const int64_t q = ((n_pix + 127) / 128 * 128) * C * (int64_t)sizeof(float);  // whole 128-pixel tiles (the C = 192 tensor-core pair hands q over tile by tile)
-  const int64_t parts = (int64_t)kDgammaGrid * ((int64_t)C * C + C) * (int64_t)sizeof(float);
-  return q + parts + 256;
-}
-
-int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, const void* dy_dev,
-                            void* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix, int C,
-                            int dtype, int flags, float alpha, float epsilon, void* stream) {
-  if (n_pix < 0 || C <= 0) return fail(TFCB_INVALID_ARGUMENT, "bad GDN shape: n_pix=%lld C=%d", (long long)n_pix, C);
-  if (dtype != 1 && dtype != 2) return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: dtype must be 1 (float16) or 2 (bfloat16)");
   if (!x_dev || !gamma_dev || !beta_dev || !dy_dev || !dx_dev || !dgamma_dev || !dbeta_dev || !workspace_dev)
     return fail(TFCB_INVALID_ARGUMENT, "null pointer");
   cudaStream_t s = as_stream(stream);
@@ -569,18 +538,49 @@ int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const flo
     TFCB_CUDA_TRY(cudaMemsetAsync(dbeta_dev, 0, (size_t)C * sizeof(float), s));
     return TFCB_OK;
   }
-  // the same workspace layout as the float32 entry: q (C = 192: bf16 operand planes), then the per-CTA partials
+  // the workspace: q (the C = 192 tensor-core kernels: its bf16 operand planes), then the per-CTA partial sums
   float* q = reinterpret_cast<float*>(workspace_dev);
   float* part_g = q + (size_t)((n_pix + 127) / 128 * 128) * C;
-  float* part_b = part_g + (size_t)kDgammaGrid * C * C;
+  float* part_b = part_g + (size_t)kGdnPartSlots * C * C;
   bool handled = false;
   int n_parts = 0;
-  TFCB_TRY(gdn_tc_backward16(x_dev, gamma_dev, beta_dev, dy_dev, dx_dev, q, part_g, part_b, &n_parts, n_pix, C, flags,
-                             alpha, epsilon, dtype, s, &handled));
-  if (!handled)
-    return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit backward: only C in {128, 192} with fixed alpha in {1, 2}, epsilon in "
-                "{1, 1/2}, 16-byte aligned x / dy / dx / workspace and fewer than 2^31 pixels has a native 16-bit kernel; "
-                "convert to float32 for this configuration");
+  TFCB_TRY(gdn_tc_backward(io, x_dev, gamma_dev, beta_dev, dy_dev, dx_dev, q, part_g, part_b, &n_parts, n_pix, C, flags,
+                           alpha, epsilon, s, &handled));
+  if (!handled) {
+    if (io != 0)
+      return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit backward: only C in {128, 192} with fixed alpha in {1, 2}, epsilon in "
+                  "{1, 1/2}, 16-byte aligned x / dy / dx / workspace and fewer than 2^31 pixels has a native 16-bit kernel; "
+                  "convert to float32 for this configuration");
+    const float* x = static_cast<const float*>(x_dev);
+    const float* dy = static_cast<const float*>(dy_dev);
+    float* dx = static_cast<float*>(dx_dev);
+    GdnFlags f;
+    parse_flags(flags, alpha, epsilon, &f);
+    if (!fast_c(C)) {
+      const long long blocks = (n_pix + 3) / 4;
+      gdn_bwd_generic_kernel<<<(unsigned)blocks, 128, 0, s>>>(x, gamma_dev, beta_dev, dy, q, dx, n_pix, C, f);
+      const long long e = (long long)C * C + C;
+      gdn_bwd_generic_dgamma_kernel<<<(unsigned)((e + 127) / 128), 128, 0, s>>>(x, q, dgamma_dev, dbeta_dev, n_pix, C, f);
+      TFCB_LAUNCHED();
+      TFCB_LAUNCHED();
+      TFCB_CUDA_TRY(cudaGetLastError());
+      return TFCB_OK;
+    }
+    const size_t smem = fast_smem(C);
+    const long long n_tiles = (n_pix + kTM - 1) / kTM;
+    const int grid = (int)std::min<long long>(n_tiles, device_sm_count());
+    n_parts = (int)std::min<long long>((n_pix + 31) / 32, kGdnPartSlots);
+    DISPATCH_CPL(C, {
+      TFCB_TRY(set_smem(gdn_bwd_q_kernel<CPL>, smem));
+      TFCB_TRY(set_smem(gdn_bwd_dx_kernel<CPL>, smem));
+      gdn_bwd_q_kernel<CPL><<<grid, kThreads, smem, s>>>(x, gamma_dev, beta_dev, dy, q, dx, n_pix, f);
+      gdn_bwd_dx_kernel<CPL><<<grid, kThreads, smem, s>>>(x, gamma_dev, q, dx, n_pix, f);
+      gdn_bwd_dgamma_kernel<CPL><<<n_parts, 256, 0, s>>>(x, q, part_g, part_b, n_pix, f);
+    });
+    TFCB_LAUNCHED();
+    TFCB_LAUNCHED();
+    TFCB_LAUNCHED();
+  }
   const long long ng = (long long)C * C;
   reduce_partials_kernel<<<(unsigned)((ng + 255) / 256), 256, 0, s>>>(part_g, n_parts, ng, dgamma_dev);
   reduce_partials_kernel<<<(unsigned)((C + 255) / 256), 256, 0, s>>>(part_b, n_parts, C, dbeta_dev);
@@ -590,65 +590,40 @@ int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const flo
   return TFCB_OK;
 }
 
+}  // namespace
+
+extern "C" {
+
+int tfcb_gdn_forward(const float* x_dev, const float* gamma_dev, const float* beta_dev, float* y_dev,
+                     int64_t n_pix, int C, int flags, float alpha, float epsilon, void* stream) {
+  return gdn_forward(0, x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, flags, alpha, epsilon, stream);
+}
+
+int tfcb_gdn_forward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, void* y_dev, int64_t n_pix,
+                           int C, int dtype, int flags, float alpha, float epsilon, void* stream) {
+  if (dtype != 1 && dtype != 2) return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: dtype must be 1 (float16) or 2 (bfloat16)");
+  return gdn_forward(dtype, x_dev, gamma_dev, beta_dev, y_dev, n_pix, C, flags, alpha, epsilon, stream);
+}
+
+int64_t tfcb_gdn_backward_workspace_bytes(int64_t n_pix, int C) {
+  const int64_t q = ((n_pix + 127) / 128 * 128) * C * (int64_t)sizeof(float);  // whole 128-pixel tiles (the C = 192 tensor-core pair hands q over tile by tile)
+  const int64_t parts = (int64_t)kGdnPartSlots * ((int64_t)C * C + C) * (int64_t)sizeof(float);
+  return q + parts + 256;
+}
+
 int tfcb_gdn_backward(const float* x_dev, const float* gamma_dev, const float* beta_dev, const float* dy_dev,
                       float* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix,
                       int C, int flags, float alpha, float epsilon, void* stream) {
-  if (n_pix < 0 || C <= 0) return fail(TFCB_INVALID_ARGUMENT, "bad GDN shape: n_pix=%lld C=%d", (long long)n_pix, C);
-  if (!x_dev || !gamma_dev || !beta_dev || !dy_dev || !dx_dev || !dgamma_dev || !dbeta_dev || !workspace_dev)
-    return fail(TFCB_INVALID_ARGUMENT, "null pointer");
-  cudaStream_t s = as_stream(stream);
-  GdnFlags f;
-  parse_flags(flags, alpha, epsilon, &f);
-  if (n_pix == 0) {
-    TFCB_CUDA_TRY(cudaMemsetAsync(dgamma_dev, 0, (size_t)C * C * sizeof(float), s));
-    TFCB_CUDA_TRY(cudaMemsetAsync(dbeta_dev, 0, (size_t)C * sizeof(float), s));
-    return TFCB_OK;
-  }
-  float* q = reinterpret_cast<float*>(workspace_dev);
-  float* part_g = q + (size_t)((n_pix + 127) / 128 * 128) * C;
-  float* part_b = part_g + (size_t)kDgammaGrid * C * C;
-  bool handled = false;
-  int n_parts = 0;
-  TFCB_TRY(gdn_tc_backward(x_dev, gamma_dev, beta_dev, dy_dev, dx_dev, q, part_g, part_b, &n_parts, n_pix, C, flags,
-                           alpha, epsilon, s, &handled));
-  if (handled) {
-    const long long ng = (long long)C * C;
-    reduce_partials_kernel<<<(unsigned)((ng + 255) / 256), 256, 0, s>>>(part_g, n_parts, ng, dgamma_dev);
-    reduce_partials_kernel<<<(unsigned)((C + 255) / 256), 256, 0, s>>>(part_b, n_parts, C, dbeta_dev);
-    TFCB_LAUNCHED();
-    TFCB_LAUNCHED();
-  } else if (fast_c(C)) {
-    const size_t smem = fast_smem(C);
-    const long long n_tiles = (n_pix + kTM - 1) / kTM;
-    const int grid = (int)std::min<long long>(n_tiles, sm_count());
-    const int grid_g = (int)std::min<long long>((n_pix + 31) / 32, kDgammaGrid);
-    DISPATCH_CPL(C, {
-      TFCB_TRY(set_smem(gdn_bwd_q_kernel<CPL>, smem));
-      TFCB_TRY(set_smem(gdn_bwd_dx_kernel<CPL>, smem));
-      gdn_bwd_q_kernel<CPL><<<grid, kThreads, smem, s>>>(x_dev, gamma_dev, beta_dev, dy_dev, q, dx_dev, n_pix, f);
-      gdn_bwd_dx_kernel<CPL><<<grid, kThreads, smem, s>>>(x_dev, gamma_dev, q, dx_dev, n_pix, f);
-      gdn_bwd_dgamma_kernel<CPL><<<grid_g, 256, 0, s>>>(x_dev, q, part_g, part_b, n_pix, f);
-    });
-    TFCB_LAUNCHED();
-    TFCB_LAUNCHED();
-    TFCB_LAUNCHED();
-    const long long ng = (long long)C * C;
-    reduce_partials_kernel<<<(unsigned)((ng + 255) / 256), 256, 0, s>>>(part_g, grid_g, ng, dgamma_dev);
-    reduce_partials_kernel<<<(unsigned)((C + 255) / 256), 256, 0, s>>>(part_b, grid_g, C, dbeta_dev);
-    TFCB_LAUNCHED();
-    TFCB_LAUNCHED();
-  } else {
-    const long long blocks = (n_pix + 3) / 4;
-    gdn_bwd_generic_kernel<<<(unsigned)blocks, 128, 0, s>>>(x_dev, gamma_dev, beta_dev, dy_dev, q, dx_dev, n_pix,
-                                                            C, f);
-    const long long e = (long long)C * C + C;
-    gdn_bwd_generic_dgamma_kernel<<<(unsigned)((e + 127) / 128), 128, 0, s>>>(x_dev, q, dgamma_dev, dbeta_dev,
-                                                                             n_pix, C, f);
-    TFCB_LAUNCHED();
-    TFCB_LAUNCHED();
-  }
-  TFCB_CUDA_TRY(cudaGetLastError());
-  return TFCB_OK;
+  return gdn_backward(0, x_dev, gamma_dev, beta_dev, dy_dev, dx_dev, dgamma_dev, dbeta_dev, workspace_dev, n_pix, C,
+                      flags, alpha, epsilon, stream);
+}
+
+int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, const void* dy_dev,
+                            void* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix, int C,
+                            int dtype, int flags, float alpha, float epsilon, void* stream) {
+  if (dtype != 1 && dtype != 2) return fail(TFCB_INVALID_ARGUMENT, "GDN 16-bit: dtype must be 1 (float16) or 2 (bfloat16)");
+  return gdn_backward(dtype, x_dev, gamma_dev, beta_dev, dy_dev, dx_dev, dgamma_dev, dbeta_dev, workspace_dev, n_pix, C,
+                      flags, alpha, epsilon, stream);
 }
 
 int64_t tfcb_gdn_exponent_grads_workspace_bytes(void) { return (int64_t)kExpGrid * 2 * (int64_t)sizeof(float); }

@@ -19,8 +19,9 @@
 //   gdn_tc_bwd_dgamma2_kernel<FAST, IO>  backward, C = 192: dgamma / dbeta partials from x and q
 //   gdn_tc_prep_kernel, gdn_tc_prep2_kernel   gamma -> bf16 hi / lo operand planes
 //
-// Everything outside {C in {128, 192}, alpha in {1, 2}, eps in {1, 0.5}} (and trainable exponents) runs the fp32
-// kernels in gdn.cu.
+// tc_rule (at the end of the file) decides which calls these kernels take, for both directions and every IO;
+// gdn_tc_forward / gdn_tc_backward apply it for gdn.cu, and tfcb_gdn_native_16bit answers it for the caller of the
+// 16-bit entries.  gdn.cu runs the fp32 kernels for a float32 call the rule refuses.
 #include <cuda.h>  // CUtensorMap (types only; cuTensorMapEncodeTiled is fetched through the runtime)
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
@@ -550,11 +551,8 @@ int launch_tc_fwd2(const void* x, const float* gamma, const float* beta, void* y
       return fail(TFCB_CUDA_ERROR, "cannot reserve %d bytes of shared memory: %s", L::kBytes, cudaGetErrorString(e));
     }
   }
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  const int grid = (int)std::min<long long>(n_tiles, sms);
+  const int grid = (int)std::min<long long>(n_tiles, device_sm_count());
   gdn_tc_fwd2_kernel<FAST, IO><<<grid, kF2Threads, L::kBytes, s>>>(x, gamma, beta, y, n_pix, f);
   TFCB_LAUNCHED();
   cudaError_t e = cudaGetLastError();
@@ -969,11 +967,8 @@ int launch_tc_fwd4(const void* x, const float* gamma, const float* beta, void* y
     dev_free(planes, s);
     return fail(TFCB_CUDA_ERROR, "cannot reserve %d bytes of shared memory: %s", L::kBytes, cudaGetErrorString(e));
   }
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  const int grid = (int)std::min<long long>(n_tiles, sms);
+  const int grid = (int)std::min<long long>(n_tiles, device_sm_count());
   gdn_tc_fwd4_kernel<C, FAST, IO><<<grid, kF4Threads, L::kBytes, s>>>(x_map, y_map, x, planes, beta, n_pix, f);
   TFCB_LAUNCHED();
   e = cudaGetLastError();
@@ -1576,11 +1571,8 @@ int launch_tc_bwd3(const void* x, const float* gamma, const float* beta, const v
     dev_free(planes, s);
     return fail(TFCB_CUDA_ERROR, "cannot reserve %d bytes of shared memory: %s", L::kBytes, cudaGetErrorString(e));
   }
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
+  const int grid = (int)std::min<long long>(n_tiles, std::min(device_sm_count(), kGdnPartSlots));
   gdn_tc_bwd3_kernel<FAST, IO><<<grid, kB3Threads, L::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta, part_g,
                                                                   part_b, n_pix, f);
   TFCB_LAUNCHED();
@@ -2353,11 +2345,8 @@ int launch_tc_bwd192(const void* x, const float* gamma, const float* beta, const
   TFCB_TRY(dev_alloc((void**)&planes, (size_t)4 * C * C * sizeof(__nv_bfloat16), s));
   gdn_tc_prep2_kernel<false><<<((C / 8) * C + 255) / 256, 256, 0, s>>>(gamma, C, planes);
   TFCB_LAUNCHED();
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (n_pix + kTileM - 1) / kTileM;
-  const int grid = (int)std::min<long long>(n_tiles, std::min(sms, 148));
+  const int grid = (int)std::min<long long>(n_tiles, std::min(device_sm_count(), kGdnPartSlots));
   gdn_tc_bwd_dx2_kernel<FAST, IO><<<grid, kD2Threads, L2::kBytes, s>>>(x_map, g_map, dx_map, x, dy, planes, beta,
                                                                       reinterpret_cast<uint8_t*>(q_ws), n_pix, f);
   TFCB_LAUNCHED();
@@ -2371,10 +2360,20 @@ int launch_tc_bwd192(const void* x, const float* gamma, const float* beta, const
   return TFCB_OK;
 }
 
-// The tensor-core kernels take alpha in {1, 2}, epsilon in {1, 1/2} as fixed exponents; false otherwise.
-bool tc_flags(int flags, float alpha, float eps, TcFlags* f, bool* fast) {
-  if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return false;
+// Whether a tensor-core kernel takes a call, for either direction and every activation type io (0 float32, 1 float16,
+// 2 bfloat16); if so, *f and *fast say which instantiation and with which flags.  The pointers are those the kernels
+// move with 16-byte accesses: forward x, y (out) and beta; backward x, dy, dx (out) and, at C = 192, the q workspace.
+// The forward ignores dy and ws, the backward beta (its kernels read beta element by element).
+bool tc_rule(bool backward, int io, long long n_pix, int C, int flags, float alpha, float eps, const void* x,
+             const void* beta, const void* dy, const void* out, const void* ws, TcFlags* f, bool* fast) {
+  if ((io != 0 && io != 1 && io != 2) || (C != 128 && C != 192)) return false;
+  if (!(alpha == 1.f || alpha == 2.f) || !(eps == 1.f || eps == 0.5f)) return false;  // fixed exponents only
   if (flags & (TFCB_GDN_POW_ALPHA | TFCB_GDN_POW_EPSILON)) return false;  // trainable exponents: literal pow
+  const uintptr_t addr = backward ? (uintptr_t)x | (uintptr_t)dy | (uintptr_t)out | (C == 192 ? (uintptr_t)ws : 0)
+                                  : (uintptr_t)x | (uintptr_t)out | (uintptr_t)beta;
+  if (addr & 15) return false;
+  // TMA boxes take 32-bit row coordinates; only the C = 128 forward moves x without them
+  if ((backward || C == 192) && n_pix >= (1ll << 31)) return false;
   f->inverse = (flags & TFCB_GDN_INVERSE) ? 1 : 0;
   f->rectify = (flags & TFCB_GDN_RECTIFY) ? 1 : 0;
   f->alpha_mode = (alpha == 2.f) ? 2 : 1;
@@ -2383,95 +2382,68 @@ bool tc_flags(int flags, float alpha, float eps, TcFlags* f, bool* fast) {
   return true;
 }
 
-bool misaligned16(const void* a, const void* b, const void* c) {
-  return ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) | reinterpret_cast<uintptr_t>(c)) & 15) != 0;
-}
-
-// 16-bit activations (float16 / bfloat16 in, same type out; parameters and arithmetic float32): the same kernels as the
-// float32 path, instantiated for 16-bit elements.  *handled = false -> no native kernel for this call.
-template <int IO>
-int gdn_tc_forward16_io(const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C, TcFlags f,
-                        bool fast, cudaStream_t s) {
-  if (C == 128)
-    return fast ? launch_tc_fwd2<true, IO>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd2<false, IO>(x, gamma, beta, y, n_pix, f, s);
-  return fast ? launch_tc_fwd4<true, IO>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd4<false, IO>(x, gamma, beta, y, n_pix, f, s);
-}
-
-// Tensor-core backward; fills the per-CTA partial sums (part_g [n_parts][C][C], part_b [n_parts][C]) that the caller
-// reduces.  *handled = false -> no tensor-core kernel for this call (float32: the caller runs the fp32 kernels).
-template <int IO>
-int gdn_tc_backward_io(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
-                       float* part_g, float* part_b, int* n_parts, long long n_pix, int C, TcFlags f, bool fast,
-                       cudaStream_t s) {
-  if (C == 128)
-    return fast ? launch_tc_bwd3<true, IO>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s)
-                : launch_tc_bwd3<false, IO>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
-  return fast ? launch_tc_bwd192<true, IO>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s)
-              : launch_tc_bwd192<false, IO>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
-}
-
-// The conditions under which the box-fed backward kernels apply, whatever the activation type
-bool tc_backward_applies(const void* x, const void* dy, const void* dx, const float* q_ws, long long n_pix, int C,
-                         int flags, float alpha, float eps, TcFlags* f, bool* fast) {
-  if (C != 128 && C != 192) return false;
-  if (C == 192 && (reinterpret_cast<uintptr_t>(q_ws) & 15)) return false;
-  if (!tc_flags(flags, alpha, eps, f, fast)) return false;
-  if (misaligned16(x, dy, dx)) return false;
-  return n_pix < (1ll << 31);  // the box kernels take 32-bit TMA row coordinates
-}
+constexpr int tc_case(int C, bool fast, int io) { return (C == 192 ? 6 : 0) + (fast ? 3 : 0) + io; }
 
 }  // namespace
 
-int gdn_tc_forward(const float* x, const float* gamma, const float* beta, float* y, long long n_pix, int C,
+// *handled = false: no tensor-core kernel takes this call (tc_rule).
+int gdn_tc_forward(int io, const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C,
                    int flags, float alpha, float eps, cudaStream_t s, bool* handled) {
-  *handled = false;
-  if (!(C == 128 || C == 192)) return TFCB_OK;
   TcFlags f;
   bool fast;
-  if (!tc_flags(flags, alpha, eps, &f, &fast)) return TFCB_OK;
-  if (misaligned16(x, y, beta)) return TFCB_OK;  // 16-byte rows
-  *handled = true;
-  if (C == 128)  // x tile resident in shared memory, bulk async copies
-    return fast ? launch_tc_fwd2<true, 0>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd2<false, 0>(x, gamma, beta, y, n_pix, f, s);
-  // C == 192: x through rings of 2-D TMA boxes, gamma's lo plane streamed, y through TMA stores
-  if (n_pix >= (1ll << 31)) return fail(TFCB_INVALID_ARGUMENT, "GDN: more than 2^31 pixels in one call");
-  return fast ? launch_tc_fwd4<true, 0>(x, gamma, beta, y, n_pix, f, s) : launch_tc_fwd4<false, 0>(x, gamma, beta, y, n_pix, f, s);
-}
-
-int gdn_tc_forward16(const void* x, const float* gamma, const float* beta, void* y, long long n_pix, int C, int flags,
-                     float alpha, float eps, int dtype, cudaStream_t s, bool* handled) {
-  *handled = false;
-  if (!(C == 128 || C == 192) || (dtype != 1 && dtype != 2)) return TFCB_OK;
-  TcFlags f;
-  bool fast;
-  if (!tc_flags(flags, alpha, eps, &f, &fast)) return TFCB_OK;
-  if (misaligned16(x, y, beta)) return TFCB_OK;
-  if (C == 192 && n_pix >= (1ll << 31)) return TFCB_OK;  // 32-bit TMA row coordinates
-  *handled = true;
-  return dtype == 1 ? gdn_tc_forward16_io<1>(x, gamma, beta, y, n_pix, C, f, fast, s)
-                    : gdn_tc_forward16_io<2>(x, gamma, beta, y, n_pix, C, f, fast, s);
-}
-
-int gdn_tc_backward(const float* x, const float* gamma, const float* beta, const float* dy, float* dx, float* q_ws,
-                    float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
-                    float eps, cudaStream_t s, bool* handled) {
-  TcFlags f;
-  bool fast;
-  *handled = tc_backward_applies(x, dy, dx, q_ws, n_pix, C, flags, alpha, eps, &f, &fast);
+  *handled = tc_rule(false, io, n_pix, C, flags, alpha, eps, x, beta, nullptr, y, nullptr, &f, &fast);
   if (!*handled) return TFCB_OK;
-  return gdn_tc_backward_io<0>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, C, f, fast, s);
+  switch (tc_case(C, fast, io)) {
+    case tc_case(128, false, 0): return launch_tc_fwd2<false, 0>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(128, false, 1): return launch_tc_fwd2<false, 1>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(128, false, 2): return launch_tc_fwd2<false, 2>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(128, true, 0): return launch_tc_fwd2<true, 0>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(128, true, 1): return launch_tc_fwd2<true, 1>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(128, true, 2): return launch_tc_fwd2<true, 2>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(192, false, 0): return launch_tc_fwd4<false, 0>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(192, false, 1): return launch_tc_fwd4<false, 1>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(192, false, 2): return launch_tc_fwd4<false, 2>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(192, true, 0): return launch_tc_fwd4<true, 0>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(192, true, 1): return launch_tc_fwd4<true, 1>(x, gamma, beta, y, n_pix, f, s);
+    case tc_case(192, true, 2): return launch_tc_fwd4<true, 2>(x, gamma, beta, y, n_pix, f, s);
+  }
+  return fail(TFCB_INVALID_ARGUMENT, "GDN: no tensor-core forward for C=%d", C);  // not reached: tc_rule admits only the cases above
 }
 
-// 16-bit x, dy and dx (dtype 1 float16, 2 bfloat16); float32 parameters, partial sums and arithmetic
-int gdn_tc_backward16(const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
-                      float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha,
-                      float eps, int dtype, cudaStream_t s, bool* handled) {
+// Fills the per-CTA partial sums (part_g [n_parts][C][C], part_b [n_parts][C]) that the caller reduces.
+// *handled = false: no tensor-core kernel takes this call (tc_rule).
+int gdn_tc_backward(int io, const void* x, const float* gamma, const float* beta, const void* dy, void* dx, float* q_ws,
+                    float* part_g, float* part_b, int* n_parts, long long n_pix, int C, int flags, float alpha, float eps,
+                    cudaStream_t s, bool* handled) {
   TcFlags f;
   bool fast;
-  *handled = (dtype == 1 || dtype == 2) && tc_backward_applies(x, dy, dx, q_ws, n_pix, C, flags, alpha, eps, &f, &fast);
+  *handled = tc_rule(true, io, n_pix, C, flags, alpha, eps, x, beta, dy, dx, q_ws, &f, &fast);
   if (!*handled) return TFCB_OK;
-  return dtype == 1 ? gdn_tc_backward_io<1>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, C, f, fast, s)
-                    : gdn_tc_backward_io<2>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, C, f, fast, s);
+  switch (tc_case(C, fast, io)) {
+    case tc_case(128, false, 0): return launch_tc_bwd3<false, 0>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(128, false, 1): return launch_tc_bwd3<false, 1>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(128, false, 2): return launch_tc_bwd3<false, 2>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(128, true, 0): return launch_tc_bwd3<true, 0>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(128, true, 1): return launch_tc_bwd3<true, 1>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(128, true, 2): return launch_tc_bwd3<true, 2>(x, gamma, beta, dy, dx, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(192, false, 0): return launch_tc_bwd192<false, 0>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(192, false, 1): return launch_tc_bwd192<false, 1>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(192, false, 2): return launch_tc_bwd192<false, 2>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(192, true, 0): return launch_tc_bwd192<true, 0>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(192, true, 1): return launch_tc_bwd192<true, 1>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+    case tc_case(192, true, 2): return launch_tc_bwd192<true, 2>(x, gamma, beta, dy, dx, q_ws, part_g, part_b, n_parts, n_pix, f, s);
+  }
+  return fail(TFCB_INVALID_ARGUMENT, "GDN: no tensor-core backward for C=%d", C);  // not reached: tc_rule admits only the cases above
 }
 
 }  // namespace tfcb
+
+extern "C" int tfcb_gdn_native_16bit(int backward, const void* x_dev, const void* beta_dev, const void* dy_dev,
+                                     int64_t n_pix, int C, int dtype, int flags, float alpha, float epsilon) {
+  // the caller allocates y / dx and the workspace, so they are aligned
+  tfcb::TcFlags f;
+  bool fast;
+  return n_pix > 0 && (dtype == 1 || dtype == 2) &&
+         tfcb::tc_rule(backward != 0, dtype, n_pix, C, flags, alpha, epsilon, x_dev, beta_dev, dy_dev, nullptr, nullptr,
+                       &f, &fast);
+}

@@ -1606,16 +1606,6 @@ __global__ void __launch_bounds__(32) legacy_decode_kernel(const uint8_t* bytes,
 // ---------------------------------------------------------------------------------------------
 // Host-side handles
 // ---------------------------------------------------------------------------------------------
-int device_sm_count() {
-  static int n = 0;
-  if (n == 0) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-    if (n <= 0) n = 148;
-  }
-  return n;
-}
 
 // ---------------------------------------------------------------------------------------------
 // Device-table cache.  A model creates a handle per compress()/decompress() call with the same `lookup`

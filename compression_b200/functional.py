@@ -42,33 +42,23 @@ def _gdn_args(x, gamma, beta):
   return x, gamma, beta, C_, x.numel() // C_
 
 
-def _native16(x, beta, C_, n_pix, alpha, epsilon, pow_alpha, pow_epsilon, dy=None, boxes=True):
-  """True where a kernel reads and writes the 16-bit activations itself (mixed precision, gdn_test.py:200-210):
-  C in {128, 192}, fixed alpha in {1, 2} and epsilon in {1, 1/2}, at least one pixel (fewer than 2^31 where the
-  kernel moves x in TMA boxes, which take 32-bit row coordinates), 16-byte aligned x / beta / dy, and dy of x's
-  type.  Everything else converts to float32 and back."""
-  return (x.dtype in _IO16 and C_ in (128, 192) and not pow_alpha and not pow_epsilon and
-          float(alpha) in (1.0, 2.0) and float(epsilon) in (1.0, 0.5) and n_pix > 0 and
-          (n_pix < 2**31 or not boxes) and (dy is None or dy.dtype == x.dtype) and
-          all(t.data_ptr() % 16 == 0 for t in (x, beta) + (() if dy is None else (dy,))))
-
-
 def gdn_forward(x, gamma, beta, inverse=False, rectify=False, alpha=1.0, epsilon=1.0, pow_alpha=False,
                 pow_epsilon=False):
   """x: float32 / float16 / bfloat16 CUDA [..., C] (channels-last, contiguous) -> y of the same shape and type."""
   x, gamma, beta, C_, n_pix = _gdn_args(x, gamma, beta)
+  flags = _flags(inverse, rectify, pow_alpha, pow_epsilon)
   if x.dtype in _IO16:
-    # 16-bit activations, float32 parameters and arithmetic: the kernel reads and writes the 16-bit elements where
-    # _native16 allows it (C = 128 keeps the whole tile in shared memory and needs no boxes); otherwise convert.
-    if _native16(x, beta, C_, n_pix, alpha, epsilon, pow_alpha, pow_epsilon, boxes=C_ != 128):
+    # 16-bit activations, float32 parameters and arithmetic (mixed precision, gdn_test.py:200-210): the kernel reads
+    # and writes the 16-bit elements where the library has one for this call; otherwise convert
+    if _lib.lib().tfcb_gdn_native_16bit(0, _p(x), _p(beta), None, n_pix, C_, _IO16[x.dtype], flags, float(alpha),
+                                        float(epsilon)):
       y = torch.empty_like(x)
-      check(_lib.lib().tfcb_gdn_forward_16bit(_p(x), _p(gamma), _p(beta), _p(y), n_pix, C_, _IO16[x.dtype],
-                                              _flags(inverse, rectify), float(alpha), float(epsilon), _stream()))
+      check(_lib.lib().tfcb_gdn_forward_16bit(_p(x), _p(gamma), _p(beta), _p(y), n_pix, C_, _IO16[x.dtype], flags,
+                                              float(alpha), float(epsilon), _stream()))
       return y
     return gdn_forward(x.float(), gamma, beta, inverse, rectify, alpha, epsilon, pow_alpha, pow_epsilon).to(x.dtype)
   y = torch.empty_like(x)
-  check(_lib.lib().tfcb_gdn_forward(_p(x), _p(gamma), _p(beta), _p(y), n_pix, C_,
-                                    _flags(inverse, rectify, pow_alpha, pow_epsilon), float(alpha), float(epsilon),
+  check(_lib.lib().tfcb_gdn_forward(_p(x), _p(gamma), _p(beta), _p(y), n_pix, C_, flags, float(alpha), float(epsilon),
                                     _stream()))
   return y
 
@@ -77,16 +67,18 @@ def gdn_backward(x, gamma, beta, dy, inverse=False, rectify=False, alpha=1.0, ep
                  pow_epsilon=False):
   """Returns (dx, dgamma, dbeta) for upstream gradient dy; dx has x's type, dgamma / dbeta are float32."""
   x, gamma, beta, C_, n_pix = _gdn_args(x, gamma, beta)
+  flags = _flags(inverse, rectify, pow_alpha, pow_epsilon)
   if x.dtype in _IO16:
     dy16 = dy.contiguous()
-    if _native16(x, beta, C_, n_pix, alpha, epsilon, pow_alpha, pow_epsilon, dy=dy16):
+    if dy16.dtype == x.dtype and _lib.lib().tfcb_gdn_native_16bit(1, _p(x), _p(beta), _p(dy16), n_pix, C_, _IO16[x.dtype],
+                                                                  flags, float(alpha), float(epsilon)):
       dx = torch.empty_like(x)
       dgamma = torch.empty_like(gamma)
       dbeta = torch.empty_like(beta)
       ws = torch.empty(int(_lib.lib().tfcb_gdn_backward_workspace_bytes(n_pix, C_)), dtype=torch.uint8, device=x.device)
       check(_lib.lib().tfcb_gdn_backward_16bit(_p(x), _p(gamma), _p(beta), _p(dy16), _p(dx), _p(dgamma), _p(dbeta),
-                                               _p(ws), n_pix, C_, _IO16[x.dtype], _flags(inverse, rectify), float(alpha),
-                                               float(epsilon), _stream()))
+                                               _p(ws), n_pix, C_, _IO16[x.dtype], flags, float(alpha), float(epsilon),
+                                               _stream()))
       return dx, dgamma, dbeta
     # no native kernel (or a float32 dy, which keeps its precision): convert, run, hand dx back in x's type
     dx, dgamma, dbeta = gdn_backward(x.float(), gamma, beta, dy, inverse, rectify, alpha, epsilon, pow_alpha, pow_epsilon)
@@ -98,8 +90,7 @@ def gdn_backward(x, gamma, beta, dy, inverse=False, rectify=False, alpha=1.0, ep
   ws_bytes = int(_lib.lib().tfcb_gdn_backward_workspace_bytes(n_pix, C_))
   ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
   check(_lib.lib().tfcb_gdn_backward(_p(x), _p(gamma), _p(beta), _p(dy), _p(dx), _p(dgamma), _p(dbeta), _p(ws),
-                                     n_pix, C_, _flags(inverse, rectify, pow_alpha, pow_epsilon), float(alpha),
-                                     float(epsilon), _stream()))
+                                     n_pix, C_, flags, float(alpha), float(epsilon), _stream()))
   return dx, dgamma, dbeta
 
 

@@ -202,9 +202,11 @@ int tfcb_stochastic_round(const void* inputs_dev, int dtype, int64_t n, float st
  *   y_i = u_i / n_i^eps  (GDN)   or   u_i * n_i^eps  (IGDN)
  * x, y: float32 [n_pix, C] row-major;  gamma float32 [C, C] (row j, column i);  beta float32 [C].
  * alpha in {1, 2} and eps in {1, 0.5} take the reference's fast paths; other values use powf.
- * C in {128, 192} with those alpha / eps and 16-byte aligned pointers run on the tensor cores (bf16 split with
- * fp32 accumulation: <= 1e-5 relative forward, <= 2e-5 of the largest gradient backward); every other shape
- * runs the fp32 kernels.
+ * C in {128, 192} with those alpha / eps (not trainable) and 16-byte aligned activations run on the tensor cores (bf16
+ * split with fp32 accumulation: <= 1e-5 relative forward, <= 2e-5 of the largest gradient backward); every other
+ * call runs the fp32 kernels.  The aligned pointers are x, y and beta forward, x, dy, dx and (C = 192) the workspace
+ * backward; every kernel but the C = 128 forward also needs fewer than 2^31 pixels.  tfcb_gdn_native_16bit states the
+ * rule.
  * The reference has no native GDN code (TF graph of abs / conv1x1 / bias_add / div); the backward
  * pass replaces TF autodiff of that graph.
  * ---------------------------------------------------------------------------------------------- */
@@ -220,9 +222,8 @@ int tfcb_gdn_forward(const float* x_dev, const float* gamma_dev, const float* be
 
 /* Mixed-precision variant (gdn_test.py:200-210: float32 variables, float16 / bfloat16 activations): x and y in
  * 16 bits (dtype 1 float16, 2 bfloat16), arithmetic in float32, y rounded once to nearest even -- 4 bytes of HBM
- * traffic per element instead of 8.  Native kernels for C in {128, 192} with fixed alpha in {1, 2}, epsilon in
- * {1, 1/2} and 16-byte aligned x, y and beta (C = 192: fewer than 2^31 pixels); TFCB_INVALID_ARGUMENT otherwise (the
- * caller converts to float32). */
+ * traffic per element instead of 8.  Runs the tensor-core kernels only; TFCB_INVALID_ARGUMENT where they do not take
+ * the call (tfcb_gdn_native_16bit returns 0; the caller converts to float32). */
 int tfcb_gdn_forward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, void* y_dev,
                            int64_t n_pix, int C, int dtype, int flags, float alpha, float epsilon, void* stream);
 
@@ -236,12 +237,17 @@ int tfcb_gdn_backward(const float* x_dev, const float* gamma_dev, const float* b
                       float epsilon, void* stream);
 /* Mixed-precision backward: x, dy and dx in 16 bits of the same dtype (1 float16, 2 bfloat16); gamma, beta, dgamma,
  * dbeta float32; arithmetic float32, dx rounded once to nearest even -- 6 bytes of HBM traffic per element for x, dy
- * and dx.  Same workspace as tfcb_gdn_backward.  Native kernels for C in {128, 192} with fixed alpha in {1, 2},
- * epsilon in {1, 1/2}, 16-byte aligned x, dy, dx and workspace and fewer than 2^31 pixels; TFCB_INVALID_ARGUMENT
- * otherwise (the caller converts to float32).  n_pix == 0 zeroes dgamma and dbeta. */
+ * and dx.  Same workspace as tfcb_gdn_backward.  Runs the tensor-core kernels only; TFCB_INVALID_ARGUMENT where they
+ * do not take the call (the caller converts to float32).  n_pix == 0 zeroes dgamma and dbeta. */
 int tfcb_gdn_backward_16bit(const void* x_dev, const float* gamma_dev, const float* beta_dev, const void* dy_dev,
                             void* dx_dev, float* dgamma_dev, float* dbeta_dev, void* workspace_dev, int64_t n_pix,
                             int C, int dtype, int flags, float alpha, float epsilon, void* stream);
+/* 1 where tfcb_gdn_forward_16bit (backward = 0) or tfcb_gdn_backward_16bit (backward = 1) has a kernel for the call,
+ * 0 otherwise, including n_pix == 0.  Host only: reads none of the pointers, only their alignment.  The forward looks
+ * at x and beta, the backward at x and dy; y, dx and the workspace are taken to be 16-byte aligned, as fresh
+ * allocations are. */
+int tfcb_gdn_native_16bit(int backward, const void* x_dev, const void* beta_dev, const void* dy_dev, int64_t n_pix,
+                          int C, int dtype, int flags, float alpha, float epsilon);
 
 /* Number of kernel launches issued by this library since load (bench.py's `gpu_launches`). */
 /* Gradients of the loss with respect to the scalar exponents alpha and epsilon (gdn.py:345-367 makes them

@@ -199,6 +199,34 @@ def test_misaligned_view_takes_the_conversion_path(F, C):
 
 
 @pytest.mark.gpu
+@pytest.mark.parametrize("C", [128, 192])
+def test_misaligned_beta_keeps_the_native_backward(F, C):
+  """The backward kernels read beta element by element, so a beta view off a 16-byte boundary does not send a 16-bit
+  backward through the conversion path (the forward's C = 128 kernel reads beta with 16-byte loads and still does)."""
+  from compression_b200 import _lib
+  n_pix = 65536 + 77
+  gamma, beta = _params(C, 121)
+  g = gamma.cuda()
+  b = torch.empty(C + 1, device="cuda")[1:]
+  b.copy_(beta)
+  assert b.data_ptr() % 16 != 0
+  dtype = torch.bfloat16
+  x = _x(n_pix, C, 122).to(dtype).cuda()
+  dy = _dy(n_pix, C, 123).to(dtype).cuda()
+  ws = int(_lib.lib().tfcb_gdn_backward_workspace_bytes(n_pix, C))
+  torch.cuda.synchronize()
+  torch.cuda.reset_peak_memory_stats()
+  base = torch.cuda.memory_allocated()
+  dx, dg, db = F.gdn_backward(x, g, b, dy)
+  torch.cuda.synchronize()
+  # dx, dgamma, dbeta, the workspace; the conversion path would add x, dy and dx in float32, 12 B/element
+  assert torch.cuda.max_memory_allocated() - base <= 2 * n_pix * C + 4 * (C * C + C) + ws + (1 << 20)
+  dx32, dg32, db32 = F.gdn_backward(x.float(), g, b, dy.float())
+  assert torch.equal(dx, dx32.to(dtype))
+  assert _of_max(dg, dg32) <= 1e-6 and _of_max(db, db32) <= 1e-6  # (C = 128 sums dbeta with shared-memory atomics)
+
+
+@pytest.mark.gpu
 def test_float32_dy_keeps_its_precision(F):
   C, n_pix = 192, 700
   gamma, beta = _params(C, 101)
